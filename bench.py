@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Diamond PPO hot path on B200 (contract: see the task statement / DESIGN.md §Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[4], "synthetic scale"): ONE 4096-env x 128-step buffer, obs_dim 64, default actor-critic
 MLP at hidden 256, 4 actions, 4 epochs x 8 minibatches.  A "step" is one PPO.learn() over that buffer: pre-update pass,
@@ -306,8 +306,17 @@ def bench_train_iteration(reps=3):
             "sample_updates_per_s": E * T * N_ENVS / (ms_iter * 1e-3)}
 
 
-def time_learn(agent, buf, host, steps, warmup, world, dist, ctx):
-    """(ms per learn() device-resident, per-phase ms, launches, clocks, ms per learn() end to end, h2d bytes, losses)."""
+def learn_outputs(agent):
+    """What learn() leaves its caller: the per-minibatch losses [E*MB, 4] (policy, value, entropy, total) and the updated
+    network parameters."""
+    out = {"losses": agent.last_losses.cpu().numpy()}
+    out.update({f"params.{n}": p.detach().cpu().numpy() for n, p in agent.network.named_parameters()})
+    return out
+
+
+def time_learn(agent, buf, host, steps, warmup, world, dist, ctx, keep_outputs=False):
+    """(ms per learn() device-resident, per-phase ms, launches, clocks, ms per learn() end to end, h2d bytes, losses).
+    keep_outputs: also return learn_outputs() of the last timed learn(), read after the timed region."""
     def barrier():
         if world > 1:
             dist.barrier()
@@ -337,6 +346,8 @@ def time_learn(agent, buf, host, steps, warmup, world, dist, ctx):
               "gae_and_stats": float(np.mean([ev["prepass_end"].elapsed_time(ev["gae_end"]) for ev in ev_all])),
               "update_loop": float(np.mean([ev["gae_end"].elapsed_time(ev["update_end"]) for ev in ev_all]))}
     out = dict(ms=float(ms_total) / steps, phases=phases, launches=launches, clocks=clocks)
+    if keep_outputs:
+        out["outputs"] = learn_outputs(agent)
     if host is None:
         return out
     # ---- end to end through the public API with host buffers ----
@@ -377,6 +388,14 @@ def time_learn(agent, buf, host, steps, warmup, world, dist, ctx):
     return out
 
 
+def dump_outputs(path, arrays):
+    """DIR/<name>.npy per array, float32 or float64, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def replicas_identical(agent, dist):
     flat = agent.engine.P.clone()
     ref = flat.clone()
@@ -413,8 +432,10 @@ def run_ours(args, rank, world, local_rank):
     buf.load_host(*host)
     torch.cuda.synchronize()
     np.random.seed(123)
-    main = time_learn(agent, buf, host, args.steps, args.warmup, world, dist, ctx)
+    main = time_learn(agent, buf, host, args.steps, args.warmup, world, dist, ctx, keep_outputs=args.dump_outputs is not None and rank == 0)
     agent.engine.check_health()
+    if "outputs" in main:
+        dump_outputs(args.dump_outputs, main["outputs"])
     ms_per_step, clocks, launches = main["ms"], main["clocks"], main["launches"]
     t_pre, t_gae, t_upd = (main["phases"][k] for k in ("prepass", "gae_and_stats", "update_loop"))
     sample_updates = E * T * N_ENVS
@@ -507,7 +528,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--dp-exchange", default="fused", choices=["fused", "nccl"])
     ap.add_argument("--no-weak", action="store_true", help="skip the extra weak-scaling measurement at --gpus > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed learn() computed (losses, updated parameters) as DIR/<name>.npy; the inputs "
+                         "are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, world, local_rank = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":

@@ -12,6 +12,7 @@ numpy 2.3.5 CPU.  Loss components are captured with call hooks; no reference
 source is edited (the recurrent case applies the documented 2-line None-check
 fix, SURVEY.md §0.4).
 """
+import io
 import os
 import sys
 
@@ -96,6 +97,21 @@ class LossHooks:
         torch.distributions.Normal.entropy = self._nent
 
 
+MAX_FILE_BYTES = 1_000_000
+
+
+def save_learn_fixture(name, out):
+    """learn_<name>.npz; where that file would exceed 1 MB, the outputs after the last epoch go to learn_<name>.e<E>.npz
+    (tests/test_agents_gpu.py load_fixture merges the two)."""
+    tag = f"e{int(out['meta'][5])}."
+    whole = io.BytesIO()
+    np.savez_compressed(whole, **out)
+    if whole.tell() > MAX_FILE_BYTES and tag != "e1.":
+        np.savez_compressed(os.path.join(HERE, f"learn_{name}.{tag}npz"), **{k: v for k, v in out.items() if k.startswith(tag)})
+        out = {k: v for k, v in out.items() if not k.startswith(tag)}
+    np.savez_compressed(os.path.join(HERE, f"learn_{name}.npz"), **out)
+
+
 def sd_np(sd, prefix):
     return {f"{prefix}{k}": v.detach().cpu().numpy().copy() for k, v in sd.items()}
 
@@ -159,7 +175,7 @@ def learn_case(name, kind, D, act, H, N, T, E, MB, seed_exp, save_adam=False, ex
                     out[f"e1.exp_avg.{n}"] = st[i]["exp_avg"].numpy().copy()
                     out[f"e1.exp_avg_sq.{n}"] = st[i]["exp_avg_sq"].numpy().copy()
                     out[f"e1.step.{n}"] = np.float64(float(st[i]["step"]))
-    np.savez_compressed(os.path.join(HERE, f"learn_{name}.npz"), **out)
+    save_learn_fixture(name, out)
     print(name, "losses[0]", out["e1.losses"][0], "n_mb", len(out["e1.losses"]))
 
 
@@ -194,7 +210,7 @@ def seeded_learn_case(name, D, act, H, N, T, E, MB, seed):
         out[f"{tag}.losses"] = np.asarray(lh.rows, dtype=np.float64)
         if tag == "e1":
             out["gae.values16"], out["gae.next_values16"], out["gae.advantages16"] = (captured[k] for k in ("values", "next_values", "advantages"))
-    np.savez_compressed(os.path.join(HERE, f"learn_{name}.npz"), **out)
+    save_learn_fixture(name, out)
     print(name, "losses[0]", out["e1.losses"][0], "n_mb", len(out["e1.losses"]))
 
 

@@ -89,7 +89,14 @@ def _run_learn(name, epochs_tag, extra=None):
 @pytest.mark.parametrize("name", ["C", "L", "Ssmall", "Pn", "Pn3"])
 def test_learn_oracle_one_epoch(name):
     g, p, state, losses, inter, names = _run_learn(name, "e1")
-    np.testing.assert_array_equal(inter["advantages"], g["gae.advantages"])
+    # GAE is bit-exact on the reference's own values.  The oracle's values come from the host's float32 GEMMs, whose rounding
+    # depends on the CPU's instruction set (MKL picks its kernels per CPU), so they and the advantages computed from them are
+    # compared to a tolerance.
+    rollout = [np.asarray(g[k]).astype(np.float32) for k in ("rewards", "terminations", "truncations")]
+    cfg = O.default_cfg()
+    np.testing.assert_array_equal(O.gae(*rollout, g["gae.values"], g["gae.next_values"], cfg["gamma"], cfg["gae_lambda"]),
+                                  g["gae.advantages"])
+    assert np.abs(inter["advantages"] - g["gae.advantages"]).max() / np.abs(g["gae.advantages"]).max() <= 1e-5
     np.testing.assert_allclose(inter["values"], g["gae.values"], rtol=1e-5, atol=1e-6)
     ref_l = g["e1.losses"]
     got = np.array([[l[k] for k in ("policy", "value", "entropy", "total")] for l in losses])
