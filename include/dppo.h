@@ -72,9 +72,10 @@ typedef struct dppo_hyper {
                                  when set, the Adam kernel reads its two step-dependent constants (and the data-parallel exchange
                                  kernel the sequence number it publishes / waits for) from device memory instead of from lr / step,
                                  so a captured CUDA graph of an optimiser step can be replayed */
-    double* grad_sumsq;       /* optional DEVICE buffer of dppo_grad_sumsq_bytes(): dppo_mlp_grad_minibatch leaves the fp64 partial
-                                 sums of squares of the gradient it assembled there and dppo_clip_adam_step reads them instead of
-                                 launching its own norm kernel (single-GPU path; under DP the norm is taken after the exchange) */
+    double* grad_sumsq;       /* optional DEVICE buffer of dppo_grad_sumsq_bytes(): dppo_mlp_grad_minibatch and
+                                 dppo_rnn_grad_minibatch leave the fp64 partial sums of squares of the gradient they assembled there
+                                 and dppo_clip_adam_step reads them instead of launching its own norm kernel (single-GPU path; under
+                                 DP the norm is taken after the exchange) */
 } dppo_hyper;
 
 /* ---- context -------------------------------------------------------------------------- */
@@ -299,8 +300,10 @@ int dppo_rnn_forward(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* para
                      float* values, float* hx_out, void* ws, int64_t ws_bytes, void* stream);
 /* One optimiser step's gradient (recurrent_ppo.py:335-362): full-sequence forward with the current parameters, the rows
  * idx[0..M) of the flattened [T*N] outputs enter the PPO loss (idx NULL: all rows in order, M = T*N), back-propagation
- * through all T steps.  actions int32 [T*N]; old_log_probs / adv / returns f32 [T*N]; flat gradient -> grads,
- * (policy, value, entropy, total) -> losses[0..3]. */
+ * through all T steps.  The entries of idx must be distinct and in [0, T*N): d(loss)/d(h_t) is scattered back to row idx[i],
+ * so there are no padding rows (unlike dppo_mlp_grad_minibatch) and a repeated row would lose a contribution.
+ * actions int32 [T*N]; old_log_probs / adv / returns f32 [T*N]; flat gradient -> grads, (policy, value, entropy, total) ->
+ * losses[0..3]. */
 int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* params, float* grads, const float* obs,
                             const unsigned char* prev_dones, const float* hx0, int T, int N, const int32_t* actions,
                             const float* old_log_probs, const float* adv, const float* returns, const double* adv_stats,

@@ -154,7 +154,19 @@ CONFIGS = [
     (64, 256, 3, True, 4096, 1501),
     (16, 128, 2, True, 2048, 1023),
     (16, 128, 1, False, 2048, 7),
+    # H = 512: head_train_kernel<16, 4, 1> / head_eval_kernel<16>, a 1024-row discrete minibatch and a Gaussian one
+    (32, 512, 4, False, 4096, 1024),
+    (6, 512, 9, True, 2048, 700),
+    # A = 32 (DPPO_MAX_ACT: every lane of the warp an action) with H not a multiple of 32; (A + 1) * H = 4950 needs 178 KB of
+    # shared memory in the head kernel, under its 200 KB bound
+    (10, 150, 32, False, 1000, 333),
+    (12, 40, 32, True, 700, 255),
 ]
+
+
+def f64(p):
+    """The oracle is dtype-generic: parameters (and inputs) in float64 make it a float64 reference."""
+    return {k: v.double() for k, v in p.items()}
 
 
 @pytest.mark.parametrize("D,H,A,cont,B,M", CONFIGS)
@@ -166,7 +178,8 @@ def test_mlp_forward_and_logprob(ctx, D, H, A, cont, B, M):
     fm = FlatMlp(D, H, A, cont)
     flat = fm.pack(p, device="cuda")
     obs = rng.standard_normal((B, D)).astype(np.float32)
-    ref_out, ref_v = O.mlp_forward(p, torch.as_tensor(obs), cont)
+    p64 = f64(p)
+    ref_out, ref_v = O.mlp_forward(p64, torch.as_tensor(obs).double(), cont)
     ws = torch.empty(ctx.mlp_workspace_bytes(fm.desc, 300, False) // 4, device="cuda")      # forces row chunking
     out = torch.empty(B, A, device="cuda"); val = torch.empty(B, device="cuda")
     ctx.mlp_forward(fm.desc, flat, dev(obs), B, 3, out, val, ws)
@@ -181,7 +194,7 @@ def test_mlp_forward_and_logprob(ctx, D, H, A, cont, B, M):
     if cont:
         act = rng.standard_normal((B, A)).astype(np.float32)
         ctx.logprob_gaussian(out, flat[fm.layout.log_std:fm.layout.log_std + A], dev(act), lp)
-        ref_lp = O.normal_log_prob(ref_out, p["actor_log_std"].expand_as(ref_out), torch.as_tensor(act))
+        ref_lp = O.normal_log_prob(ref_out, p64["actor_log_std"].expand_as(ref_out), torch.as_tensor(act).double())
     else:
         act = rng.integers(0, A, B)
         ctx.logprob_categorical(out, dev(act, torch.int32), lp)
@@ -215,9 +228,9 @@ def test_mlp_grad_minibatch_vs_oracle(ctx, D, H, A, cont, B, M):
     ret = rng.standard_normal(B).astype(np.float32)
     idx = rng.permutation(B)[:M].astype(np.int32)
     hyper, cfg = make_hyper(N, M)
-    t = torch.as_tensor
+    t = lambda a: torch.as_tensor(a).double() if a.dtype.kind == "f" else torch.as_tensor(a)
     sel = torch.as_tensor(idx.astype(np.int64))
-    losses_ref, g_ref = O.loss_and_grads(p, t(obs)[sel], t(act)[sel], t(old_lp)[sel], t(adv)[sel], t(ret)[sel], cfg, cont)
+    losses_ref, g_ref = O.loss_and_grads(f64(p), t(obs)[sel], t(act)[sel], t(old_lp)[sel], t(adv)[sel], t(ret)[sel], cfg, cont)
 
     grads = torch.full((fm.total,), 7.0, device="cuda")
     losses = torch.zeros(4, device="cuda")
@@ -237,6 +250,40 @@ def test_mlp_grad_minibatch_vs_oracle(ctx, D, H, A, cont, B, M):
     for n, (off, shape) in fm.slices.items():
         used[off:off + int(np.prod(shape))] = True
     assert float(grads.cpu()[~used].abs().sum()) == 0.0
+
+
+def test_head_shape_over_the_shared_memory_bound_is_refused(ctx):
+    """H = 512 with A = 12 needs (A + 1) * H floats of weights plus per-warp accumulators: over the head kernel's 200 KB of shared
+    memory.  The host-side check refuses the launch with NativeError (nothing runs in a broken state), and the context keeps
+    working: the next call with a valid shape computes the right gradient."""
+    from diamond import _native as N
+    from diamond.flat import FlatMlp
+    rng = np.random.default_rng(12)
+    for D, H, A, ok in ((8, 512, 12, False), (8, 512, 4, True)):
+        B = M = 256
+        p = rand_params(rng, O.DISCRETE_PARAM_NAMES, D, H, A, False)
+        fm = FlatMlp(D, H, A, False)
+        obs = rng.standard_normal((B, D)).astype(np.float32)
+        act = rng.integers(0, A, B)
+        old_lp, adv, ret = (rng.standard_normal(B).astype(np.float32) for _ in range(3))
+        hyper, cfg = make_hyper(N, M)
+        grads = torch.zeros(fm.total, device="cuda"); losses = torch.zeros(4, device="cuda")
+        ws = torch.empty(ctx.mlp_workspace_bytes(fm.desc, M, True) // 4 + 64, device="cuda")
+        args = (fm.desc, fm.pack(p, device="cuda"), grads, dev(obs), dev(act, torch.int32), dev(old_lp), dev(adv), dev(ret), None,
+                dev(np.arange(M), torch.int32), M, hyper, losses, ws)
+        if not ok:
+            with pytest.raises(N.NativeError, match="too large for shared memory"):
+                ctx.mlp_grad_minibatch(*args)
+            continue
+        ctx.mlp_grad_minibatch(*args)
+        torch.cuda.synchronize()
+        t = lambda a: torch.as_tensor(a).double() if a.dtype.kind == "f" else torch.as_tensor(a)
+        losses_ref, g_ref = O.loss_and_grads(f64(p), t(obs), t(act), t(old_lp), t(adv), t(ret), cfg, False)
+        np.testing.assert_allclose(losses.cpu().numpy(), [losses_ref[k] for k in ("policy", "value", "entropy", "total")],
+                                   rtol=1e-4, atol=1e-6)
+        gv = fm.views(grads)
+        for n in O.DISCRETE_PARAM_NAMES:
+            assert nerr(gv[n].cpu().numpy(), g_ref[n].numpy()) <= 2e-5, n
 
 
 def test_update_gradient_is_additive_over_samples_at_full_size(ctx):
