@@ -7,12 +7,18 @@
 // steps and keeps W_hh and the running hidden state on chip.
 //   Hg <= 32 (the default 16): one environment per Hg-lane group of a warp, this lane's three W_hh rows (forward) or columns
 //   (backward) in registers, the hidden vector exchanged with shuffles -- no block barrier inside the time loop;
-//   otherwise: W_hh in shared memory, hidden vectors double-buffered in shared memory, one barrier per step.
+//   Hg <= 128: W_hh in shared memory, hidden vectors double-buffered in shared memory, one barrier per step;
+//   128 < Hg <= 512: W_hh split by hidden unit over the CTAs of a thread-block cluster, hidden state exchanged over distributed
+//   shared memory, one cluster barrier per step.
 // GRU cell (torch nn.GRU, gate order r, z, n): r = s(gi_r + W_hr h + b_hr), z = s(gi_z + W_hz h + b_hz),
 // n = tanh(gi_n + r * (W_hn h + b_hn)), h' = (1 - z) * n + z * h, with h <- 0 where prev_dones[t] (recurrent_ppo.py:84).
+#include <cooperative_groups.h>
+
 #include "common.cuh"
 #include "heads.cuh"
 #include "optim.cuh"
+
+namespace cg = cooperative_groups;
 
 namespace {
 
@@ -454,6 +460,232 @@ gru_scan_bwd_tiled_kernel(ScanBwdArgs a, int G)
     }
 }
 
+// ---- cluster scans, 128 < Hg <= 512: W_hh spread over the C CTAs of a thread-block cluster ----------------------------------
+// 3 Hg^2 floats of W_hh no longer fit one SM (768 KB at Hg = 256).  CTA c of a cluster owns hidden units [c U, min(Hg, (c+1) U)),
+// U = ceil(Hg / C), and keeps the r, z, n rows of those units in shared memory (3U x Hg floats, ~100 KB at Hg = 256 with C = 8,
+// ~194 KB at Hg = 512 with C = 16).  Thread (group, j) handles unit j of the CTA for E environments; the cluster owns G * E
+// environments for all T steps, and clusters are independent of each other.
+//   forward: all-gather.  Each CTA writes the masked hidden values of its units into the hidden-vector buffer of every peer over
+//     distributed shared memory, double-buffered by the parity of t, so one cluster barrier per step orders the writes of step t
+//     before their reads and the reads of step t before the writes of step t + 2.  The products then run as in the tiled kernel
+//     (k ascending, one FMA chain per gate; rows padded to a multiple of 4 with zeros for LDS.128).
+//   backward: reduce-scatter over the same row slice (no transposed copy of W_hh).  CTA c forms the gate gradients of its units,
+//     the partial P_c[k] = sum over its 3U rows g (ascending) of dg[g] W_hh[g][k] for every k, and sends the slice k in units(c')
+//     to CTA c'.  After the barrier each CTA adds the C partials in rank order 0..C-1 (deterministic), then dh_direct, then the
+//     done cut.  Each environment moves Hg floats per step in each direction.
+// Every per-environment result is independent of E, G and the cluster an environment lands in.
+template <int E>
+__global__ void __launch_bounds__(256)
+gru_scan_fwd_cluster_kernel(ScanFwdArgs a, int G)
+{
+    extern __shared__ __align__(16) float smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int C = (int)cluster.num_blocks(), rank = (int)cluster.block_rank();
+    const int Hg = a.Hg, U = (Hg + C - 1) / C, HP = (Hg + 3) & ~3, WS = HP + 4;
+    const int u0 = rank * U, nu = max(0, min(U, Hg - u0));      // units of this CTA: [u0, u0 + nu)
+    float* w = smem;                                            // [3U][WS]: row q U + u = W_hh row q Hg + u0 + u, zero-padded
+    float* hb = w + 3 * U * WS;                                 // [2][G * E][HP] gathered masked hidden vectors (zero past Hg)
+    for (int i = threadIdx.x; i < 3 * U * WS; i += blockDim.x) {
+        const int g = i / WS, k = i % WS, q = g / U, u = g % U;
+        w[i] = (u < nu && k < Hg) ? a.whh[(int64_t)(q * Hg + u0 + u) * Hg + k] : 0.f;
+    }
+    for (int i = threadIdx.x; i < 2 * G * E * HP; i += blockDim.x) hb[i] = 0.f;
+    const int grp = threadIdx.x / U, j = threadIdx.x % U;
+    const bool unit = j < nu;
+    const int ju = u0 + (unit ? j : 0);                         // global hidden unit of this thread
+    const int64_t env0 = ((int64_t)(blockIdx.x / C) * G + grp) * E;
+    const float br = unit ? a.bhh[ju] : 0.f, bz = unit ? a.bhh[Hg + ju] : 0.f, bn = unit ? a.bhh[2 * Hg + ju] : 0.f;
+    const int64_t rs = (int64_t)a.N;
+    bool on[E];
+    int64_t e[E];
+    float h[E], gr[E], gz[E], gn[E];
+    unsigned char dn[E];
+#pragma unroll
+    for (int i = 0; i < E; ++i) {
+        on[i] = unit && env0 + i < a.N;
+        e[i] = env0 + i < a.N ? env0 + i : 0;
+        h[i] = (on[i] && a.hx0) ? a.hx0[e[i] * Hg + ju] : 0.f;
+        const float* g = a.gi + e[i] * 3 * Hg;
+        gr[i] = g[ju]; gz[i] = g[Hg + ju]; gn[i] = g[2 * Hg + ju];
+        dn[i] = a.dones ? a.dones[e[i]] : 0;
+    }
+    const float4* wr4 = reinterpret_cast<const float4*>(w + (size_t)j * WS);
+    const float4* wz4 = reinterpret_cast<const float4*>(w + (size_t)(U + j) * WS);
+    const float4* wn4 = reinterpret_cast<const float4*>(w + (size_t)(2 * U + j) * WS);
+    cluster.sync();                                             // every peer's buffers are initialised before the first remote write
+    for (int t = 0; t < a.T; ++t) {
+        float gr1[E], gz1[E], gn1[E];
+        unsigned char dn1[E];
+#pragma unroll
+        for (int i = 0; i < E; ++i) {
+            gr1[i] = gz1[i] = gn1[i] = 0.f; dn1[i] = 0;
+            if (t + 1 < a.T) {
+                const int64_t row1 = (int64_t)(t + 1) * rs + e[i];
+                const float* g1 = a.gi + row1 * 3 * Hg;
+                gr1[i] = g1[ju]; gz1[i] = g1[Hg + ju]; gn1[i] = g1[2 * Hg + ju];
+                if (a.dones) dn1[i] = a.dones[row1];
+            }
+        }
+        float* cur = hb + (size_t)(t & 1) * G * E * HP + (size_t)grp * E * HP;
+        float m[E], ar[E], az[E], an[E];
+#pragma unroll
+        for (int i = 0; i < E; ++i) { m[i] = dn[i] ? 0.f : h[i]; ar[i] = br; az[i] = bz; an[i] = bn; }   // recurrent_ppo.py:84
+        if (unit)
+            for (int q = 0; q < C; ++q) {
+                float* peer = cluster.map_shared_rank(cur, q);
+#pragma unroll
+                for (int i = 0; i < E; ++i) peer[i * HP + ju] = m[i];
+            }
+        cluster.sync();                                         // one barrier per step (arrive.release / wait.acquire)
+        for (int k4 = 0; k4 < HP / 4; ++k4) {
+            const float4 a_r = wr4[k4], a_z = wz4[k4], a_n = wn4[k4];
+#pragma unroll
+            for (int i = 0; i < E; ++i) {
+                const float4 hv = reinterpret_cast<const float4*>(cur + i * HP)[k4];
+                ar[i] = fmaf(a_r.x, hv.x, ar[i]); az[i] = fmaf(a_z.x, hv.x, az[i]); an[i] = fmaf(a_n.x, hv.x, an[i]);
+                ar[i] = fmaf(a_r.y, hv.y, ar[i]); az[i] = fmaf(a_z.y, hv.y, az[i]); an[i] = fmaf(a_n.y, hv.y, an[i]);
+                ar[i] = fmaf(a_r.z, hv.z, ar[i]); az[i] = fmaf(a_z.z, hv.z, az[i]); an[i] = fmaf(a_n.z, hv.z, an[i]);
+                ar[i] = fmaf(a_r.w, hv.w, ar[i]); az[i] = fmaf(a_z.w, hv.w, az[i]); an[i] = fmaf(a_n.w, hv.w, an[i]);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < E; ++i) {
+            const float r = sigmoidf_(gr[i] + ar[i]), z = sigmoidf_(gz[i] + az[i]);
+            const float n = tanhf(gn[i] + r * an[i]);
+            h[i] = (1.0f - z) * n + z * m[i];
+            if (on[i]) {
+                const int64_t row = (int64_t)t * rs + e[i];
+                a.hs[row * Hg + ju] = h[i];
+                if (a.hm) {
+                    a.hm[row * Hg + ju] = m[i];
+                    float* go = a.gates + row * 3 * Hg;
+                    go[ju] = r; go[Hg + ju] = z; go[2 * Hg + ju] = n;
+                    a.hn[row * Hg + ju] = an[i];
+                }
+            }
+            gr[i] = gr1[i]; gz[i] = gz1[i]; gn[i] = gn1[i]; dn[i] = dn1[i];
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < E; ++i)
+        if (on[i] && a.hx_out) a.hx_out[e[i] * Hg + ju] = h[i];
+    cluster.sync();                                             // no CTA exits while a peer may still access its shared memory
+}
+
+template <int C, int E>
+__global__ void __launch_bounds__(256)
+gru_scan_bwd_cluster_kernel(ScanBwdArgs a, int G)
+{
+    extern __shared__ __align__(16) float smem[];
+    cg::cluster_group cluster = cg::this_cluster();
+    const int rank = (int)cluster.block_rank();
+    const int Hg = a.Hg, U = (Hg + C - 1) / C, U3 = 3 * U;
+    const int u0 = rank * U, nu = max(0, min(U, Hg - u0));
+    float* w = smem;                                            // [3U][Hg]: row q U + u = W_hh row q Hg + u0 + u (zero for u >= nu)
+    float* dgb = w + (size_t)U3 * Hg;                           // [G * E][3U] this CTA's dr | dz | dghn of the current step
+    float* rb = dgb + (size_t)G * E * U3;                       // [2][G * E][C][U] partials received from each rank, by parity of t
+    for (int i = threadIdx.x; i < U3 * Hg; i += blockDim.x) {
+        const int g = i / Hg, k = i % Hg, q = g / U, u = g % U;
+        w[i] = u < nu ? a.whh[(int64_t)(q * Hg + u0 + u) * Hg + k] : 0.f;
+    }
+    const int grp = threadIdx.x / U, j = threadIdx.x % U;
+    const bool unit = j < nu;
+    const int ju = u0 + (unit ? j : 0);
+    const int64_t env0 = ((int64_t)(blockIdx.x / C) * G + grp) * E;
+    const int64_t rs = (int64_t)a.N;
+    bool on[E];
+    int64_t e[E];
+    float carry[E];
+#pragma unroll
+    for (int i = 0; i < E; ++i) { on[i] = unit && env0 + i < a.N; e[i] = env0 + i < a.N ? env0 + i : 0; carry[i] = 0.f; }
+    float sr = 0.f, sz = 0.f, sn = 0.f, sgn = 0.f;
+    cluster.sync();
+    for (int t = a.T - 1; t >= 0; --t) {
+        float direct[E];
+        bool dn[E];
+#pragma unroll
+        for (int i = 0; i < E; ++i) {
+            const int64_t row = (int64_t)t * rs + e[i];
+            dn[i] = a.dones && a.dones[row];
+            direct[i] = 0.f;
+            if (unit) {
+                const float* g = a.gates + row * 3 * Hg;
+                const float r = g[ju], z = g[Hg + ju], n = g[2 * Hg + ju];
+                const float hn = a.hn[row * Hg + ju], m = a.hm[row * Hg + ju];
+                const float dh = (on[i] ? a.dhs[row * Hg + ju] : 0.f) + carry[i];
+                const CellGrad c = gru_cell_grad(dh, r, z, n, hn, m);
+                float* d = dgb + (size_t)(grp * E + i) * U3;
+                d[j] = c.dr; d[U + j] = c.dz; d[2 * U + j] = c.dghn;
+                if (on[i]) {
+                    float* o = a.dgi + row * 3 * Hg;
+                    o[ju] = c.dr; o[Hg + ju] = c.dz; o[2 * Hg + ju] = c.dn;
+                    float* p = a.dgh + row * 3 * Hg;
+                    p[ju] = c.dr; p[Hg + ju] = c.dz; p[2 * Hg + ju] = c.dghn;
+                    sr += c.dr; sz += c.dz; sn += c.dn; sgn += c.dghn;
+                }
+                direct[i] = c.dh_direct;
+            }
+        }
+        __syncthreads();
+        // P_rank[k] for k = q U + j (unit j of rank q), sent to rank q; the C * E chains run side by side, each over g ascending
+        float* cur = rb + (size_t)(t & 1) * G * E * C * U;
+        float p[C][E];
+#pragma unroll
+        for (int q = 0; q < C; ++q)
+#pragma unroll
+            for (int i = 0; i < E; ++i) p[q][i] = 0.f;
+        for (int gate = 0; gate < 3; ++gate)
+            for (int u = 0; u < nu; ++u) {
+                const int g = gate * U + u;
+                float dv[E];
+#pragma unroll
+                for (int i = 0; i < E; ++i) dv[i] = dgb[(size_t)(grp * E + i) * U3 + g];
+                const float* wg = w + (size_t)g * Hg;
+#pragma unroll
+                for (int q = 0; q < C; ++q) {
+                    const float wv = wg[min(q * U + j, Hg - 1)];          // k >= Hg (past the last unit): computed, not sent
+#pragma unroll
+                    for (int i = 0; i < E; ++i) p[q][i] = fmaf(dv[i], wv, p[q][i]);
+                }
+            }
+#pragma unroll
+        for (int q = 0; q < C; ++q) {
+            if (q * U + j >= Hg) continue;
+            float* peer = cluster.map_shared_rank(cur, q);
+#pragma unroll
+            for (int i = 0; i < E; ++i) peer[((size_t)(grp * E + i) * C + rank) * U + j] = p[q][i];
+        }
+        cluster.sync();                                         // one barrier per step; also orders dgb's reads before its next writes
+#pragma unroll
+        for (int i = 0; i < E; ++i) {
+            float acc = 0.f;
+            if (unit) {
+                const float* in = cur + (size_t)(grp * E + i) * C * U + j;
+                acc = in[0];
+                for (int src = 1; src < C; ++src) acc += in[(size_t)src * U];
+                acc += direct[i];
+            }
+            carry[i] = dn[i] ? 0.f : acc;                       // hm = keep * h_{t-1}
+        }
+    }
+    __syncthreads();
+    // bias-gradient partial of this cluster (one part per cluster); this CTA writes the columns of its own units
+    float* red = rb;                                            // G * U * 4 <= 2 * G * E * C * U floats
+    red[threadIdx.x * 4 + 0] = sr; red[threadIdx.x * 4 + 1] = sz; red[threadIdx.x * 4 + 2] = sn; red[threadIdx.x * 4 + 3] = sgn;
+    __syncthreads();
+    if (threadIdx.x < nu) {
+        float s[4] = {0.f, 0.f, 0.f, 0.f};
+        for (int i = threadIdx.x; i < G * U; i += U)
+#pragma unroll
+            for (int q = 0; q < 4; ++q) s[q] += red[i * 4 + q];
+        float* o = a.bias_partials + (int64_t)(blockIdx.x / C) * 6 * Hg;
+        const int u = u0 + threadIdx.x;
+        o[u] = s[0]; o[Hg + u] = s[1]; o[2 * Hg + u] = s[2];
+        o[3 * Hg + u] = s[0]; o[4 * Hg + u] = s[1]; o[5 * Hg + u] = s[3];
+    }
+    cluster.sync();                                             // no CTA exits while a peer may still access its shared memory
+}
+
 // dst[idx[m], :] = src[m, :] (rows of a minibatch back to their place in the [T*N, C] sequence tensor; dst is zero elsewhere)
 __global__ void scatter_rows_kernel(const float* __restrict__ src, const int32_t* __restrict__ idx, float* __restrict__ dst,
                                     int64_t rows, int C)
@@ -486,16 +718,84 @@ int tiled_scan_groups(int N, int Hg, int E)
     return g < need ? g : need;
 }
 
+// cluster kernels (128 < Hg <= 512): C CTAs per cluster, U units per CTA, G groups of E environments per cluster
+constexpr int kScanSmemFloats = 227 * 1024 / 4;                // dynamic shared memory of one B200 block
+constexpr int kClusterMaxGroups = 8;                            // <= 8 * 32 = 256 threads per CTA
+struct ClusterPlan { int C, U, E, G, clusters; };
+bool cluster_scan_ok(int Hg) { return Hg > 128 && Hg <= 512; }
+int64_t cluster_fwd_smem_floats(int Hg, int C, int envs)
+{
+    const int U = (Hg + C - 1) / C, HP = (Hg + 3) & ~3;
+    return (int64_t)3 * U * (HP + 4) + (int64_t)2 * envs * HP;
+}
+int64_t cluster_bwd_smem_floats(int Hg, int C, int envs)
+{
+    const int U = (Hg + C - 1) / C;
+    return (int64_t)3 * U * Hg + (int64_t)envs * (3 * U + 2 * C * U);
+}
+// Environments per cluster: enough to cover N with one wave of clusters (148 / C of them), spread thinly at small N as the tiled
+// kernels do, and at most what the shared memory left after the weight slice holds (8 at Hg = 512).  E > 1 once a cluster
+// holds more than kClusterMaxGroups environments: every W_hh value read from shared memory then serves E environments.
+ClusterPlan cluster_plan(int N, int Hg)
+{
+    ClusterPlan p;
+    p.C = Hg <= 256 ? 8 : 16;
+    p.U = (Hg + p.C - 1) / p.C;
+    int cap = 1;
+    while (cluster_fwd_smem_floats(Hg, p.C, cap + 1) <= kScanSmemFloats && cluster_bwd_smem_floats(Hg, p.C, cap + 1) <= kScanSmemFloats)
+        ++cap;
+    const int slots = 148 / p.C;
+    const int want = (int)(((int64_t)N + slots - 1) / slots);
+    int ec = want < cap ? want : cap;
+    if (ec > 4 * kClusterMaxGroups) ec = 4 * kClusterMaxGroups;
+    p.E = ec <= kClusterMaxGroups ? 1 : ec <= 2 * kClusterMaxGroups ? 2 : 4;
+    p.G = (ec + p.E - 1) / p.E;
+    while (p.G > 1 && p.G * p.E > cap) --p.G;
+    p.clusters = (int)(((int64_t)N + p.G * p.E - 1) / (p.G * p.E));
+    return p;
+}
+
 int scan_blocks(int N, int Hg)
 {
+    if (cluster_scan_ok(Hg)) return cluster_plan(N, Hg).clusters;   // bias partials: one part per cluster
     if (warp_scan_ok(Hg)) return (int)(((int64_t)N * Hg + 127) / 128);
     if (tiled_scan_ok(Hg)) { const int E = tiled_scan_E(N, Hg), per = tiled_scan_groups(N, Hg, E) * E; return (N + per - 1) / per; }
     const int eb = smem_scan_envs(Hg);
     return (N + eb - 1) / eb;
 }
 
+// grid of p.clusters clusters of p.C CTAs; refuses (instead of launching) when no such cluster fits on the device
+template <typename Args>
+int launch_cluster_scan(dppo_ctx* ctx, void (*kern)(Args, int), const Args& a, const ClusterPlan& p, size_t smem, cudaStream_t st,
+                        const char* what)
+{
+    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess ||
+        (p.C > 8 && cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) != cudaSuccess))
+        DPPO_FAIL(ctx, "%s: cudaFuncSetAttribute failed (%s)", what, cudaGetErrorString(cudaGetLastError()));
+    cudaLaunchConfig_t lc = {};
+    lc.gridDim = dim3((unsigned)p.clusters * p.C); lc.blockDim = dim3(p.G * p.U); lc.dynamicSmemBytes = smem; lc.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = p.C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    lc.attrs = attr; lc.numAttrs = 1;
+    int active = 0;
+    if (cudaOccupancyMaxActiveClusters(&active, kern, &lc) != cudaSuccess || active < 1)
+        DPPO_FAIL(ctx, "%s: no %d-CTA cluster with %zu bytes of shared memory per CTA fits on this device (%s)", what, p.C, smem,
+                  cudaGetErrorString(cudaGetLastError()));
+    cudaLaunchKernelEx(&lc, kern, a, p.G);
+    DPPO_CHECK_LAUNCH(ctx, what);
+    return 0;
+}
+
 int launch_scan_fwd(dppo_ctx* ctx, const ScanFwdArgs& a, cudaStream_t st)
 {
+    if (cluster_scan_ok(a.Hg)) {
+        const ClusterPlan p = cluster_plan(a.N, a.Hg);
+        const size_t smem = (size_t)cluster_fwd_smem_floats(a.Hg, p.C, p.G * p.E) * sizeof(float);
+        if (p.E == 4) return launch_cluster_scan(ctx, gru_scan_fwd_cluster_kernel<4>, a, p, smem, st, "gru_scan_fwd_cluster_kernel");
+        if (p.E == 2) return launch_cluster_scan(ctx, gru_scan_fwd_cluster_kernel<2>, a, p, smem, st, "gru_scan_fwd_cluster_kernel");
+        return launch_cluster_scan(ctx, gru_scan_fwd_cluster_kernel<1>, a, p, smem, st, "gru_scan_fwd_cluster_kernel");
+    }
     const int blocks = scan_blocks(a.N, a.Hg);
     if (a.Hg == 8) gru_scan_fwd_warp_kernel<8><<<blocks, 128, 0, st>>>(a);
     else if (a.Hg == 16) gru_scan_fwd_warp_kernel<16><<<blocks, 128, 0, st>>>(a);
@@ -524,6 +824,14 @@ int launch_scan_fwd(dppo_ctx* ctx, const ScanFwdArgs& a, cudaStream_t st)
 
 int launch_scan_bwd(dppo_ctx* ctx, const ScanBwdArgs& a, cudaStream_t st)
 {
+    if (cluster_scan_ok(a.Hg)) {
+        const ClusterPlan p = cluster_plan(a.N, a.Hg);
+        const size_t smem = (size_t)cluster_bwd_smem_floats(a.Hg, p.C, p.G * p.E) * sizeof(float);
+#define SCAN_BWD(C_, E_) return launch_cluster_scan(ctx, gru_scan_bwd_cluster_kernel<C_, E_>, a, p, smem, st, "gru_scan_bwd_cluster_kernel")
+        if (p.C == 8) { if (p.E == 4) SCAN_BWD(8, 4); if (p.E == 2) SCAN_BWD(8, 2); SCAN_BWD(8, 1); }
+        if (p.E == 4) SCAN_BWD(16, 4); if (p.E == 2) SCAN_BWD(16, 2); SCAN_BWD(16, 1);
+#undef SCAN_BWD
+    }
     const int blocks = scan_blocks(a.N, a.Hg);
     if (a.Hg == 8) gru_scan_bwd_warp_kernel<8><<<blocks, 128, 0, st>>>(a);
     else if (a.Hg == 16) gru_scan_bwd_warp_kernel<16><<<blocks, 128, 0, st>>>(a);
@@ -553,7 +861,7 @@ int launch_scan_bwd(dppo_ctx* ctx, const ScanBwdArgs& a, cudaStream_t st)
 int check_desc(dppo_ctx* ctx, const dppo_rnn_desc* d)
 {
     if (!d || d->obs_dim < 1 || d->hidden < 1 || d->gru_hidden < 1 || d->act_dim < 1) DPPO_FAIL(ctx, "rnn: bad descriptor");
-    if (d->gru_hidden > 128) DPPO_FAIL(ctx, "rnn: gru_hidden_dim %d > 128 is not supported", d->gru_hidden);
+    if (d->gru_hidden > 512) DPPO_FAIL(ctx, "rnn: gru_hidden_dim %d > 512 is not supported", d->gru_hidden);
     if (d->hidden > 512) DPPO_FAIL(ctx, "rnn: network_hidden_dim %d > 512 is not supported", d->hidden);
     if (d->act_dim > DPPO_MAX_ACT) DPPO_FAIL(ctx, "rnn: more than %d actions", DPPO_MAX_ACT);
     return 0;

@@ -277,7 +277,7 @@ int64_t dppo_ppo_loss_workspace_bytes(int64_t M, int A);
 typedef struct dppo_rnn_desc {
     int32_t obs_dim;      /* D */
     int32_t hidden;       /* H  = cfg.network_hidden_dim */
-    int32_t gru_hidden;   /* Hg = cfg.gru_hidden_dim (<= 128) */
+    int32_t gru_hidden;   /* Hg = cfg.gru_hidden_dim (<= 512; 129-512 run on thread-block-cluster scans) */
     int32_t act_dim;      /* A  = Discrete.n */
 } dppo_rnn_desc;
 /* Offsets (floats, multiples of 4) in the flat parameter / gradient / Adam buffers; the GRU tensors are nn.GRU's
