@@ -145,15 +145,18 @@ WImages carve_images(const dppo_mlp_desc* d, char* base)
 struct TrainWs {
     float *h1, *h2, *h3, *d3, *d2, *d1, *xg;
     float *p3, *p2, *p1, *c2, *c1, *hp;
-    int s3, s2, s1, tiles2, tiles1, head_blocks, head_stride;
+    int s3, s2, s1, tiles2, tiles1, head_blocks, head_stride;   // head_*: per-CTA partials of the head kernel (GEMM heads: of wide_loss_kernel)
     int t3, t2, t1;          // split counts of the tcgen05 weight-gradient kernels (0: shape unsupported)
     bool multi;              // the three weight gradients run as one balanced launch (t3/t2/t1 then come from the joint plan)
+    float *zd, *pa, *ca;     // GEMM heads: head outputs, overwritten by d(loss)/dz [M, A] | dWa split-K partials | actor db3 column sums
+    int sa, tiles_a;
     int64_t img_off;
     int64_t bytes;
 };
 
-// Carves the training workspace for M rows.  sm_count fixes the split-K / head grid sizes.
-TrainWs carve_train(const dppo_mlp_desc* d, int64_t M, int sm_count, char* base)
+// Carves the training workspace for M rows.  sm_count fixes the split-K / head grid sizes.  gemm_heads: the head stage of
+// dppo_mlp_grad_minibatch_gemm_heads (its partials are O(A + H) per CTA instead of the head kernel's O(A * H)).
+TrainWs carve_train(const dppo_mlp_desc* d, int64_t M, int sm_count, char* base, bool gemm_heads = false)
 {
     dppo_ctx fake = {}; fake.sm_count = sm_count;
     const int64_t D = d->obs_dim, H = d->hidden, A = d->act_dim;
@@ -185,8 +188,20 @@ TrainWs carve_train(const dppo_mlp_desc* d, int64_t M, int sm_count, char* base)
     const int cparts = mx(dppo_tc3_colsum_rows(&fake, M, (int)H), w.tiles2);
     w.c2 = take((int64_t)cparts * H);
     w.c1 = take((int64_t)cparts * H);
-    w.head_blocks = head_train_blocks(&fake, M, (int)H, (int)A);
-    w.head_stride = (int)align_up(head_partial_floats((int)H, (int)A), 4);
+    w.zd = w.pa = w.ca = nullptr;
+    w.sa = w.tiles_a = 0;
+    if (gemm_heads) {
+        w.zd = take(M * A);
+        w.sa = dppo_wgrad_splits(&fake, M, (int)A, (int)H);
+        w.pa = take((int64_t)w.sa * A * H);
+        w.tiles_a = dppo_gemm_row_tiles(M, (int)H);
+        w.ca = take((int64_t)w.tiles_a * H);
+        w.head_blocks = wide_loss_blocks(&fake, M, (int)H, (int)A);
+        w.head_stride = wide_offsets((int)H, (int)A).total;
+    } else {
+        w.head_blocks = head_train_blocks(&fake, M, (int)H, (int)A);
+        w.head_stride = (int)align_up(head_partial_floats((int)H, (int)A), 4);
+    }
     w.hp = take((int64_t)w.head_blocks * w.head_stride);
     o = align_up(o, 1024);
     w.img_off = o;
@@ -215,6 +230,24 @@ extern "C" int64_t dppo_mlp_workspace_bytes(const dppo_mlp_desc* d, int64_t rows
     int sms = current_sm_count();
     if (sms < 148) sms = 148;
     return carve_train(d, rows, sms, nullptr).bytes;
+}
+
+extern "C" int dppo_mlp_fused_heads_supported(const dppo_mlp_desc* d)
+{
+    return d && head_train_supported(d->hidden, d->act_dim) ? 1 : 0;
+}
+
+static bool gemm_heads_in_bound(const dppo_mlp_desc* d)
+{
+    return d->hidden >= 1 && d->hidden <= DPPO_GEMM_HEADS_MAX_HIDDEN && d->act_dim >= 1 && d->act_dim <= DPPO_GEMM_HEADS_MAX_ACT;
+}
+
+extern "C" int64_t dppo_mlp_gemm_heads_workspace_bytes(const dppo_mlp_desc* d, int64_t rows)
+{
+    if (!d || rows <= 0 || d->obs_dim < 1 || !gemm_heads_in_bound(d)) return 0;
+    int sms = current_sm_count();
+    if (sms < 148) sms = 148;
+    return carve_train(d, rows, sms, nullptr, true).bytes;
 }
 
 extern "C" int dppo_mlp_forward(dppo_ctx* ctx, const dppo_mlp_desc* d, const float* params, const float* obs,
@@ -291,27 +324,33 @@ extern "C" int dppo_mlp_forward(dppo_ctx* ctx, const dppo_mlp_desc* d, const flo
         } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, h2, H, nullptr, params + L.w3 + w3off, H, params + L.b3 + b3off, h3, n3, n, n3, H, st)) return 1;
         const float* ha = actor ? h3 : nullptr;
         const float* hc = critic ? (actor ? h3 + H : h3) : nullptr;
-        if (launch_head_eval(ctx, ha, hc, n3, params + L.wa, params + L.ba, params + L.wc, params + L.bc,
-                             head_out ? head_out + r0 * A : nullptr, values ? values + r0 : nullptr, n, H, A, (sweep >> 1) & 1, st)) return 1;
+        if (launch_heads_forward(ctx, ha, hc, n3, params + L.wa, params + L.ba, params + L.wc, params + L.bc,
+                                 head_out ? head_out + r0 * A : nullptr, values ? values + r0 : nullptr, n, H, A, (sweep >> 1) & 1, st)) return 1;
     }
     return 0;
 }
 
-extern "C" int dppo_mlp_grad_minibatch(dppo_ctx* ctx, const dppo_mlp_desc* d, const float* params, float* grads,
-                                       const float* obs, const void* actions, const float* old_log_probs, const float* adv,
-                                       const float* returns, const double* adv_stats, const int32_t* idx, int64_t M,
-                                       const dppo_hyper* hy, float* losses, void* ws, int64_t ws_bytes, void* stream)
+// One minibatch gradient (ppo.py:258-283).  The trunk (gather, forward GEMMs, dgrad chain, weight gradients, gradient assembly) is
+// shared; gemm_heads selects the head stage: the fused head kernel (head_train_kernel, A <= 32 and (A+1) H within its shared
+// memory) or GEMM heads (actor products and head weight gradients as GEMMs around wide_loss_kernel).
+static int mlp_grad_minibatch_impl(dppo_ctx* ctx, const char* what, bool gemm_heads, const dppo_mlp_desc* d, const float* params,
+                                   float* grads, const float* obs, const void* actions, const float* old_log_probs, const float* adv,
+                                   const float* returns, const double* adv_stats, const int32_t* idx, int64_t M, const dppo_hyper* hy,
+                                   float* losses, void* ws, int64_t ws_bytes, void* stream)
 {
     if (!ctx) return 1;
     if (!d || !params || !grads || !obs || !actions || !old_log_probs || !adv || !returns || !hy || !ws)
-        DPPO_FAIL(ctx, "mlp_grad_minibatch: null argument");
-    if (M <= 0) DPPO_FAIL(ctx, "mlp_grad_minibatch: empty minibatch");
-    if (hy->advantage_norm && (!adv_stats || hy->adv_count < 2)) DPPO_FAIL(ctx, "mlp_grad_minibatch: advantage_norm needs adv_stats and adv_count >= 2");
+        DPPO_FAIL(ctx, "%s: null argument", what);
+    if (M <= 0) DPPO_FAIL(ctx, "%s: empty minibatch", what);
+    if (hy->advantage_norm && (!adv_stats || hy->adv_count < 2)) DPPO_FAIL(ctx, "%s: advantage_norm needs adv_stats and adv_count >= 2", what);
     dppo_mlp_layout L;
-    if (dppo_mlp_layout_compute(d, &L)) DPPO_FAIL(ctx, "mlp_grad_minibatch: bad descriptor");
+    if (dppo_mlp_layout_compute(d, &L)) DPPO_FAIL(ctx, "%s: bad descriptor", what);
+    if (gemm_heads && !gemm_heads_in_bound(d))
+        DPPO_FAIL(ctx, "%s: hidden %d / %d actions outside the GEMM-head bound (hidden <= %d, 1..%d actions)", what, d->hidden, d->act_dim,
+                  DPPO_GEMM_HEADS_MAX_HIDDEN, DPPO_GEMM_HEADS_MAX_ACT);
     const int D = d->obs_dim, H = d->hidden, A = d->act_dim;
-    TrainWs w = carve_train(d, M, ctx->sm_count, (char*)ws);
-    if (w.bytes > ws_bytes) DPPO_FAIL(ctx, "mlp_grad_minibatch: workspace too small (%lld < %lld)", (long long)ws_bytes, (long long)w.bytes);
+    TrainWs w = carve_train(d, M, ctx->sm_count, (char*)ws, gemm_heads);
+    if (w.bytes > ws_bytes) DPPO_FAIL(ctx, "%s: workspace too small (%lld < %lld)", what, (long long)ws_bytes, (long long)w.bytes);
     cudaStream_t st = (cudaStream_t)stream;
     const float inv_m = 1.0f / (float)(hy->loss_denominator > 0 ? hy->loss_denominator : M);
 
@@ -367,20 +406,42 @@ extern "C" int dppo_mlp_grad_minibatch(dppo_ctx* ctx, const dppo_mlp_desc* d, co
     } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, nullptr, params + L.w3, H, params + L.b3, w.h3, 2 * H, M, 2 * H, H, st)) return 1;
 
     // heads + loss (ppo.py:264-280) + backward into the first head layers
-    HeadTrainArgs ha;
-    ha.h3 = w.h3; ha.d3 = w.d3;
-    ha.wa = params + L.wa; ha.ba = params + L.ba; ha.wc = params + L.wc; ha.bc = params + L.bc;
-    ha.log_std = d->continuous ? params + L.log_std : nullptr;
-    ha.idx = idx;
-    ha.actions_i = d->continuous ? nullptr : (const int32_t*)actions;
-    ha.actions_f = d->continuous ? (const float*)actions : nullptr;
-    ha.old_logp = old_log_probs; ha.adv = adv; ha.ret = returns;
-    ha.adv_stats = adv_stats; ha.adv_count = hy->adv_count; ha.advantage_norm = hy->advantage_norm;
-    ha.M = M; ha.H = H; ha.A = A;
-    ha.clip = hy->ppo_clip; ha.vw = hy->value_loss_weight; ha.beta = hy->entropy_beta; ha.inv_m = inv_m;
-    ha.partials = w.hp; ha.partial_stride = w.head_stride;
-    ha.rev = (sweep >> 1) & 1; ha.keep_d3 = (sweep >> 2) & 1; ha.h3_first = (sweep >> 3) & 1;
-    if (launch_head_train_kernel(ctx, ha, d->continuous, w.head_blocks, st)) return 1;
+    if (!gemm_heads) {
+        HeadTrainArgs ha;
+        ha.h3 = w.h3; ha.d3 = w.d3;
+        ha.wa = params + L.wa; ha.ba = params + L.ba; ha.wc = params + L.wc; ha.bc = params + L.bc;
+        ha.log_std = d->continuous ? params + L.log_std : nullptr;
+        ha.idx = idx;
+        ha.actions_i = d->continuous ? nullptr : (const int32_t*)actions;
+        ha.actions_f = d->continuous ? (const float*)actions : nullptr;
+        ha.old_logp = old_log_probs; ha.adv = adv; ha.ret = returns;
+        ha.adv_stats = adv_stats; ha.adv_count = hy->adv_count; ha.advantage_norm = hy->advantage_norm;
+        ha.M = M; ha.H = H; ha.A = A;
+        ha.clip = hy->ppo_clip; ha.vw = hy->value_loss_weight; ha.beta = hy->entropy_beta; ha.inv_m = inv_m;
+        ha.partials = w.hp; ha.partial_stride = w.head_stride;
+        ha.rev = (sweep >> 1) & 1; ha.keep_d3 = (sweep >> 2) & 1; ha.h3_first = (sweep >> 3) & 1;
+        if (launch_head_train_kernel(ctx, ha, d->continuous, w.head_blocks, st)) return 1;
+    } else {
+        // z = h3a Wa^T + ba (ppo.py:63-71)
+        if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS, w.h3, 2 * H, nullptr, params + L.wa, H, params + L.ba, w.zd, A, M, A, H, st)) return 1;
+        // distribution + loss -> dz (in place), critic head -> d3[:, H:], small per-CTA partials
+        WideLossArgs la = {};
+        la.z = w.zd; la.dz = w.zd;
+        la.log_std = d->continuous ? params + L.log_std : nullptr;
+        la.h3 = w.h3; la.d3 = w.d3; la.wc = params + L.wc; la.bc = params + L.bc;
+        la.idx = idx;
+        la.actions_i = d->continuous ? nullptr : (const int32_t*)actions;
+        la.actions_f = d->continuous ? (const float*)actions : nullptr;
+        la.old_logp = old_log_probs; la.adv = adv; la.ret = returns;
+        la.adv_stats = adv_stats; la.adv_count = hy->adv_count; la.advantage_norm = hy->advantage_norm;
+        la.M = M; la.H = H; la.A = A;
+        la.clip = hy->ppo_clip; la.vw = hy->value_loss_weight; la.beta = hy->entropy_beta; la.inv_m = inv_m;
+        la.partials = w.hp; la.partial_stride = w.head_stride;
+        if (launch_wide_loss_train(ctx, la, d->continuous, w.head_blocks, st)) return 1;
+        // d3[:, :H] = (dz Wa) .* (1 - h3a^2) with the actor db3 column sums; dWa = dz^T h3a as split-K partials
+        if (dppo_gemm_nn_tanh_bwd(ctx, w.zd, A, params + L.wa, H, w.h3, 2 * H, w.d3, 2 * H, w.ca, M, H, A, st)) return 1;
+        if (dppo_wgrad(ctx, w.zd, A, w.h3, 2 * H, nullptr, w.pa, w.sa, M, A, H, st)) return 1;
+    }
 
     // backward (ppo.py:283): dgrad chain with the tanh' factors and bias-gradient column sums fused
     int tiles2 = w.tiles2, tiles1 = w.tiles1;
@@ -424,10 +485,19 @@ extern "C" int dppo_mlp_grad_minibatch(dppo_ctx* ctx, const dppo_mlp_desc* d, co
     seg(L.w2, (int64_t)H * H, w.p2, (int64_t)H * H, n2p);
     seg(L.b2, H, w.c2, H, tiles2);
     seg(L.w3, (int64_t)2 * H * H, w.p3, (int64_t)2 * H * H, n3p);
-    const HeadOffsets ho = head_offsets(H, A);
-    const int off_dba = ho.dba, off_dwc = ho.dwc, off_dbc = ho.dbc, off_dls = ho.dls, off_b3 = ho.b3, off_loss = ho.loss;
-    seg(L.b3, 2 * H, w.hp + off_b3, w.head_stride, w.head_blocks);
-    seg(L.wa, (int64_t)A * H, w.hp, w.head_stride, w.head_blocks);
+    int off_dba, off_dwc, off_dbc, off_dls, off_loss;
+    if (!gemm_heads) {
+        const HeadOffsets ho = head_offsets(H, A);
+        off_dba = ho.dba; off_dwc = ho.dwc; off_dbc = ho.dbc; off_dls = ho.dls; off_loss = ho.loss;
+        seg(L.b3, 2 * H, w.hp + ho.b3, w.head_stride, w.head_blocks);
+        seg(L.wa, (int64_t)A * H, w.hp, w.head_stride, w.head_blocks);
+    } else {
+        const WideOffsets wo = wide_offsets(H, A);
+        off_dba = wo.dba; off_dwc = wo.dwc; off_dbc = wo.dbc; off_dls = wo.dls; off_loss = 0;
+        seg(L.b3, H, w.ca, H, w.tiles_a);                                   // actor half: column sums of the dgrad GEMM
+        seg(L.b3 + H, H, w.hp + wo.db3, w.head_stride, w.head_blocks);      // critic half: wide_loss_kernel
+        seg(L.wa, (int64_t)A * H, w.pa, (int64_t)A * H, w.sa);
+    }
     seg(L.ba, A, w.hp + off_dba, w.head_stride, w.head_blocks);
     seg(L.wc, H, w.hp + off_dwc, w.head_stride, w.head_blocks);
     seg(L.bc, 1, w.hp + off_dbc, w.head_stride, w.head_blocks);
@@ -435,6 +505,24 @@ extern "C" int dppo_mlp_grad_minibatch(dppo_ctx* ctx, const dppo_mlp_desc* d, co
     tab.nseg = n;
     return launch_grad_reduce(ctx, tab, grads, L.total, w.hp + off_loss, w.head_blocks, w.head_stride, hy->value_loss_weight,
                               hy->entropy_beta, inv_m, losses, hy->grad_sumsq, st);
+}
+
+extern "C" int dppo_mlp_grad_minibatch(dppo_ctx* ctx, const dppo_mlp_desc* d, const float* params, float* grads,
+                                       const float* obs, const void* actions, const float* old_log_probs, const float* adv,
+                                       const float* returns, const double* adv_stats, const int32_t* idx, int64_t M,
+                                       const dppo_hyper* hy, float* losses, void* ws, int64_t ws_bytes, void* stream)
+{
+    return mlp_grad_minibatch_impl(ctx, "mlp_grad_minibatch", false, d, params, grads, obs, actions, old_log_probs, adv, returns,
+                                   adv_stats, idx, M, hy, losses, ws, ws_bytes, stream);
+}
+
+extern "C" int dppo_mlp_grad_minibatch_gemm_heads(dppo_ctx* ctx, const dppo_mlp_desc* d, const float* params, float* grads,
+                                                  const float* obs, const void* actions, const float* old_log_probs, const float* adv,
+                                                  const float* returns, const double* adv_stats, const int32_t* idx, int64_t M,
+                                                  const dppo_hyper* hy, float* losses, void* ws, int64_t ws_bytes, void* stream)
+{
+    return mlp_grad_minibatch_impl(ctx, "mlp_grad_minibatch_gemm_heads", true, d, params, grads, obs, actions, old_log_probs, adv,
+                                   returns, adv_stats, idx, M, hy, losses, ws, ws_bytes, stream);
 }
 
 // ---- V(final observation) only where it is needed (SURVEY.md 8f-2), shapes decided on the device --------------------
@@ -547,8 +635,8 @@ extern "C" int dppo_mlp_next_values(dppo_ctx* ctx, const dppo_mlp_desc* d, const
                       : dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, nullptr, params + L.w2, H, params + L.b2, w.h2, H, B, H, H, st);
     if (!rc) rc = tc2 ? dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, img.w3f, params + L.b3 + H, nullptr, 0, w.h3, H, nullptr, B, H, H, 0, st)
                       : dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, nullptr, params + L.w3 + (int64_t)H * H, H, params + L.b3 + H, w.h3, H, B, H, H, st);
-    if (!rc) rc = launch_head_eval(ctx, nullptr, w.h3, H, params + L.wa, params + L.ba, params + L.wc, params + L.bc, nullptr, w.tmp, B, H,
-                                   d->act_dim, 0, st);
+    if (!rc) rc = launch_heads_forward(ctx, nullptr, w.h3, H, params + L.wa, params + L.ba, params + L.wc, params + L.bc, nullptr, w.tmp, B, H,
+                                       d->act_dim, 0, st);
     ctx->rows_dev = nullptr;
     if (rc) return 1;
     scatter_values_kernel<<<blocks, 256, 0, st>>>(w.tmp, w.idx, w.count, next_values);

@@ -930,6 +930,190 @@ __global__ void loss_finalize_kernel(const float* __restrict__ partials, int npa
     }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Wide heads (any A, any H up to the GEMM-head bound).  One warp per row; lane l handles actions l, l+32, ... and critic
+// columns l, l+32, ...  The row's logits / means are read in passes (max, sum of exponentials, entropy, gradient), every one a
+// lane-strided sum in a fixed order followed by the fixed shuffle tree of warp_sum, so the result does not depend on the launch.
+// Same per-element formulas as eval_dist / loss_rows_kernel / head_train_kernel.
+// TRAIN: rows are gathered through idx (idx < 0: padding row, contributes nothing), advantages normalised from adv_stats, and
+// the critic head of the row is evaluated from h3 (v = h3c.wc + bc, d3c = dv wc (1 - h3c^2)).  Per-warp accumulators
+// [dba A | dlog_std A | dWc H | db3 H] live in shared memory (one lane per entry: no atomics) and are summed over the warps in
+// fixed order into one partial per CTA.  Standalone (custom network_cls): rows already gathered, values given, accumulator
+// [dlog_std A] only.
+// ---------------------------------------------------------------------------------------------
+template <bool CONT, bool TRAIN>
+__global__ void __launch_bounds__(256, 1)
+wide_loss_kernel(const WideLossArgs a)
+{
+    extern __shared__ float smem[];
+    const int A = a.A, H = TRAIN ? a.H : 0;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    const int wf = TRAIN ? 2 * (A + H) : A;
+    float* s_wc = smem;                                          // [H]
+    float* acc = smem + H + (size_t)warp * wf;
+    float* s_small = smem + H + (size_t)nw * wf;                 // [nw][4]: policy, value, entropy, dbc
+    float* acc_dba = acc;
+    float* acc_dls = TRAIN ? acc + A : acc;
+    float* acc_dwc = acc + 2 * A;
+    float* acc_db3 = acc + 2 * A + H;
+    DPPO_PDL_ENTER();
+    for (int i = threadIdx.x; i < H; i += blockDim.x) s_wc[i] = a.wc[i];
+    for (int i = lane; i < wf; i += 32) acc[i] = 0.f;
+    __syncthreads();
+
+    float mean = 0.f, denom = 1.f;
+    if (TRAIN) adv_norm_consts(a.adv_stats, a.adv_count, a.advantage_norm, mean, denom);
+    const float bias_c = TRAIN ? a.bc[0] : 0.f;
+    const float ent_scale = a.beta * a.inv_m;
+    float l_pol = 0.f, l_val = 0.f, l_ent = 0.f, s_dbc = 0.f;
+    for (int64_t m = (int64_t)blockIdx.x * nw + warp; m < a.M; m += (int64_t)gridDim.x * nw) {
+        int64_t src = m;
+        bool live = true;
+        if (TRAIN) {
+            const int64_t s = a.idx ? (int64_t)__ldg(a.idx + m) : m;
+            live = s >= 0;
+            src = live ? s : 0;
+        }
+        const float* z = a.z + m * A;                            // plain loads: dz may alias z
+        const float* ls = CONT ? (a.ls_stride ? a.log_std + m * a.ls_stride : a.log_std) : nullptr;
+        const float* act_f = CONT ? a.actions_f + src * A : nullptr;
+        const float old_lp = __ldg(a.old_logp + src);
+        const float advv = (__ldg(a.adv + src) - mean) / denom;
+        float new_lp, entropy, lse = 0.f;
+        int act = 0;
+        if (!CONT) {
+            // torch/distributions/categorical.py:78 (logits - logsumexp), :151-163 (log_prob, entropy)
+            act = __ldg(a.actions_i + src);
+            float mx = -CUDART_INF_F;
+            for (int j = lane; j < A; j += 32) mx = fmaxf(mx, z[j]);
+            mx = warp_max(mx);
+            float s = 0.f;
+            for (int j = lane; j < A; j += 32) s += expf(z[j] - mx);
+            lse = mx + logf(warp_sum(s));
+            float en = 0.f;
+            for (int j = lane; j < A; j += 32) { const float lsm = z[j] - lse; en += expf(lsm) * lsm; }
+            entropy = -warp_sum(en);
+            new_lp = z[act] - lse;
+        } else {
+            // torch/distributions/normal.py:87-102, :114-115, summed over dims (continuous_ppo.py:40-47)
+            float lp = 0.f, en = 0.f;
+            for (int j = lane; j < A; j += 32) {
+                const float sigma = expf(ls[j]);
+                const float log_scale = logf(sigma);
+                const float diff = __ldg(act_f + j) - z[j];
+                lp += -(diff * diff) / (2.0f * (sigma * sigma)) - log_scale - 0.91893853320467274178f;
+                en += 0.5f + 0.91893853320467274178f + log_scale;
+            }
+            new_lp = warp_sum(lp);
+            entropy = warp_sum(en);
+        }
+        const RowTerms t = policy_terms(new_lp, old_lp, advv, a.clip, a.inv_m);
+        float* dz = a.dz + m * A;
+        for (int j = lane; j < A; j += 32) {
+            float g = 0.f;
+            if (!CONT) {
+                const float lsm = z[j] - lse, p = expf(lsm);
+                if (live) g = t.dlogp * ((j == act ? 1.0f : 0.0f) - p) + ent_scale * p * (lsm + entropy);
+            } else if (live) {
+                const float sigma = expf(ls[j]);
+                const float var = sigma * sigma;
+                const float diff = __ldg(act_f + j) - z[j];
+                g = t.dlogp * diff / var;
+                const float dls = t.dlogp * (diff * diff / var - 1.0f) - ent_scale;
+                if (a.ls_stride) a.dls_rows[m * A + j] = dls;
+                else acc_dls[j] += dls;
+            }
+            dz[j] = g;                                           // after this lane's last read of z[j]
+            if (TRAIN) acc_dba[j] += g;
+        }
+        float verr;
+        if (TRAIN) {
+            const float* hc = a.h3 + m * (2 * (int64_t)H) + H;
+            float vp = 0.f;
+            for (int k = lane; k < H; k += 32) vp = fmaf(__ldg(hc + k), s_wc[k], vp);
+            verr = warp_sum(vp) + bias_c - __ldg(a.ret + src);
+            const float dv = live ? a.vw * verr * a.inv_m : 0.f;
+            float* dc = a.d3 + m * (2 * (int64_t)H) + H;
+            for (int k = lane; k < H; k += 32) {
+                const float h = __ldg(hc + k);
+                const float g = dv * s_wc[k] * (1.0f - h * h);
+                dc[k] = g;
+                acc_dwc[k] = fmaf(dv, h, acc_dwc[k]);
+                acc_db3[k] += g;
+            }
+            s_dbc += dv;
+        } else {
+            verr = __ldg(a.values + m) - __ldg(a.ret + m);
+            if (lane == 0) a.dvalues[m] = a.vw * verr * a.inv_m;
+        }
+        if (live) { l_pol += t.policy; l_val += verr * verr; l_ent += entropy; }
+    }
+    if (lane == 0) { s_small[warp * 4] = l_pol; s_small[warp * 4 + 1] = l_val; s_small[warp * 4 + 2] = l_ent; s_small[warp * 4 + 3] = s_dbc; }
+    __syncthreads();
+
+    const WideOffsets o = wide_offsets(H, A);
+    float* out = a.partials + (int64_t)blockIdx.x * a.partial_stride;
+    for (int i = threadIdx.x; i < wf; i += blockDim.x) {
+        float s = 0.f;
+        for (int w = 0; w < nw; ++w) s += smem[H + (size_t)w * wf + i];
+        int dst = o.dls + i;
+        if (TRAIN) dst = i < A ? o.dba + i : i < 2 * A ? o.dls + (i - A) : i < 2 * A + H ? o.dwc + (i - 2 * A) : o.db3 + (i - 2 * A - H);
+        out[dst] = s;
+    }
+    if (threadIdx.x < 4) {
+        float s = 0.f;
+        for (int w = 0; w < nw; ++w) s += s_small[w * 4 + threadIdx.x];
+        if (threadIdx.x < 3) out[threadIdx.x] = s;
+        else { out[3] = 0.f; out[o.dbc] = s; }
+    }
+}
+
+__global__ void wide_loss_finalize_kernel(const float* __restrict__ partials, int nparts, int stride, int dls_off, int A, float vw,
+                                          float beta, float inv_m, float* __restrict__ losses, float* __restrict__ dlog_std)
+{
+    __shared__ float l[3];
+    for (int i = threadIdx.x; i < 3 + A; i += blockDim.x) {
+        const int off = i < 3 ? i : dls_off + (i - 3);
+        float s = 0.f;
+        for (int p = 0; p < nparts; ++p) s += partials[(int64_t)p * stride + off];
+        if (i < 3) l[i] = s;
+        else if (dlog_std) dlog_std[i - 3] = s;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const float pol = l[0] * inv_m, val = 0.5f * l[1] * inv_m, ent = l[2] * inv_m;
+        losses[0] = pol; losses[1] = val; losses[2] = ent; losses[3] = pol + vw * val + -beta * ent;
+    }
+}
+
+// Critic head of the forward pass at H > 512: one warp per row, wc in shared memory (the actor head is a GEMM there).
+__global__ void __launch_bounds__(256)
+critic_value_kernel(const float* __restrict__ hc, int ld, const float* __restrict__ wc, const float* __restrict__ bc,
+                    float* __restrict__ values, int64_t rows, int H, const int* __restrict__ rows_dev)
+{
+    extern __shared__ float s_wc[];
+    if (rows_dev != nullptr && *rows_dev < rows) rows = *rows_dev;
+    for (int i = threadIdx.x; i < H; i += blockDim.x) s_wc[i] = wc[i];
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int64_t w0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t ws = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t m = w0; m < rows; m += ws) {
+        float part = 0.f;
+        for (int k = lane; k < H; k += 32) part = fmaf(__ldg(hc + m * ld + k), s_wc[k], part);
+        part = warp_sum(part);
+        if (lane == 0) values[m] = part + bc[0];
+    }
+}
+
+// warps per CTA of the training variant: two CTAs per SM while the per-warp accumulators allow it
+int wide_train_warps(int H, int A)
+{
+    int nw = 8;
+    while (nw > 1 && ((size_t)nw * (2 * (A + H) + 4) + H) * sizeof(float) > 110 * 1024) nw >>= 1;
+    return nw;
+}
+
 template <int KPL, int VEC, int R>
 int launch_head_train(dppo_ctx* ctx, const HeadTrainArgs& a, int continuous, int blocks, size_t smem, cudaStream_t st)
 {
@@ -958,15 +1142,26 @@ int head_train_blocks(dppo_ctx* ctx, int64_t M, int H, int A)
     return (int)(want < cap ? want : cap);
 }
 
+// dynamic shared memory of head_train_kernel: Wa | wc, then the per-warp accumulators (reused as the flush scratch)
+static size_t head_train_smem(int H, int A)
+{
+    size_t accf = (size_t)HEAD_WARPS * (A + 1) * H;
+    const size_t scratchf = (size_t)HEAD_WARPS * (2 * H + 100);
+    if (accf < scratchf) accf = scratchf;
+    return ((size_t)(A + 1) * H + accf) * sizeof(float);
+}
+
+bool head_train_supported(int H, int A)
+{
+    return A >= 1 && A <= DPPO_MAX_ACT && H >= 1 && H <= 512 && head_train_smem(H, A) <= 200 * 1024;
+}
+
 int launch_head_train_kernel(dppo_ctx* ctx, const HeadTrainArgs& a, int continuous, int blocks, cudaStream_t st)
 {
     const int H = a.H, A = a.A;
     if (A < 1 || A > DPPO_MAX_ACT) DPPO_FAIL(ctx, "head kernel supports 1..%d actions/action dims, got %d", DPPO_MAX_ACT, A);
     if (H < 1 || H > 512) DPPO_FAIL(ctx, "head kernel supports hidden <= 512, got %d", H);
-    size_t accf = (size_t)HEAD_WARPS * (A + 1) * H;
-    const size_t scratchf = (size_t)HEAD_WARPS * (2 * H + 100);
-    if (accf < scratchf) accf = scratchf;
-    const size_t smem = ((size_t)(A + 1) * H + accf) * sizeof(float);
+    const size_t smem = head_train_smem(H, A);
     if (smem > 200 * 1024) DPPO_FAIL(ctx, "head kernel: (A+1)*H = %d too large for shared memory", (A + 1) * H);
     const bool vec = (H % 128 == 0) && ((reinterpret_cast<uintptr_t>(a.h3) & 15u) == 0) && ((reinterpret_cast<uintptr_t>(a.d3) & 15u) == 0);
     if (vec && head_split_shape(H, A)) {
@@ -1024,6 +1219,44 @@ int launch_head_eval(dppo_ctx* ctx, const float* ha, const float* hc, int ld, co
     return 0;
 }
 
+int launch_heads_forward(dppo_ctx* ctx, const float* ha, const float* hc, int ld, const float* wa, const float* ba, const float* wc,
+                         const float* bc, float* head_out, float* values, int64_t rows, int H, int A, int rev, cudaStream_t st)
+{
+    if (A >= 1 && A <= DPPO_MAX_ACT && H >= 1 && H <= 512)
+        return launch_head_eval(ctx, ha, hc, ld, wa, ba, wc, bc, head_out, values, rows, H, A, rev, st);
+    if (A < 1 || A > DPPO_GEMM_HEADS_MAX_ACT || H < 1 || H > DPPO_GEMM_HEADS_MAX_HIDDEN)
+        DPPO_FAIL(ctx, "heads: hidden %d / %d actions outside the GEMM-head bound (hidden <= %d, 1..%d actions)", H, A,
+                  DPPO_GEMM_HEADS_MAX_HIDDEN, DPPO_GEMM_HEADS_MAX_ACT);
+    // logits / means = h3a Wa^T + ba (ppo.py:63-71)
+    if (ha && dppo_gemm_nt(ctx, DPPO_EPI_BIAS, ha, ld, nullptr, wa, H, ba, head_out, A, rows, A, H, st)) return 1;
+    if (hc) {
+        int64_t want = (rows + 7) / 8;
+        const int blocks = (int)(want < 4 * (int64_t)ctx->sm_count ? want : 4 * (int64_t)ctx->sm_count);
+        critic_value_kernel<<<blocks, 256, (size_t)H * sizeof(float), st>>>(hc, ld, wc, bc, values, rows, H, ctx->rows_dev);
+        DPPO_CHECK_LAUNCH(ctx, "critic_value_kernel");
+    }
+    return 0;
+}
+
+int wide_loss_blocks(dppo_ctx* ctx, int64_t M, int H, int A)
+{
+    const int nw = wide_train_warps(H, A);
+    const int64_t want = (M + nw - 1) / nw;
+    const int64_t cap = 2 * (int64_t)ctx->sm_count;
+    return (int)(want < cap ? want : cap);
+}
+
+int launch_wide_loss_train(dppo_ctx* ctx, const WideLossArgs& a, int continuous, int blocks, cudaStream_t st)
+{
+    const int nw = wide_train_warps(a.H, a.A);
+    const size_t smem = ((size_t)nw * (2 * (a.A + a.H) + 4) + a.H) * sizeof(float);
+    auto kern = continuous ? wide_loss_kernel<true, true> : wide_loss_kernel<false, true>;
+    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    dppo_launch_pdl(ctx, kern, dim3(blocks), dim3(nw * 32), smem, st, a);
+    DPPO_CHECK_LAUNCH(ctx, "wide_loss_kernel");
+    return 0;
+}
+
 extern "C" int dppo_logprob_categorical(dppo_ctx* ctx, const float* logits, const int32_t* actions, float* log_probs,
                                         int64_t rows, int A, void* stream)
 {
@@ -1055,12 +1288,14 @@ static int loss_blocks(dppo_ctx* ctx, int64_t M)
     return (int)(want < cap ? want : cap);
 }
 
+// floats per CTA partial: loss_rows_kernel's 40 up to DPPO_MAX_ACT actions, wide_loss_kernel's above
+static int loss_partial_floats(int A) { return A <= DPPO_MAX_ACT ? 40 : wide_offsets(0, A).total; }
+
 extern "C" int64_t dppo_ppo_loss_workspace_bytes(int64_t M, int A)
 {
-    (void)A;
     int64_t blocks = (M + 7) / 8;
     if (blocks > 2 * 256) blocks = 2 * 256;            // upper bound on 2*SMs
-    return blocks * 40 * (int64_t)sizeof(float);
+    return blocks * loss_partial_floats(A) * (int64_t)sizeof(float);
 }
 
 static int ppo_loss_common(dppo_ctx* ctx, bool cont, const float* head, const float* log_std, int64_t ls_stride, const float* values,
@@ -1070,11 +1305,30 @@ static int ppo_loss_common(dppo_ctx* ctx, bool cont, const float* head, const fl
 {
     if (!ctx) return 1;
     if (M <= 0) DPPO_FAIL(ctx, "ppo_loss: empty minibatch");
-    if (A < 1 || A > DPPO_MAX_ACT) DPPO_FAIL(ctx, "ppo_loss supports 1..%d actions/action dims, got %d", DPPO_MAX_ACT, A);
+    if (A < 1 || A > DPPO_GEMM_HEADS_MAX_ACT) DPPO_FAIL(ctx, "ppo_loss supports 1..%d actions/action dims, got %d", DPPO_GEMM_HEADS_MAX_ACT, A);
     const int blocks = loss_blocks(ctx, M);
-    if (ws_bytes < (int64_t)blocks * 40 * (int64_t)sizeof(float)) DPPO_FAIL(ctx, "ppo_loss: workspace too small");
+    if (ws_bytes < (int64_t)blocks * loss_partial_floats(A) * (int64_t)sizeof(float)) DPPO_FAIL(ctx, "ppo_loss: workspace too small");
     const float inv_m = 1.0f / (float)(h->loss_denominator > 0 ? h->loss_denominator : M);
     float* partials = (float*)ws;
+    if (A > DPPO_MAX_ACT) {
+        // more actions than lanes: lanes stride over the actions (wide_loss_kernel without its critic part)
+        WideLossArgs a = {};
+        a.z = head; a.dz = dhead; a.log_std = log_std; a.ls_stride = cont ? ls_stride : 0; a.dls_rows = ls_stride ? dlog_std : nullptr;
+        a.values = values; a.dvalues = dvalues;
+        a.actions_i = actions_i; a.actions_f = actions_f; a.old_logp = old_lp; a.adv = adv; a.ret = ret;
+        a.M = M; a.H = 0; a.A = A;
+        a.clip = h->ppo_clip; a.vw = h->value_loss_weight; a.beta = h->entropy_beta; a.inv_m = inv_m;
+        a.partials = partials; a.partial_stride = loss_partial_floats(A);
+        const size_t smem = ((size_t)8 * (A + 4)) * sizeof(float);
+        auto kern = cont ? wide_loss_kernel<true, false> : wide_loss_kernel<false, false>;
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        kern<<<blocks, 256, smem, st>>>(a);
+        DPPO_CHECK_LAUNCH(ctx, "wide_loss_kernel");
+        wide_loss_finalize_kernel<<<1, 256, 0, st>>>(partials, blocks, a.partial_stride, wide_offsets(0, A).dls, A, h->value_loss_weight,
+                                                    h->entropy_beta, inv_m, losses, (cont && !ls_stride) ? dlog_std : nullptr);
+        DPPO_CHECK_LAUNCH(ctx, "wide_loss_finalize_kernel");
+        return 0;
+    }
     if (cont)
         loss_rows_kernel<true><<<blocks, 256, 0, st>>>(head, log_std, ls_stride, values, actions_i, actions_f, old_lp, adv, ret, M, A,
                                                        h->ppo_clip, h->value_loss_weight, h->entropy_beta, inv_m, dhead,

@@ -43,6 +43,55 @@ __host__ __device__ inline HeadOffsets head_offsets(int H, int A)
 }
 int head_partial_floats(int H, int A);
 int head_train_blocks(dppo_ctx* ctx, int64_t M, int H, int A);
+bool head_train_supported(int H, int A);      // the shapes launch_head_train_kernel accepts (dppo_mlp_fused_heads_supported)
 int launch_head_train_kernel(dppo_ctx* ctx, const HeadTrainArgs& a, int continuous, int blocks, cudaStream_t st);
 int launch_head_eval(dppo_ctx* ctx, const float* ha, const float* hc, int ld, const float* wa, const float* ba, const float* wc,
                      const float* bc, float* head_out, float* values, int64_t rows, int H, int A, int rev, cudaStream_t st);
+// launch_head_eval where it accepts the shape (A <= 32, H <= 512), else the actor product as a GEMM and critic_value_kernel
+int launch_heads_forward(dppo_ctx* ctx, const float* ha, const float* hc, int ld, const float* wa, const float* ba, const float* wc,
+                         const float* bc, float* head_out, float* values, int64_t rows, int H, int A, int rev, cudaStream_t st);
+
+// ---- GEMM-head path (any shape up to DPPO_GEMM_HEADS_MAX_HIDDEN / _ACT) -----------------------------------------------------
+// The head products, their backward and the head weight gradients are GEMMs (api.cu); wide_loss_kernel evaluates the distribution,
+// the loss and d(loss)/dz of one row per warp (lanes stride over the actions) and, in training, the critic head of the row.
+struct WideLossArgs {
+    const float* z;           // [M, A] head outputs (logits / means)
+    float* dz;                // [M, A] d(loss)/dz; may alias z (each lane reads z[j] before it writes dz[j])
+    const float* log_std;     // [A] shared, or [M, ls_stride] per row (standalone loss only)
+    int64_t ls_stride;
+    float* dls_rows;          // [M, A] per-row d(loss)/d(log_std) when ls_stride != 0
+    const float* values;      // standalone: [M] critic outputs
+    float* dvalues;           // standalone: [M] d(loss)/d(values)
+    const float* h3;          // training: [M, 2H] first-head-layer activations (the critic half is read)
+    float* d3;                // training: [M, 2H] the critic half d3[:, H:] is written
+    const float *wc, *bc;     // training: critic_head.2
+    const int32_t* idx;       // training: minibatch row -> flat sample index (may be null; < 0: padding row)
+    const int32_t* actions_i; // discrete: [B]
+    const float* actions_f;   // continuous: [B, A]
+    const float *old_logp, *adv, *ret;
+    const double* adv_stats;  // training: advantage normalisation (adv_norm_consts)
+    int64_t adv_count;
+    int advantage_norm;
+    int64_t M;
+    int H, A;
+    float clip, vw, beta, inv_m;
+    float* partials;          // [blocks, partial_stride], layout wide_offsets(H, A) (standalone: H = 0)
+    int partial_stride;
+};
+// One partial per CTA: [losses 4 (policy, value, entropy, 0) | dbc | dba A | dlog_std A | dWc H | critic db3 H], each block on a
+// multiple of 4 floats.  O(A + H) per CTA; dWa is not part of it (a split-K GEMM computes it).
+struct WideOffsets { int dbc, dba, dls, dwc, db3, total; };
+__host__ __device__ inline WideOffsets wide_offsets(int H, int A)
+{
+    auto up4 = [](int x) { return (x + 3) / 4 * 4; };
+    WideOffsets o;
+    o.dbc = 4;
+    o.dba = 8;
+    o.dls = up4(o.dba + A);
+    o.dwc = up4(o.dls + A);
+    o.db3 = up4(o.dwc + H);
+    o.total = up4(o.db3 + H);
+    return o;
+}
+int wide_loss_blocks(dppo_ctx* ctx, int64_t M, int H, int A);
+int launch_wide_loss_train(dppo_ctx* ctx, const WideLossArgs& a, int continuous, int blocks, cudaStream_t st);

@@ -56,12 +56,19 @@ grad_reduce_kernel(GradSegTable tab, float* __restrict__ grads, int64_t total, c
                         acc.z = (a[0].z + a[1].z) + (a[2].z + a[3].z);
                         acc.w = (a[0].w + a[1].w) + (a[2].w + a[3].w);
                     } else {
+                        // element by element; an element past this segment's end may start the next one (a tensor whose
+                        // gradient comes from two sources, e.g. the halves of b3 on the GEMM-head path, at an odd split)
                         float o[4] = {0.f, 0.f, 0.f, 0.f};
-                        for (int e = 0; e < 4; ++e) {
-                            if (i + e >= sg.dst + sg.count) break;
-                            float s0 = 0.f;
-                            for (int q = y; q < sg.nparts; q += RED_Y) s0 += __ldg(p + e + (int64_t)q * sg.stride);
-                            o[e] = s0;
+                        for (int e = 0; e < 4 && i + e < total; ++e) {
+                            for (int g2 = g; g2 < tab.nseg; ++g2) {
+                                const GradSeg& s2 = tab.seg[g2];
+                                if (i + e < s2.dst || i + e >= s2.dst + s2.count) continue;
+                                const float* p2 = s2.src + (i + e - s2.dst);
+                                float s0 = 0.f;
+                                for (int q = y; q < s2.nparts; q += RED_Y) s0 += __ldg(p2 + (int64_t)q * s2.stride);
+                                o[e] = s0;
+                                break;
+                            }
                         }
                         acc = make_float4(o[0], o[1], o[2], o[3]);
                     }

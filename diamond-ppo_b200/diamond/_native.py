@@ -59,7 +59,8 @@ EXPORTS = [
     "dppo_buffer_store_step", "dppo_step_record_bytes", "dppo_sample_categorical", "dppo_sample_gaussian",
     "dppo_gae_f32", "dppo_adv_normalize_f32", "dppo_permutation_mt19937", "dppo_permutation_mt19937_skip", "dppo_mt19937_seed",
     "dppo_gather_rows_f32", "dppo_mlp_layout_compute", "dppo_mlp_workspace_bytes", "dppo_mlp_forward", "dppo_mlp_next_values", "dppo_mlp_next_values_workspace_bytes",
-    "dppo_logprob_categorical", "dppo_logprob_gaussian", "dppo_mlp_grad_minibatch", "dppo_small_update", "dppo_small_update_supported", "dppo_clip_adam_step",
+    "dppo_logprob_categorical", "dppo_logprob_gaussian", "dppo_mlp_grad_minibatch", "dppo_mlp_fused_heads_supported",
+    "dppo_mlp_gemm_heads_workspace_bytes", "dppo_mlp_grad_minibatch_gemm_heads", "dppo_small_update", "dppo_small_update_supported", "dppo_clip_adam_step",
     "dppo_clip_adam_workspace_bytes", "dppo_grad_sumsq_bytes", "dppo_ppo_loss_discrete", "dppo_ppo_loss_gaussian",
     "dppo_ppo_loss_workspace_bytes", "dppo_fma_peak_kernel", "dppo_tc_linear_f32", "dppo_tc_linear_workspace_bytes",
     "dppo_tc_colsum_parts", "dppo_tc_wgrad_f32", "dppo_tc_wgrad_workspace_bytes", "dppo_tc_mma_probe", "dppo_dp_create", "dppo_dp_handle_bytes", "dppo_dp_handle", "dppo_dp_connect", "dppo_dp_destroy", "dppo_dp_status",
@@ -85,7 +86,8 @@ def load_library() -> C.CDLL:
             lib.dppo_last_error.argtypes = [C.c_void_p]
             for name in ("dppo_step_record_bytes", "dppo_mlp_workspace_bytes", "dppo_clip_adam_workspace_bytes", "dppo_grad_sumsq_bytes",
                          "dppo_ppo_loss_workspace_bytes", "dppo_tc_linear_workspace_bytes", "dppo_tc_wgrad_workspace_bytes", "dppo_launch_count", "dppo_dp_workspace_bytes", "dppo_grad_sumsq_bytes",
-                         "dppo_rnn_workspace_bytes", "dppo_episode_stats_workspace_bytes", "dppo_mlp_next_values_workspace_bytes"):
+                         "dppo_rnn_workspace_bytes", "dppo_episode_stats_workspace_bytes", "dppo_mlp_next_values_workspace_bytes",
+                         "dppo_mlp_gemm_heads_workspace_bytes"):
                 getattr(lib, name).restype = C.c_int64
             lib.dppo_dp_slot.restype = C.c_void_p
             _lib = lib
@@ -125,6 +127,11 @@ def rnn_layout(desc: RnnDesc) -> RnnLayout:
 
 
 # ---- host-only entry points (usable without a GPU) -------------------------------------------
+def fused_heads_supported(desc: MlpDesc) -> bool:
+    """dppo_mlp_fused_heads_supported: whether dppo_mlp_grad_minibatch's fused head kernel takes this network shape."""
+    return bool(load_library().dppo_mlp_fused_heads_supported(C.byref(desc)))
+
+
 def mt19937_seed(seed: int):
     key = np.zeros(624, np.uint32)
     pos = C.c_int32(0)
@@ -314,6 +321,24 @@ class Context:
                                                      _ptr(losses), _ptr(ws), C.c_int64(ws.numel() * ws.element_size()),
                                                      _stream()), "dppo_mlp_grad_minibatch")
         self.launches += 10
+
+    # ---- GEMM heads: every shape up to DPPO_GEMM_HEADS_MAX_HIDDEN / _ACT (include/dppo.h) ---------------------------------
+    def mlp_fused_heads_supported(self, desc) -> bool:
+        """True exactly for the shapes the fused head kernel of mlp_grad_minibatch accepts."""
+        return fused_heads_supported(desc)
+
+    def mlp_gemm_heads_workspace_bytes(self, desc, rows):
+        return int(self.lib.dppo_mlp_gemm_heads_workspace_bytes(C.byref(desc), C.c_int64(rows)))
+
+    def mlp_grad_minibatch_gemm_heads(self, desc, params, grads, obs, actions, old_logp, adv, returns, adv_stats, idx, M, hyper,
+                                      losses, ws):
+        """mlp_grad_minibatch with the heads as GEMMs around the wide loss kernel (same gradient layout and losses)."""
+        self._check(self.lib.dppo_mlp_grad_minibatch_gemm_heads(self.h, C.byref(desc), _ptr(params), _ptr(grads), _ptr(obs),
+                                                                _ptr(actions), _ptr(old_logp), _ptr(adv), _ptr(returns),
+                                                                _ptr(adv_stats), _ptr(idx), C.c_int64(M), C.byref(hyper),
+                                                                _ptr(losses), _ptr(ws), C.c_int64(ws.numel() * ws.element_size()),
+                                                                _stream()), "dppo_mlp_grad_minibatch_gemm_heads")
+        self.launches += 13
 
     def small_update_supported(self, desc) -> bool:
         return bool(self.lib.dppo_small_update_supported(C.byref(desc)))

@@ -479,6 +479,13 @@ class FusedMlpEngine(_EngineBase):
         self.fwd_rows = 65536
         self.speculate_permutations = True      # generate the next learn()'s numpy-stream permutations in the background (validated)
         self.fwd_ws = torch.empty(ctx.mlp_workspace_bytes(self.fm.desc, self.fwd_rows, False) // 4 + 256, device=device)
+        # heads of the training step: the fused head kernel where it takes the shape (A <= 32 and (A+1) H within its shared
+        # memory), else GEMM heads (hidden <= 2048, up to 1024 actions); both write the same flat gradient and losses
+        self.fused_heads = ctx.mlp_fused_heads_supported(self.fm.desc)
+        if self.fused_heads:
+            self._grad_minibatch, self._train_ws_bytes = ctx.mlp_grad_minibatch, (lambda rows: ctx.mlp_workspace_bytes(self.fm.desc, rows, True))
+        else:
+            self._grad_minibatch, self._train_ws_bytes = ctx.mlp_grad_minibatch_gemm_heads, (lambda rows: ctx.mlp_gemm_heads_workspace_bytes(self.fm.desc, rows))
         self._train_ws = None
         self._bufs = {}
         self.draws = 0
@@ -579,7 +586,7 @@ class FusedMlpEngine(_EngineBase):
                  done=[torch.cuda.Event() for _ in range(2)], plan=plan)
         for ev in b["done"]:
             ev.record()
-        b["train_ws"] = torch.empty(self.ctx.mlp_workspace_bytes(self.fm.desc, plan["rows"], True) // 4 + 256, **f)
+        b["train_ws"] = torch.empty(self._train_ws_bytes(plan["rows"]) // 4 + 256, **f)
         b["m_max"] = plan["rows"]
         self._bufs[key] = b
         return b
@@ -663,12 +670,12 @@ class FusedMlpEngine(_EngineBase):
             # env-sharded DP, fused exchange: the local gradient and loss sums go straight into this exchange's slot of the
             # exchange buffer; one kernel per rank then sums all ranks' slots over NVLink and starts the optimiser step
             slot = ctx.dp_slot(self.dpx, seq)
-            ctx.mlp_grad_minibatch(desc, self.P, slot, obs_flat, actions, old_logp, adv, ret, b["stats"], idx_k, rows, hyper,
-                                   slot + 4 * self.total, b["train_ws"])
+            self._grad_minibatch(desc, self.P, slot, obs_flat, actions, old_logp, adv, ret, b["stats"], idx_k, rows, hyper,
+                                 slot + 4 * self.total, b["train_ws"])
             ctx.dp_allreduce_clip_adam(self.dpx, seq, self.P, self.G, self.M, self.V, hyper, losses_k, self.adam_ws, self.grad_norm)
             return
-        ctx.mlp_grad_minibatch(desc, self.P, self.G, obs_flat, actions, old_logp, adv, ret, b["stats"], idx_k, rows, hyper, losses_k,
-                               b["train_ws"])
+        self._grad_minibatch(desc, self.P, self.G, obs_flat, actions, old_logp, adv, ret, b["stats"], idx_k, rows, hyper, losses_k,
+                             b["train_ws"])
         if self.dist.enabled:
             self.dist.all_reduce_sum(self.G)              # env-sharded DP over NCCL: sum of per-shard gradients
             self.dist.all_reduce_sum(losses_k)
@@ -950,6 +957,7 @@ class AutogradEngine(_EngineBase):
             else:
                 logits, values = net.get_logits_and_values(obs)
                 ctx.logprob_categorical(logits.reshape(B, -1).contiguous(), buf.actions.view(B), old_logp)
+                n_out = logits.shape[-1]                               # the buffer keeps one action index per sample
             next_values = net.get_values(nobs)
         values = values.reshape(T, N_).contiguous().clone()
         next_values = next_values.reshape(T, N_).contiguous().clone()
@@ -966,7 +974,7 @@ class AutogradEngine(_EngineBase):
         obs_flat, adv_f, ret_f = obs.view(B, -1), adv.view(B), ret.view(B)
         act_bits = buf.actions.view(B, A) if self.continuous else buf.actions.view(B).view(torch.float32)
         losses = torch.zeros(E * MB, 4, device=dev)
-        loss_ws = torch.empty(ctx.ppo_loss_workspace_bytes(M, max(A, 32)) // 4 + 64, device=dev)
+        loss_ws = torch.empty(ctx.ppo_loss_workspace_bytes(M, max(A if self.continuous else n_out, 32)) // 4 + 64, device=dev)
         idx = torch.empty(E, B, dtype=torch.int32, device=dev)
         for e in range(E):
             worker.wait(e)

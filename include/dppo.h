@@ -29,6 +29,8 @@ extern "C" {
 
 #define DPPO_VERSION 100
 #define DPPO_MAX_ACT 32          /* action count / action dims handled by the fused head kernels */
+#define DPPO_GEMM_HEADS_MAX_HIDDEN 2048   /* bounds of the GEMM-head path (dppo_mlp_grad_minibatch_gemm_heads) */
+#define DPPO_GEMM_HEADS_MAX_ACT 1024
 
 typedef struct dppo_ctx dppo_ctx;
 
@@ -206,6 +208,24 @@ int dppo_mlp_grad_minibatch(dppo_ctx* ctx, const dppo_mlp_desc* desc, const floa
                             const float* obs, const void* actions, const float* old_log_probs, const float* adv,
                             const float* returns, const double* adv_stats, const int32_t* idx, int64_t M,
                             const dppo_hyper* hyper, float* losses, void* ws, int64_t ws_bytes, void* stream);
+/* dppo_mlp_grad_minibatch runs its output heads in one fused kernel (one warp per row, lane a <-> action a, Wa and per-warp
+ * [(A+1), H] weight-gradient accumulators in shared memory).  That kernel takes 1 <= act_dim <= 32, hidden <= 512 and
+ * 9 (act_dim + 1) hidden floats within 200 KB; it refuses every other shape.  dppo_mlp_fused_heads_supported returns 1 exactly
+ * for the shapes it takes (host only, no context needed).
+ * dppo_mlp_grad_minibatch_gemm_heads computes the same gradient with GEMM heads: the head products, their backward and the head
+ * weight gradients are GEMMs, and a row kernel evaluates the distribution, the loss and the critic head.  Same arguments, same
+ * flat-gradient layout, losses and hyper->grad_sumsq partials as dppo_mlp_grad_minibatch (results agree to fp32 summation
+ * order), no synchronisation, no allocation; ws of dppo_mlp_gemm_heads_workspace_bytes(desc, M) bytes.  It takes every shape
+ * with hidden <= DPPO_GEMM_HEADS_MAX_HIDDEN and 1 <= act_dim <= DPPO_GEMM_HEADS_MAX_ACT, including those the fused kernel
+ * takes, and refuses larger ones with an error naming the bound; the workspace size is 0 for them.
+ * dppo_mlp_forward and dppo_mlp_next_values choose by themselves: the fused head evaluation up to 32 actions and hidden 512,
+ * else the actor product as a GEMM and one warp per row for the critic. */
+int dppo_mlp_fused_heads_supported(const dppo_mlp_desc* desc);
+int64_t dppo_mlp_gemm_heads_workspace_bytes(const dppo_mlp_desc* desc, int64_t rows);
+int dppo_mlp_grad_minibatch_gemm_heads(dppo_ctx* ctx, const dppo_mlp_desc* desc, const float* params, float* grads,
+                                       const float* obs, const void* actions, const float* old_log_probs, const float* adv,
+                                       const float* returns, const double* adv_stats, const int32_t* idx, int64_t M,
+                                       const dppo_hyper* hyper, float* losses, void* ws, int64_t ws_bytes, void* stream);
 
 /* The whole update loop of a learn() for the DEFAULT 64-wide network (ppo.py:258-285; BASELINE north_star item 4) in ONE launch:
  * `steps` consecutive optimiser steps (all epochs x minibatches), each on `rows` samples idx[step*rows .. +rows) (idx < 0: padding
@@ -257,7 +277,9 @@ int dppo_dp_allreduce_clip_adam(dppo_ctx* ctx, dppo_dp* dp, int64_t seq, float* 
 
 /* Standalone loss forward+backward for custom network_cls modules (readme.md:89-111): the user
  * module runs under PyTorch autograd, this provides loss values and d(loss)/d(outputs).
- * Rows are already gathered (M rows).  losses[0..3] = policy, value, entropy, total. */
+ * Rows are already gathered (M rows).  losses[0..3] = policy, value, entropy, total.
+ * 1 <= A <= DPPO_GEMM_HEADS_MAX_ACT; above 32 actions the lanes of a row's warp stride over the actions (size ws with
+ * dppo_ppo_loss_workspace_bytes(M, A)). */
 int dppo_ppo_loss_discrete(dppo_ctx* ctx, const float* logits, const float* values, const int32_t* actions,
                            const float* old_log_probs, const float* adv, const float* returns, int64_t M, int A,
                            const dppo_hyper* hyper, float* losses, float* dlogits, float* dvalues,
