@@ -229,12 +229,16 @@ int dppo_mlp_grad_minibatch_gemm_heads(dppo_ctx* ctx, const dppo_mlp_desc* desc,
 
 /* The whole update loop of a learn() for the DEFAULT 64-wide network (ppo.py:258-285; BASELINE north_star item 4) in ONE launch:
  * `steps` consecutive optimiser steps (all epochs x minibatches), each on `rows` samples idx[step*rows .. +rows) (idx < 0: padding
- * row), run by one thread-block cluster of 8 CTAs with the parameters, the gradient partials and the sharded Adam state resident
- * in (distributed) shared memory -- gather, forward, loss, backward, gradient reduce-scatter, global-norm clip, Adam and parameter
- * all-gather never leave the SMs.  step_consts: DEVICE float [steps][2] = {sqrt(1 - beta2^t), -lr / (1 - beta1^t)} of each step
- * (torch/optim/adam.py:531-547, computed by the caller in double).  params / exp_avg / exp_avg_sq are updated in place, grads
- * receives the clipped gradient of the last step, losses [steps][4] = policy, value, entropy, total per step.  Supported:
- * hidden == 64, obs_dim <= 64, act_dim <= 8 (dppo_small_update_supported); meant for minibatches of up to ~1024 rows. */
+ * row), run by one thread-block cluster of 8 CTAs (rows <= 256) or 16 CTAs (more rows) with the parameters, the gradient partials
+ * and the sharded Adam state resident in (distributed) shared memory -- gather, forward, loss, backward, gradient reduce-scatter,
+ * global-norm clip, Adam and parameter all-gather never leave the SMs.  1 <= rows <= 2048 and steps >= 1; anything else is refused
+ * before launch.  Padding rows (idx < 0) and hyper->loss_denominator (0: rows) behave as in dppo_mlp_grad_minibatch: a padding
+ * row enters no loss term and no gradient, and the loss means divide by the denominator.  step_consts: DEVICE float [steps][2] =
+ * {sqrt(1 - beta2^t), -lr / (1 - beta1^t)} of each step (torch/optim/adam.py:531-547, computed by the caller in double).  params /
+ * exp_avg / exp_avg_sq are updated in place, grads receives the clipped gradient of the last step, grad_norm_out (optional) its
+ * pre-clip norm, losses [steps][4] = policy, value, entropy, total per step.  Supported (dppo_small_update_supported): hidden == 64,
+ * 1 <= act_dim <= 8, and 1 <= obs_dim <= 64 with the kernel's shared memory within 220 KB, which bounds obs_dim at 30 (8 actions)
+ * to 36 (1 action). */
 int dppo_small_update_supported(const dppo_mlp_desc* desc);
 int dppo_small_update(dppo_ctx* ctx, const dppo_mlp_desc* desc, float* params, float* grads, float* exp_avg, float* exp_avg_sq,
                       const float* obs, const void* actions, const float* old_log_probs, const float* adv, const float* returns,

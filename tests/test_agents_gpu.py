@@ -525,11 +525,13 @@ def test_train_resume_is_bit_identical_to_uninterrupted_run(tmp_path, kind):
 
 
 @pytest.mark.parametrize("cont,D,A,N_,T,MB", [(False, 4, 2, 8, 128, 8), (False, 8, 4, 5, 20, 1), (True, 3, 1, 64, 64, 8), (True, 5, 3, 7, 33, 3),
-                                              (False, 64, 8, 16, 64, 2), (False, 17, 5, 4, 100, 4)])
+                                              (False, 30, 8, 16, 64, 2), (False, 17, 5, 4, 100, 4),
+                                              (False, 4, 2, 64, 128, 8), (True, 6, 3, 64, 128, 8), (False, 5, 3, 37, 40, 2), (True, 3, 2, 37, 40, 2)])
 def test_small_net_cluster_kernel_matches_per_layer_kernels(cont, D, A, N_, T, MB):
     """Default 64-wide networks: the one-launch cluster kernel (dppo_small_update: whole update loop in distributed shared memory)
     against the per-layer kernel path on the same learn(): losses and parameters agree to fp32 summation order, Adam moments too.
-    Ragged shapes: rows per minibatch that are not multiples of the 16-row tile or of the 8 CTAs."""
+    Ragged shapes: rows per minibatch that are not multiples of the 16-row tile or of the 8 CTAs.  1024 rows (the SMALL_ROWS bound)
+    and 740 rows give each CTA two tiles, full and ragged.  D = 30 is the largest obs_dim the kernel takes with 8 actions."""
     from diamond import PPO, PPOConfig, ContinuousPPO, ContinuousPPOConfig, envs
     Agent, Cfg = (ContinuousPPO, ContinuousPPOConfig) if cont else (PPO, PPOConfig)
     rng = np.random.default_rng(D * 7 + A)
@@ -545,6 +547,7 @@ def test_small_net_cluster_kernel_matches_per_layer_kernels(cont, D, A, N_, T, M
         agent.learn(exp)
         agent.learn(exp)                                   # Adam moments / step carried into a second launch
         torch.cuda.synchronize()
+        assert any("small" in b for b in agent.engine._bufs.values()) == small       # the cluster kernel ran exactly when enabled
         outs.append((agent.engine.P.clone(), agent.engine.M.clone(), agent.engine.V.clone(), agent.last_losses.clone(), agent.engine.adam_step))
     (p1, m1, v1, l1, s1), (p0, m0, v0, l0, s0) = outs
     assert s1 == s0 == 2 * 3 * MB
