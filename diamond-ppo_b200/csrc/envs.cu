@@ -8,8 +8,16 @@
 // Dynamics follow Gymnasium's classic-control environments (third-party, not in the reference tree; gymnasium >= 1.0.0,
 // `classic_control/cartpole.py` CartPole-v1: Euler integrator, tau 0.02, termination |x| > 2.4 or |theta| > 12 deg, 500-step
 // time limit; `classic_control/pendulum.py` Pendulum-v1: dt 0.05, g 10, torque clipped to [-2, 2], speed clipped to [-8, 8],
-// 200-step time limit, never terminates) with the state held in float64 as Gymnasium does, observations cast to float32.
-// The checker is oracle/env_oracle.py; reset draws come from Philox4x32-10 keyed by (seed, global env id, episode index),
+// 200-step time limit, never terminates; `classic_control/acrobot.py` Acrobot-v1: "book" dynamics, one RK4 step of dt 0.2,
+// angles wrapped into [-pi, pi], speeds bounded to 4 pi / 9 pi, torque a - 1, 500-step time limit;
+// `classic_control/mountain_car.py` MountainCar-v0: force (a - 1) * 0.001, 200-step time limit;
+// `classic_control/continuous_mountain_car.py` MountainCarContinuous-v0: 999-step time limit) with the state held in float64
+// as Gymnasium does, observations cast to float32.  MountainCarContinuous keeps Gymnasium's float32 state: under NumPy 2's
+// promotion rules (NEP 50) its step runs in float32 except cos(3 p) and, for an action outside [-1, 1], the force term,
+// which are double; the explicitly rounded intrinsics below keep the compiler from contracting those operations into FMAs.
+// The time limit is the repository's convention: truncated = steps >= limit && !terminated.
+// The checkers are oracle/env_oracle.py (CartPole, Pendulum) and tests/classic_env_oracle.py (Acrobot, MountainCar,
+// MountainCarContinuous); reset draws come from Philox4x32-10 keyed by (seed, global env id, episode index),
 // so a run does not depend on launch geometry or GPU count.
 #include "common.cuh"
 
@@ -31,7 +39,8 @@ __device__ __forceinline__ double u01d(uint32_t x) { return ((double)x + 0.5) * 
 
 struct EnvArgs {
     int kind, N, D, A, t, auto_reset;
-    double* state;              // [N, 4]  CartPole: x, x_dot, theta, theta_dot; Pendulum: theta, theta_dot; synthetic: unused
+    double* state;              // [N, 4]  CartPole: x, x_dot, theta, theta_dot; Pendulum: theta, theta_dot; Acrobot: theta1,
+                                //         theta2, theta1_dot, theta2_dot; MountainCar(Continuous): position, velocity; synthetic: unused
     int32_t* steps;             // [N] steps taken in the current episode
     int64_t* episode;           // [N] episodes started so far (reset draw index)
     double* ep_return;          // [N] running return
@@ -46,28 +55,55 @@ struct EnvArgs {
     float p_term, p_trunc;      // synthetic env
 };
 
+template <int KIND>
 __device__ __forceinline__ void reset_state(const EnvArgs& a, int e, double* s)
 {
     const unsigned long long env = (unsigned long long)(a.env_offset + e);
     const unsigned long long ep = (unsigned long long)a.episode[e];
     const uint4 r = philox4x32_10(make_uint4((uint32_t)env, (uint32_t)(env >> 32), (uint32_t)ep, (uint32_t)(ep >> 32) ^ 0x52534554u),
                                   make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-    if (a.kind == 0) {            // uniform(-0.05, 0.05) x 4
+    if constexpr (KIND == 0) {    // uniform(-0.05, 0.05) x 4
         s[0] = -0.05 + 0.1 * u01d(r.x); s[1] = -0.05 + 0.1 * u01d(r.y); s[2] = -0.05 + 0.1 * u01d(r.z); s[3] = -0.05 + 0.1 * u01d(r.w);
-    } else {                      // theta ~ U(-pi, pi), theta_dot ~ U(-1, 1)
+    } else if constexpr (KIND == 1) {   // theta ~ U(-pi, pi), theta_dot ~ U(-1, 1)
         s[0] = -3.14159265358979323846 + 6.28318530717958647692 * u01d(r.x); s[1] = -1.0 + 2.0 * u01d(r.y); s[2] = 0.0; s[3] = 0.0;
+    } else if constexpr (KIND == 4) {   // uniform(-0.1, 0.1) x 4 rounded to float32, as Gymnasium's .astype(np.float32)
+        s[0] = (float)(-0.1 + 0.2 * u01d(r.x)); s[1] = (float)(-0.1 + 0.2 * u01d(r.y));
+        s[2] = (float)(-0.1 + 0.2 * u01d(r.z)); s[3] = (float)(-0.1 + 0.2 * u01d(r.w));
+    } else {                            // position ~ U(-0.6, -0.4) (float32 state for the continuous car), velocity 0
+        const double p = -0.6 + 0.2 * u01d(r.x);
+        s[0] = KIND == 6 ? (double)(float)p : p; s[1] = 0.0; s[2] = 0.0; s[3] = 0.0;
     }
     a.episode[e] += 1;
     a.steps[e] = 0;
 }
 
-__device__ __forceinline__ void write_obs(int kind, const double* s, float* o)
+template <int KIND>
+__device__ __forceinline__ void write_obs(const double* s, float* o)
 {
-    if (kind == 0) { o[0] = (float)s[0]; o[1] = (float)s[1]; o[2] = (float)s[2]; o[3] = (float)s[3]; }
-    else { o[0] = (float)cos(s[0]); o[1] = (float)sin(s[0]); o[2] = (float)s[1]; }
+    if constexpr (KIND == 0) { o[0] = (float)s[0]; o[1] = (float)s[1]; o[2] = (float)s[2]; o[3] = (float)s[3]; }
+    else if constexpr (KIND == 1) { o[0] = (float)cos(s[0]); o[1] = (float)sin(s[0]); o[2] = (float)s[1]; }
+    else if constexpr (KIND == 4) {
+        o[0] = (float)cos(s[0]); o[1] = (float)sin(s[0]); o[2] = (float)cos(s[1]); o[3] = (float)sin(s[1]); o[4] = (float)s[2]; o[5] = (float)s[3];
+    } else { o[0] = (float)s[0]; o[1] = (float)s[1]; }
+}
+
+// Acrobot-v1 `_dsdt` ("book" dynamics; m1 = m2 = l1 = 1, lc1 = lc2 = 0.5, I1 = I2 = 1, g = 9.8) in Gymnasium's operation order
+__device__ __forceinline__ void acrobot_dsdt(const double* y, double torque, double* dy)
+{
+    const double m1 = 1.0, m2 = 1.0, l1 = 1.0, lc1 = 0.5, lc2 = 0.5, I1 = 1.0, I2 = 1.0, g = 9.8, pi = 3.14159265358979323846;
+    const double th1 = y[0], th2 = y[1], dth1 = y[2], dth2 = y[3];
+    const double c2 = cos(th2), s2 = sin(th2);
+    const double d1 = m1 * (lc1 * lc1) + m2 * (l1 * l1 + lc2 * lc2 + 2.0 * l1 * lc2 * c2) + I1 + I2;
+    const double d2 = m2 * (lc2 * lc2 + l1 * lc2 * c2) + I2;
+    const double phi2 = m2 * lc2 * g * cos(th1 + th2 - pi / 2.0);
+    const double phi1 = -m2 * l1 * lc2 * (dth2 * dth2) * s2 - 2.0 * m2 * l1 * lc2 * dth2 * dth1 * s2 + (m1 * lc1 + m2 * l1) * g * cos(th1 - pi / 2.0)
+                        + phi2;
+    const double ddth2 = (torque + d2 / d1 * phi1 - m2 * l1 * lc2 * (dth1 * dth1) * s2 - phi2) / (m2 * (lc2 * lc2) + I2 - d2 * d2 / d1);
+    dy[0] = dth1; dy[1] = dth2; dy[2] = -(d2 * ddth2 + phi1) / d1; dy[3] = ddth2;
 }
 
 // mode 0: step (t, actions); mode 1: reset the environments with mask[e] != 0 (mask null: all)
+template <int KIND>
 __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __restrict__ mask)
 {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -77,18 +113,19 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
     for (int i = 0; i < 4; ++i) s[i] = a.state[(int64_t)e * 4 + i];
     if (mode == 1) {
         if (mask == nullptr || mask[e]) {
-            reset_state(a, e, s);
+            reset_state<KIND>(a, e, s);
             a.ep_return[e] = 0.0;
 #pragma unroll
             for (int i = 0; i < 4; ++i) a.state[(int64_t)e * 4 + i] = s[i];
-            write_obs(a.kind, s, a.cur_obs + (int64_t)e * a.D);
+            write_obs<KIND>(s, a.cur_obs + (int64_t)e * a.D);
         }
         return;
     }
-    if (a.obs_t) write_obs(a.kind, s, a.obs_t + (int64_t)e * a.D);
+    if (a.obs_t) write_obs<KIND>(s, a.obs_t + (int64_t)e * a.D);
     double reward;
-    bool term = false, trunc;
-    if (a.kind == 0) {
+    bool term = false;
+    int limit;                                                          // TimeLimit of the registered id
+    if constexpr (KIND == 0) {
         const long long act = reinterpret_cast<const long long*>(a.actions)[e];
         if (a.act_t) reinterpret_cast<int32_t*>(a.act_t)[e] = (int32_t)act;
         const double gravity = 9.8, masscart = 1.0, masspole = 0.1, length = 0.5, force_mag = 10.0, tau = 0.02;
@@ -102,9 +139,8 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
         s[0] = x; s[1] = xd; s[2] = th; s[3] = thd;
         term = fabs(x) > 2.4 || fabs(th) > 12.0 * 2.0 * 3.14159265358979323846 / 360.0;
         reward = 1.0;
-        a.steps[e] += 1;
-        trunc = a.steps[e] >= 500 && !term;
-    } else {
+        limit = 500;
+    } else if constexpr (KIND == 1) {
         const float af = reinterpret_cast<const float*>(a.actions)[(int64_t)e * a.A];
         if (a.act_t) reinterpret_cast<float*>(a.act_t)[(int64_t)e * a.A] = af;
         const double max_speed = 8.0, max_torque = 2.0, dt = 0.05, g = 10.0, m = 1.0, l = 1.0, pi = 3.14159265358979323846;
@@ -117,10 +153,69 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
         thd = fmin(fmax(thd, -max_speed), max_speed);
         s[1] = thd;
         s[0] = s[0] + thd * dt;
-        a.steps[e] += 1;
-        trunc = a.steps[e] >= 200;
+        limit = 200;
+    } else if constexpr (KIND == 4) {                                   // Acrobot-v1
+        const long long act = reinterpret_cast<const long long*>(a.actions)[e];
+        if (a.act_t) reinterpret_cast<int32_t*>(a.act_t)[e] = (int32_t)act;
+        const double torque = (double)(act - 1), dt = 0.2, pi = 3.14159265358979323846;
+        double k1[4], k2[4], k3[4], k4[4], y[4];
+        acrobot_dsdt(s, torque, k1);                                    // rk4 over [0, dt]: y0 + dt / 6 (k1 + 2 k2 + 2 k3 + k4)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) y[i] = s[i] + dt / 2.0 * k1[i];
+        acrobot_dsdt(y, torque, k2);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) y[i] = s[i] + dt / 2.0 * k2[i];
+        acrobot_dsdt(y, torque, k3);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) y[i] = s[i] + dt * k3[i];
+        acrobot_dsdt(y, torque, k4);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) s[i] = s[i] + dt / 6.0 * (k1[i] + 2.0 * k2[i] + 2.0 * k3[i] + k4[i]);
+#pragma unroll
+        for (int i = 0; i < 2; ++i) {                                   // Gymnasium's `wrap` into [-pi, pi]: loops, not fmod
+            while (s[i] > pi) s[i] = s[i] - 2.0 * pi;
+            while (s[i] < -pi) s[i] = s[i] + 2.0 * pi;
+        }
+        s[2] = fmin(fmax(s[2], -4.0 * pi), 4.0 * pi);
+        s[3] = fmin(fmax(s[3], -9.0 * pi), 9.0 * pi);
+        term = -cos(s[0]) - cos(s[1] + s[0]) > 1.0;
+        reward = term ? 0.0 : -1.0;
+        limit = 500;
+    } else if constexpr (KIND == 5) {                                   // MountainCar-v0, float64 (no contraction: numpy has none)
+        const long long act = reinterpret_cast<const long long*>(a.actions)[e];
+        if (a.act_t) reinterpret_cast<int32_t*>(a.act_t)[e] = (int32_t)act;
+        double p = s[0], v = s[1];
+        v = __dadd_rn(v, __dadd_rn(__dmul_rn((double)(act - 1), 0.001), __dmul_rn(cos(__dmul_rn(3.0, p)), -0.0025)));
+        v = fmin(fmax(v, -0.07), 0.07);
+        p = fmin(fmax(__dadd_rn(p, v), -1.2), 0.6);
+        if (p == -1.2 && v < 0.0) v = 0.0;
+        s[0] = p; s[1] = v;
+        term = p >= 0.5 && v >= 0.0;
+        reward = -1.0;
+        limit = 200;
+    } else {                                                            // MountainCarContinuous-v0, float32 state
+        const float af = reinterpret_cast<const float*>(a.actions)[(int64_t)e * a.A];
+        if (a.act_t) reinterpret_cast<float*>(a.act_t)[(int64_t)e * a.A] = af;
+        float p = (float)s[0], v = (float)s[1];
+        const double c = cos((double)__fmul_rn(3.0f, p));                // math.cos on the float32 product
+        // min(max(action[0], -1.0), 1.0) is the float32 action when in range (float32 multiply), a Python float (double) when not
+        const float dv = (af > 1.0f || af < -1.0f) ? (float)__dsub_rn(af > 1.0f ? 0.0015 : -0.0015, __dmul_rn(0.0025, c))
+                                                   : __fsub_rn(__fmul_rn(af, 0.0015f), (float)__dmul_rn(0.0025, c));
+        v = __fadd_rn(v, dv);
+        if (v > 0.07f) v = 0.07f;
+        if (v < -0.07f) v = -0.07f;
+        p = __fadd_rn(p, v);
+        if (p > 0.6f) p = 0.6f;
+        if (p < -1.2f) p = -1.2f;
+        if (p == -1.2f && v < 0.0f) v = 0.0f;
+        s[0] = p; s[1] = v;
+        term = p >= 0.45f && v >= 0.0f;
+        reward = (term ? 100.0 : 0.0) - __dmul_rn(__dmul_rn((double)af, (double)af), 0.1);
+        limit = 999;
     }
-    write_obs(a.kind, s, a.next_obs_t + (int64_t)e * a.D);             // the true final observation (autoreset disabled)
+    a.steps[e] += 1;
+    const bool trunc = a.steps[e] >= limit && !term;
+    write_obs<KIND>(s, a.next_obs_t + (int64_t)e * a.D);               // the true final observation (autoreset disabled)
     a.rew_t[e] = (float)reward;
     a.term_t[e] = term ? 1.0f : 0.0f;
     a.trunc_t[e] = trunc ? 1.0f : 0.0f;
@@ -128,14 +223,14 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
     const bool done = term || trunc;
     if (done && a.done_return) a.done_return[e] = (float)ret;
     if (done && a.auto_reset) {
-        reset_state(a, e, s);                                           // envs.reset(options={"reset_mask": dones}), ppo.py:174-179
+        reset_state<KIND>(a, e, s);                                     // envs.reset(options={"reset_mask": dones}), ppo.py:174-179
         a.ep_return[e] = 0.0;
     } else {
         a.ep_return[e] = ret;
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) a.state[(int64_t)e * 4 + i] = s[i];
-    write_obs(a.kind, s, a.cur_obs + (int64_t)e * a.D);
+    write_obs<KIND>(s, a.cur_obs + (int64_t)e * a.D);
 }
 
 // Synthetic environment of the scale benchmark (shape-only stand-in, diamond/envs.py BatchedSyntheticVectorEnv): i.i.d.
@@ -210,22 +305,32 @@ __global__ void synthetic_env_kernel(EnvArgs a, int mode, const unsigned char* _
 
 int launch_env(dppo_ctx* ctx, const EnvArgs& a, int mode, const unsigned char* mask, cudaStream_t st)
 {
-    if (a.kind == 0 || a.kind == 1) {
-        classic_env_kernel<<<(a.N + 127) / 128, 128, 0, st>>>(a, mode, mask);
-        DPPO_CHECK_LAUNCH(ctx, "classic_env_kernel");
-    } else {
+    const unsigned grid = (a.N + 127) / 128;
+    switch (a.kind) {
+    case 0: classic_env_kernel<0><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 1: classic_env_kernel<1><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 4: classic_env_kernel<4><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 5: classic_env_kernel<5><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 6: classic_env_kernel<6><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    default:
         synthetic_env_kernel<<<(unsigned)(((int64_t)a.N * 32 + 255) / 256), 256, 0, st>>>(a, mode, mask);
         DPPO_CHECK_LAUNCH(ctx, "synthetic_env_kernel");
+        return 0;
     }
+    DPPO_CHECK_LAUNCH(ctx, "classic_env_kernel");
     return 0;
 }
 
 int fill_args(dppo_ctx* ctx, const dppo_env_desc* d, const dppo_env_state* s, EnvArgs& a)
 {
     if (!d || !s) DPPO_FAIL(ctx, "env: null descriptor / state");
-    if (d->kind < 0 || d->kind > 3 || d->num_envs < 1) DPPO_FAIL(ctx, "env: bad descriptor (kind %d, num_envs %d)", d->kind, d->num_envs);
-    const int want_d = d->kind == 0 ? 4 : d->kind == 1 ? 3 : d->obs_dim;
-    if (d->obs_dim != want_d || want_d < 1) DPPO_FAIL(ctx, "env: obs_dim %d does not match kind %d", d->obs_dim, d->kind);
+    if (d->kind < 0 || d->kind > 6 || d->num_envs < 1) DPPO_FAIL(ctx, "env: bad descriptor (kind %d, num_envs %d)", d->kind, d->num_envs);
+    static const int kObsDim[7] = {4, 3, 0, 0, 6, 2, 2}, kActDim[7] = {0, 0, 0, 0, 3, 3, 1};   // 0: not checked
+    if (kObsDim[d->kind] && d->obs_dim != kObsDim[d->kind])
+        DPPO_FAIL(ctx, "env: obs_dim %d does not match kind %d (expected %d)", d->obs_dim, d->kind, kObsDim[d->kind]);
+    if (d->obs_dim < 1) DPPO_FAIL(ctx, "env: obs_dim %d does not match kind %d", d->obs_dim, d->kind);
+    if (kActDim[d->kind] && d->act_dim != kActDim[d->kind])
+        DPPO_FAIL(ctx, "env: act_dim %d does not match kind %d (expected %d)", d->act_dim, d->kind, kActDim[d->kind]);
     if (!s->state || !s->steps || !s->episode || !s->ep_return || !s->cur_obs) DPPO_FAIL(ctx, "env: null state buffer");
     a.kind = d->kind; a.N = d->num_envs; a.D = d->obs_dim; a.A = d->act_dim;
     a.state = s->state; a.steps = s->steps; a.episode = s->episode; a.ep_return = s->ep_return; a.cur_obs = s->cur_obs;
@@ -253,7 +358,7 @@ extern "C" int dppo_env_step(dppo_ctx* ctx, const dppo_env_desc* desc, const dpp
     if (fill_args(ctx, desc, state, a)) return 1;
     if (!actions || !next_obs || !rewards || !terminations || !truncations || t < 0) DPPO_FAIL(ctx, "env_step: null output / bad step");
     const int64_t N = a.N, D = a.D;
-    const int cont = (a.kind == 1 || a.kind == 3);
+    const int cont = (a.kind == 1 || a.kind == 3 || a.kind == 6);
     a.t = t; a.auto_reset = auto_reset; a.actions = actions;
     a.obs_t = obs ? obs + (int64_t)t * N * D : nullptr;
     a.next_obs_t = next_obs + (int64_t)t * N * D;

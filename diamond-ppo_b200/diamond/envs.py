@@ -4,9 +4,9 @@ The GPU image has no `gymnasium` (SURVEY.md §7 hard part 6).  The agents only n
 surface the reference touches (diamond/ppo.py:124-130, 163, 174-179, 291, 312): `spaces.Box/Discrete`,
 an `Env` with reset/step, and a `SyncVectorEnv` with autoreset DISABLED whose `reset(options=
 {"reset_mask": mask})` resets only the masked sub-envs.  If the real gymnasium is importable the
-agents use it instead; these classes mirror its semantics.  CartPole-v1 and Pendulum-v1 follow the
-published Gymnasium dynamics; LunarLander needs Box2D, so `SyntheticEnv(8, 4)` stands in for its
-shapes (obs 8, 4 actions).
+agents use it instead; these classes mirror its semantics.  CartPole-v1, Pendulum-v1, Acrobot-v1,
+MountainCar-v0 and MountainCarContinuous-v0 follow the published Gymnasium dynamics; LunarLander needs
+Box2D, so `SyntheticEnv(8, 4)` stands in for its shapes (obs 8, 4 actions).
 """
 from __future__ import annotations
 
@@ -119,6 +119,164 @@ class PendulumEnv(Env):
         return self._obs(), -cost, False, self.t >= self.max_steps, {}
 
 
+def _wrap(x, m, M):
+    """Gymnasium's acrobot `wrap`: add or subtract the period until x lies in [m, M]."""
+    diff = M - m
+    while x > M:
+        x = x - diff
+    while x < m:
+        x = x + diff
+    return x
+
+
+class AcrobotEnv(Env):
+    """Acrobot-v1 (Sutton 1996; Gymnasium classic_control "book" dynamics): one RK4 step of dt 0.2, torque a - 1, 500-step limit."""
+    dt, max_vel_1, max_vel_2, max_steps = 0.2, 4 * np.pi, 9 * np.pi, 500
+    avail_torque = [-1.0, 0.0, +1]
+
+    def __init__(self):
+        high = np.array([1.0, 1.0, 1.0, 1.0, self.max_vel_1, self.max_vel_2], dtype=np.float32)
+        self.observation_space = Box(-high, high, (6,))
+        self.action_space = Discrete(3)
+        self.rng = np.random.default_rng()
+        self.state = np.zeros(4, dtype=np.float32)
+        self.t = 0
+
+    def reset(self, *, seed=None, options=None):
+        if seed is not None:
+            self.rng = np.random.default_rng(seed)
+        self.state = self.rng.uniform(-0.1, 0.1, size=4).astype(np.float32)
+        self.t = 0
+        return self._obs(), {}
+
+    def _obs(self):
+        s = self.state
+        return np.array([np.cos(s[0]), np.sin(s[0]), np.cos(s[1]), np.sin(s[1]), s[2], s[3]], dtype=np.float32)
+
+    @staticmethod
+    def _dsdt(s_augmented):
+        m1, m2, l1, lc1, lc2, I1, I2, g = 1.0, 1.0, 1.0, 0.5, 0.5, 1.0, 1.0, 9.8
+        a = s_augmented[-1]
+        theta1, theta2, dtheta1, dtheta2 = s_augmented[:-1]
+        d1 = m1 * lc1 ** 2 + m2 * (l1 ** 2 + lc2 ** 2 + 2 * l1 * lc2 * np.cos(theta2)) + I1 + I2
+        d2 = m2 * (lc2 ** 2 + l1 * lc2 * np.cos(theta2)) + I2
+        phi2 = m2 * lc2 * g * np.cos(theta1 + theta2 - np.pi / 2.0)
+        phi1 = (-m2 * l1 * lc2 * dtheta2 ** 2 * np.sin(theta2) - 2 * m2 * l1 * lc2 * dtheta2 * dtheta1 * np.sin(theta2)
+                + (m1 * lc1 + m2 * l1) * g * np.cos(theta1 - np.pi / 2) + phi2)
+        ddtheta2 = (a + d2 / d1 * phi1 - m2 * l1 * lc2 * dtheta1 ** 2 * np.sin(theta2) - phi2) / (m2 * lc2 ** 2 + I2 - d2 ** 2 / d1)
+        ddtheta1 = -(d2 * ddtheta2 + phi1) / d1
+        return dtheta1, dtheta2, ddtheta1, ddtheta2, 0.0
+
+    def step(self, action):
+        action = int(action)
+        if not 0 <= action < 3:
+            raise ValueError(f"Acrobot-v1 takes actions 0, 1, 2 (got {action})")
+        torque = self.avail_torque[action]
+        y0 = np.append(self.state, torque)             # float32 state after reset: promoted to float64 here
+        dt = self.dt
+        k1 = np.asarray(self._dsdt(y0))
+        k2 = np.asarray(self._dsdt(y0 + dt / 2.0 * k1))
+        k3 = np.asarray(self._dsdt(y0 + dt / 2.0 * k2))
+        k4 = np.asarray(self._dsdt(y0 + dt * k3))
+        ns = (y0 + dt / 6.0 * (k1 + 2 * k2 + 2 * k3 + k4))[:4]
+        ns[0] = _wrap(ns[0], -np.pi, np.pi)
+        ns[1] = _wrap(ns[1], -np.pi, np.pi)
+        ns[2] = min(max(ns[2], -self.max_vel_1), self.max_vel_1)
+        ns[3] = min(max(ns[3], -self.max_vel_2), self.max_vel_2)
+        self.state = ns
+        self.t += 1
+        terminated = bool(-np.cos(ns[0]) - np.cos(ns[1] + ns[0]) > 1.0)
+        truncated = bool(self.t >= self.max_steps and not terminated)
+        return self._obs(), -1.0 if not terminated else 0.0, terminated, truncated, {}
+
+
+class MountainCarEnv(Env):
+    """MountainCar-v0 (Moore 1990; Gymnasium classic_control): float64 state, force (a - 1) * 0.001, 200-step limit."""
+    min_position, max_position, max_speed, goal_position, force, gravity, max_steps = -1.2, 0.6, 0.07, 0.5, 0.001, 0.0025, 200
+
+    def __init__(self):
+        self.observation_space = Box(np.array([self.min_position, -self.max_speed], dtype=np.float32),
+                                     np.array([self.max_position, self.max_speed], dtype=np.float32), (2,))
+        self.action_space = Discrete(3)
+        self.rng = np.random.default_rng()
+        self.state = np.zeros(2)
+        self.t = 0
+
+    def reset(self, *, seed=None, options=None):
+        if seed is not None:
+            self.rng = np.random.default_rng(seed)
+        self.state = np.array([self.rng.uniform(-0.6, -0.4), 0])
+        self.t = 0
+        return np.array(self.state, dtype=np.float32), {}
+
+    def step(self, action):
+        action = int(action)
+        if not 0 <= action < 3:
+            raise ValueError(f"MountainCar-v0 takes actions 0, 1, 2 (got {action})")
+        position, velocity = self.state
+        velocity += (action - 1) * self.force + math.cos(3 * position) * (-self.gravity)
+        velocity = np.clip(velocity, -self.max_speed, self.max_speed)
+        position += velocity
+        position = np.clip(position, self.min_position, self.max_position)
+        if position == self.min_position and velocity < 0:
+            velocity = 0
+        terminated = bool(position >= self.goal_position and velocity >= 0)
+        self.state = (position, velocity)
+        self.t += 1
+        truncated = bool(self.t >= self.max_steps and not terminated)
+        return np.array(self.state, dtype=np.float32), -1.0, terminated, truncated, {}
+
+
+class MountainCarContinuousEnv(Env):
+    """MountainCarContinuous-v0 (Gymnasium classic_control): float32 state, force min(max(a, -1), 1) * 0.0015, 999-step limit.
+    Every step runs under NumPy 2's promotion rules (NEP 50): float32 arithmetic except math.cos and, for an action outside
+    [-1, 1], the Python-float force term.  The reset state is float32 too, so the first step of an episode is no exception."""
+    min_action, max_action, min_position, max_position, max_speed, goal_position, power, max_steps = \
+        -1.0, 1.0, -1.2, 0.6, 0.07, 0.45, 0.0015, 999
+
+    def __init__(self):
+        self.observation_space = Box(np.array([self.min_position, -self.max_speed], dtype=np.float32),
+                                     np.array([self.max_position, self.max_speed], dtype=np.float32), (2,))
+        self.action_space = Box(self.min_action, self.max_action, (1,))
+        self.rng = np.random.default_rng()
+        self.state = np.zeros(2, dtype=np.float32)
+        self.t = 0
+
+    def reset(self, *, seed=None, options=None):
+        if seed is not None:
+            self.rng = np.random.default_rng(seed)
+        self.state = np.array([self.rng.uniform(-0.6, -0.4), 0], dtype=np.float32)
+        self.t = 0
+        return self.state.copy(), {}
+
+    def step(self, action):
+        action = np.asarray(action, dtype=np.float32).reshape(-1)
+        position = self.state[0]
+        velocity = self.state[1]
+        force = min(max(action[0], self.min_action), self.max_action)
+        velocity += force * self.power - 0.0025 * math.cos(3 * position)
+        if velocity > self.max_speed:
+            velocity = self.max_speed
+        if velocity < -self.max_speed:
+            velocity = -self.max_speed
+        position += velocity
+        if position > self.max_position:
+            position = self.max_position
+        if position < self.min_position:
+            position = self.min_position
+        if position == self.min_position and velocity < 0:
+            velocity = 0
+        terminated = bool(position >= self.goal_position and velocity >= 0)
+        reward = 0
+        if terminated:
+            reward = 100.0
+        reward -= math.pow(action[0], 2) * 0.1
+        self.state = np.array([position, velocity], dtype=np.float32)
+        self.t += 1
+        truncated = bool(self.t >= self.max_steps and not terminated)
+        return self.state.copy(), reward, terminated, truncated, {}
+
+
 class SyntheticEnv(Env):
     """Shape-only stand-in (e.g. LunarLander-v3: obs 8, 4 actions): i.i.d. normal observations,
     reward depends on (obs, action), random terminations/truncations."""
@@ -214,8 +372,9 @@ class BatchedSyntheticVectorEnv:
 
 
 class DeviceVectorEnv:
-    """Vector environment that lives on the GPU (csrc/envs.cu: dppo_env_step / dppo_env_reset): CartPole-v1, Pendulum-v1
-    (Gymnasium classic-control dynamics, float64 state) and the synthetic shape stand-ins.  Same vector API and
+    """Vector environment that lives on the GPU (csrc/envs.cu: dppo_env_step / dppo_env_reset): CartPole-v1, Pendulum-v1,
+    Acrobot-v1, MountainCar-v0, MountainCarContinuous-v0 (Gymnasium classic-control dynamics, float64 state; the continuous
+    mountain car keeps Gymnasium's float32 state) and the synthetic shape stand-ins.  Same vector API and
     autoreset-DISABLED semantics as SyncVectorEnv, so any agent or user code can drive it through `step` / `reset` with host
     arrays; the default-network agents use `step_into`, which writes the step straight into the device rollout buffer and
     resets finished environments inside the same kernel (diamond/ppo.py:160-182 without a PCIe crossing).
@@ -223,7 +382,8 @@ class DeviceVectorEnv:
     Use as `env_fn = DeviceVectorEnv.factory("CartPole-v1")` (an `env_fn.vectorized` factory taking num_envs)."""
 
     device_resident = True
-    _KINDS = {"CartPole-v1": (0, 4, 2, False), "Pendulum-v1": (1, 3, 1, True)}
+    _KINDS = {"CartPole-v1": (0, 4, 2, False), "Pendulum-v1": (1, 3, 1, True), "Acrobot-v1": (4, 6, 3, False),
+              "MountainCar-v0": (5, 2, 3, False), "MountainCarContinuous-v0": (6, 2, 1, True)}
 
     def __init__(self, env_id: str, num_envs: int, seed: int = 0, device=None, obs_dim: int = 64, n_actions: int = 4,
                  continuous: bool = False, p_term: float = 0.01, p_trunc: float = 0.01, env_offset: int = 0):
@@ -246,10 +406,17 @@ class DeviceVectorEnv:
         elif kind == 1:
             high = np.array([1.0, 1.0, 8.0], dtype=np.float32)
             self.single_observation_space, self.single_action_space = Box(-high, high, (3,)), Box(-2.0, 2.0, (1,))
+        elif kind == 4:
+            high = np.array([1.0, 1.0, 1.0, 1.0, 4 * np.pi, 9 * np.pi], dtype=np.float32)
+            self.single_observation_space, self.single_action_space = Box(-high, high, (6,)), Discrete(3)
+        elif kind in (5, 6):
+            self.single_observation_space = Box(np.array([-1.2, -0.07], dtype=np.float32), np.array([0.6, 0.07], dtype=np.float32), (2,))
+            self.single_action_space = Box(-1.0, 1.0, (1,)) if kind == 6 else Discrete(3)
         else:
             self.single_observation_space = Box(-np.inf, np.inf, (D,))
             self.single_action_space = Box(-1.0, 1.0, (A,)) if cont else Discrete(A)
         self.obs_dim, self.act_dim = D, A
+        self._check_actions = kind in (4, 5)       # a host array may hold anything; the sampler's output is in range
         self.desc = N.EnvDesc(kind, self.num_envs, D, A, int(seed) & (2 ** 64 - 1), int(env_offset), float(p_term), float(p_trunc))
         n, dev = self.num_envs, self.device
         self.state = torch.zeros(n, 4, dtype=torch.float64, device=dev)
@@ -293,8 +460,10 @@ class DeviceVectorEnv:
     def step(self, actions):
         """Gymnasium vector API with host arrays (autoreset disabled: the caller resets through reset(options=...))."""
         r = self._row
-        self.ctx.env_step(self.desc, self._st, self._actions(actions), 0, False, None, r["next_obs"], None, r["rew"], r["term"],
-                          r["trunc"])
+        a = self._actions(actions)
+        if self._check_actions and bool(((a < 0) | (a >= self.act_dim)).any()):
+            raise ValueError(f"{self.env_id} takes actions 0 .. {self.act_dim - 1}; got {a.min().item()} .. {a.max().item()}")
+        self.ctx.env_step(self.desc, self._st, a, 0, False, None, r["next_obs"], None, r["rew"], r["term"], r["trunc"])
         return (r["next_obs"][0].cpu().numpy(), r["rew"][0].double().cpu().numpy(), r["term"][0].bool().cpu().numpy(),
                 r["trunc"][0].bool().cpu().numpy(), {})
 
@@ -309,7 +478,8 @@ class DeviceVectorEnv:
         pass
 
 
-_REGISTRY = {"CartPole-v1": CartPoleEnv, "Pendulum-v1": PendulumEnv,
+_REGISTRY = {"CartPole-v1": CartPoleEnv, "Pendulum-v1": PendulumEnv, "Acrobot-v1": AcrobotEnv, "MountainCar-v0": MountainCarEnv,
+             "MountainCarContinuous-v0": MountainCarContinuousEnv,
              "LunarLander-v3": lambda: SyntheticEnv(8, 4)}       # Box2D unavailable: shape stand-in
 
 

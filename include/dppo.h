@@ -339,15 +339,16 @@ int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* desc, const floa
 /* ---- device-resident vectorised environments (SURVEY.md 8f-1) ------------------------------------ */
 /* Replaces the host `envs.step(actions)` + `envs.reset(options={"reset_mask": dones})` + list append of a rollout step
  * (diamond/ppo.py:160-182): one kernel steps all environments and writes row t of the time-major rollout buffers.
- * kind 0: CartPole-v1, 1: Pendulum-v1 (Gymnasium classic-control dynamics, float64 state), 2 / 3: synthetic discrete /
+ * kind 0: CartPole-v1, 1: Pendulum-v1, 4: Acrobot-v1, 5: MountainCar-v0, 6: MountainCarContinuous-v0 (Gymnasium
+ * classic-control dynamics, float64 state; MountainCarContinuous keeps Gymnasium's float32 state), 2 / 3: synthetic discrete /
  * continuous (i.i.d. normal observations; the scale benchmark's shape stand-in).  Autoreset-DISABLED contract: next_obs[t]
  * is the true final observation; with auto_reset != 0 finished environments are then reset inside the same kernel and
  * cur_obs holds the post-reset observation (ppo.py:174-179), else the caller resets them with dppo_env_reset(mask). */
 typedef struct dppo_env_desc {
     int32_t kind;
     int32_t num_envs;
-    int32_t obs_dim;        /* 4 (CartPole), 3 (Pendulum), any (synthetic) */
-    int32_t act_dim;        /* Discrete.n, or action dims when continuous */
+    int32_t obs_dim;        /* 4 (CartPole), 3 (Pendulum), 6 (Acrobot), 2 (MountainCar, MountainCarContinuous), any (synthetic) */
+    int32_t act_dim;        /* Discrete.n, or action dims when continuous: 3 (Acrobot, MountainCar), 1 (MountainCarContinuous) */
     uint64_t seed;          /* reset / synthetic draws: Philox4x32-10 keyed by (seed, env_offset + env, episode or step) */
     int64_t env_offset;     /* global id of env 0 (env-sharded data parallelism) */
     float p_term, p_trunc;  /* synthetic kinds only */
