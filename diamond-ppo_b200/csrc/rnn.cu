@@ -860,7 +860,8 @@ int launch_scan_bwd(dppo_ctx* ctx, const ScanBwdArgs& a, cudaStream_t st)
 
 int check_desc(dppo_ctx* ctx, const dppo_rnn_desc* d)
 {
-    if (!d || d->obs_dim < 1 || d->hidden < 1 || d->gru_hidden < 1 || d->act_dim < 1) DPPO_FAIL(ctx, "rnn: bad descriptor");
+    if (!d || d->obs_dim < 1 || d->hidden < 1 || d->gru_hidden < 1 || d->act_dim < 1 || (d->continuous != 0 && d->continuous != 1))
+        DPPO_FAIL(ctx, "rnn: bad descriptor");
     if (d->gru_hidden > 512) DPPO_FAIL(ctx, "rnn: gru_hidden_dim %d > 512 is not supported", d->gru_hidden);
     if (d->hidden > 512) DPPO_FAIL(ctx, "rnn: network_hidden_dim %d > 512 is not supported", d->hidden);
     if (d->act_dim > DPPO_MAX_ACT) DPPO_FAIL(ctx, "rnn: more than %d actions", DPPO_MAX_ACT);
@@ -933,7 +934,8 @@ int rnn_trunk_forward(dppo_ctx* ctx, const dppo_rnn_desc* d, const dppo_rnn_layo
 
 extern "C" int dppo_rnn_layout_compute(const dppo_rnn_desc* d, dppo_rnn_layout* L)
 {
-    if (!d || !L || d->obs_dim < 1 || d->hidden < 1 || d->gru_hidden < 1 || d->act_dim < 1) return 1;
+    if (!d || !L || d->obs_dim < 1 || d->hidden < 1 || d->gru_hidden < 1 || d->act_dim < 1 || (d->continuous != 0 && d->continuous != 1))
+        return 1;
     const int64_t D = d->obs_dim, H = d->hidden, Hg = d->gru_hidden, A = d->act_dim;
     int64_t o = 0;
     auto take = [&](int64_t n) { int64_t p = o; o += (n + 3) / 4 * 4; return p; };
@@ -942,6 +944,7 @@ extern "C" int dppo_rnn_layout_compute(const dppo_rnn_desc* d, dppo_rnn_layout* 
     L->w3 = take(2 * H * Hg); L->b3 = take(2 * H);
     L->wa = take(A * H); L->ba = take(A);
     L->wc = take(H); L->bc = take(1);
+    L->log_std = d->continuous ? take(A) : -1;
     L->total = o;
     return 0;
 }
@@ -982,7 +985,7 @@ extern "C" int dppo_rnn_forward(dppo_ctx* ctx, const dppo_rnn_desc* d, const flo
 }
 
 extern "C" int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* d, const float* params, float* grads, const float* obs,
-                                       const unsigned char* prev_dones, const float* hx0, int T, int N, const int32_t* actions,
+                                       const unsigned char* prev_dones, const float* hx0, int T, int N, const void* actions,
                                        const float* old_log_probs, const float* adv, const float* returns, const double* adv_stats,
                                        const int32_t* idx, int64_t M, const dppo_hyper* hy, float* losses, void* ws,
                                        int64_t ws_bytes, void* stream)
@@ -994,6 +997,9 @@ extern "C" int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* d, co
     if (T < 1 || N < 1 || M < 1 || M > (int64_t)T * N) DPPO_FAIL(ctx, "rnn_grad_minibatch: bad shape T=%d N=%d M=%lld", T, N, (long long)M);
     if (!idx && M != (int64_t)T * N) DPPO_FAIL(ctx, "rnn_grad_minibatch: a partial minibatch needs row indices");
     if (hy->advantage_norm && (!adv_stats || hy->adv_count < 2)) DPPO_FAIL(ctx, "rnn_grad_minibatch: advantage_norm needs adv_stats and adv_count >= 2");
+    if (!head_train_supported(d->hidden, d->act_dim))
+        DPPO_FAIL(ctx, "rnn_grad_minibatch: the head kernel's per-warp accumulators, 9 (act_dim + 1) hidden = %d floats, exceed its 200 KB "
+                  "of shared memory", 9 * (d->act_dim + 1) * d->hidden);
     dppo_rnn_layout L;
     dppo_rnn_layout_compute(d, &L);
     const int D = d->obs_dim, H = d->hidden, Hg = d->gru_hidden, A = d->act_dim;
@@ -1012,16 +1018,17 @@ extern "C" int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* d, co
     HeadTrainArgs ha;
     ha.h3 = w.h3; ha.d3 = w.d3;
     ha.wa = params + L.wa; ha.ba = params + L.ba; ha.wc = params + L.wc; ha.bc = params + L.bc;
-    ha.log_std = nullptr;
+    ha.log_std = d->continuous ? params + L.log_std : nullptr;
     ha.idx = idx;
-    ha.actions_i = actions; ha.actions_f = nullptr;
+    ha.actions_i = d->continuous ? nullptr : static_cast<const int32_t*>(actions);
+    ha.actions_f = d->continuous ? static_cast<const float*>(actions) : nullptr;
     ha.old_logp = old_log_probs; ha.adv = adv; ha.ret = returns;
     ha.adv_stats = adv_stats; ha.adv_count = hy->adv_count; ha.advantage_norm = hy->advantage_norm;
     ha.M = M; ha.H = H; ha.A = A;
     ha.clip = hy->ppo_clip; ha.vw = hy->value_loss_weight; ha.beta = hy->entropy_beta; ha.inv_m = inv_m;
     ha.partials = w.hp; ha.partial_stride = w.head_stride;
     ha.rev = 0; ha.keep_d3 = 0; ha.h3_first = 0;
-    if (launch_head_train_kernel(ctx, ha, 0, w.head_blocks, st)) return 1;
+    if (launch_head_train_kernel(ctx, ha, d->continuous, w.head_blocks, st)) return 1;
 
     // d(loss)/d(h_t): rows of the minibatch, zero for every other (t, env)
     float* dh_rows = idx ? w.dhm : w.dhs;
@@ -1065,6 +1072,7 @@ extern "C" int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* d, co
     seg(L.ba, A, w.hp + ho.dba, w.head_stride, w.head_blocks);
     seg(L.wc, H, w.hp + ho.dwc, w.head_stride, w.head_blocks);
     seg(L.bc, 1, w.hp + ho.dbc, w.head_stride, w.head_blocks);
+    if (d->continuous) seg(L.log_std, A, w.hp + ho.dls, w.head_stride, w.head_blocks);
     tab.nseg = n;
     return launch_grad_reduce(ctx, tab, grads, L.total, w.hp + ho.loss, w.head_blocks, w.head_stride, hy->value_loss_weight,
                               hy->entropy_beta, inv_m, losses, hy->grad_sumsq, st);

@@ -1,10 +1,11 @@
 """diamond — B200-native drop-in for the hot path of Diamond PPO (same import surface as the
 reference package: diamond/__init__.py:1-3).  Submodules are imported on first use."""
-__all__ = ["PPO", "PPOConfig", "ContinuousPPO", "ContinuousPPOConfig", "RecurrentPPO", "RecurrentPPOConfig"]
+__all__ = ["PPO", "PPOConfig", "ContinuousPPO", "ContinuousPPOConfig", "RecurrentPPO", "RecurrentPPOConfig",
+           "RecurrentContinuousPPO", "RecurrentContinuousPPOConfig"]
 
 _WHERE = {
-    "PPO": "agents", "ContinuousPPO": "agents", "RecurrentPPO": "recurrent",
-    "PPOConfig": "config", "ContinuousPPOConfig": "config", "RecurrentPPOConfig": "config",
+    "PPO": "agents", "ContinuousPPO": "agents", "RecurrentPPO": "recurrent", "RecurrentContinuousPPO": "recurrent",
+    "PPOConfig": "config", "ContinuousPPOConfig": "config", "RecurrentPPOConfig": "config", "RecurrentContinuousPPOConfig": "config",
 }
 
 

@@ -29,11 +29,11 @@ class MlpLayout(C.Structure):
 
 
 class RnnDesc(C.Structure):
-    _fields_ = [("obs_dim", C.c_int32), ("hidden", C.c_int32), ("gru_hidden", C.c_int32), ("act_dim", C.c_int32)]
+    _fields_ = [("obs_dim", C.c_int32), ("hidden", C.c_int32), ("gru_hidden", C.c_int32), ("act_dim", C.c_int32), ("continuous", C.c_int32)]
 
 
 class RnnLayout(C.Structure):
-    _fields_ = [(n, C.c_int64) for n in ("w1", "b1", "wih", "whh", "bih", "bhh", "w3", "b3", "wa", "ba", "wc", "bc", "total")]
+    _fields_ = [(n, C.c_int64) for n in ("w1", "b1", "wih", "whh", "bih", "bhh", "w3", "b3", "wa", "ba", "wc", "bc", "log_std", "total")]
 
 
 class EnvDesc(C.Structure):

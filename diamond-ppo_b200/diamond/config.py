@@ -1,7 +1,8 @@
-"""Hyper-parameter dataclasses, field-for-field identical to the reference so that user code and
-subclasses (notebook cell 9) keep working: diamond/ppo.py:15-37, diamond/continuous_ppo.py:15-37,
-diamond/recurrent_ppo.py:15-38.  Fields and defaults are the reference's; nothing is added here —
-B200-specific knobs are keyword arguments of the agents, never config fields."""
+"""Hyper-parameter dataclasses.  PPOConfig, ContinuousPPOConfig and RecurrentPPOConfig are field-for-field
+identical to the reference's so that user code and subclasses (notebook cell 9) keep working: diamond/ppo.py:15-37,
+diamond/continuous_ppo.py:15-37, diamond/recurrent_ppo.py:15-38.  RecurrentContinuousPPOConfig (the Gaussian-policy
+recurrent agent, which the reference does not have) has RecurrentPPOConfig's fields and defaults, as ContinuousPPOConfig
+has PPOConfig's.  B200-specific knobs are keyword arguments of the agents, never config fields."""
 from dataclasses import dataclass
 
 
@@ -52,6 +53,16 @@ class _RecurrentExtra:
 @dataclass
 class RecurrentPPOConfig(_TailConfig, _RecurrentExtra, _CommonConfig):
     # recurrent defaults differ (recurrent_ppo.py:18-19,25-27)
+    rollout_steps: int = 32
+    num_envs: int = 32
+    num_epochs: int = 10
+    num_minibatches: int = 1
+    ppo_clip: float = 0.15
+
+
+@dataclass
+class RecurrentContinuousPPOConfig(_TailConfig, _RecurrentExtra, _CommonConfig):
+    # RecurrentPPOConfig's defaults
     rollout_steps: int = 32
     num_envs: int = 32
     num_epochs: int = 10

@@ -14,6 +14,10 @@ GEMM over all T steps followed by T hidden-state steps, instead of T one-step `n
 advantage normalisation, the bit-exact minibatch permutation, the PPO loss forward/backward, gradient clipping and Adam run
 on the libdppo kernels (`RecurrentEngine`).  The reference's `hx or zeros` / `dones or zeros` lines (recurrent_ppo.py:78-79) raise on
 every call; the intended `is None` semantics are implemented (SURVEY.md §0.4).
+
+Beyond the reference: `RecurrentContinuousPPO` / `RecurrentContinuousActorCriticNetwork`, the same agent with a Gaussian policy for
+Box action spaces (the heads of continuous_ppo.py on the GRU trunk).  It runs the same code, selected by the class attribute
+`_continuous` as in agents.py, and the same kernels (the Gaussian instantiation of the head kernel in dppo_rnn_grad_minibatch).
 """
 from __future__ import annotations
 
@@ -31,7 +35,7 @@ try:                                    # the real package when present, else th
 except ImportError:                     # pragma: no cover - the GPU image has no gymnasium
     from . import envs as gym
 from .agents import _Dist, _EngineBase, _PermWorker, _PPOBase, _require_cuda
-from .config import RecurrentPPOConfig
+from .config import RecurrentContinuousPPOConfig, RecurrentPPOConfig
 from .networks import _obs_dim, network_parameter_init_
 from .utils import Checkpointer, Logger, Ticker, Timer
 
@@ -88,15 +92,41 @@ class RecurrentActorCriticNetwork(nn.Module):
         return self.actor_head(x), self.critic_head(x).squeeze(-1), hx
 
 
+class RecurrentContinuousActorCriticNetwork(nn.Module):
+    """Linear-Tanh -> GRU -> Gaussian actor (mean head + state-independent log-std parameter (1, A), as in
+    ContinuousActorCriticNetwork) / critic head."""
+
+    def __init__(self, observation_space, action_space, cfg: RecurrentContinuousPPOConfig) -> None:
+        super().__init__()
+        assert hasattr(action_space, "shape") and not hasattr(action_space, "n"), "Only Box action spaces are supported."
+        d, h, hg = _obs_dim(observation_space), int(cfg.network_hidden_dim), int(cfg.gru_hidden_dim)
+        a = int(np.prod(action_space.shape))
+        self.base = nn.Sequential(nn.Linear(d, h), nn.Tanh())
+        self.gru = GRUCore(h, hg)
+        self.actor_mean_head = nn.Sequential(nn.Linear(hg, h), nn.Tanh(), nn.Linear(h, a))
+        self.actor_log_std = nn.Parameter(torch.zeros(1, a))
+        self.critic_head = nn.Sequential(nn.Linear(hg, h), nn.Tanh(), nn.Linear(h, 1))
+
+    def get_values(self, observations, hx, dones) -> torch.Tensor:
+        x, _ = self.gru.forward(self.base(observations), hx, dones)
+        return self.critic_head(x).squeeze(-1)
+
+    def get_means_log_stds_values_and_hx(self, observations, hx, dones):
+        """(mean [T,B,A], log_std broadcast to [T,B,A], values [T,B], hx [1,B,Hg])."""
+        x, hx = self.gru.forward(self.base(observations), hx, dones)
+        mean = self.actor_mean_head(x)
+        return mean, torch.broadcast_to(self.actor_log_std, mean.shape), self.critic_head(x).squeeze(-1), hx
+
+
 class RecurrentRollout:
     """Device-resident rollout of the recurrent agent; iterating yields the reference's 10-item step records
-    (recurrent_ppo.py:234-245)."""
+    (recurrent_ppo.py:234-245).  Actions: int64 [T, N], or f32 [T, N, act_dim] when act_dim is given (Gaussian policy)."""
 
-    def __init__(self, T, N_, D, Hg, device):
+    def __init__(self, T, N_, D, Hg, device, act_dim=None):
         f = dict(dtype=torch.float32, device=device)
         self.T, self.N = T, N_
         self.obs = torch.empty(T, N_, D, **f)
-        self.actions = torch.empty(T, N_, dtype=torch.int64, device=device)
+        self.actions = torch.empty(T, N_, dtype=torch.int64, device=device) if act_dim is None else torch.empty(T, N_, act_dim, **f)
         self.rewards, self.terminations, self.truncations = (torch.empty(T, N_, **f) for _ in range(3))
         self.prev_dones = torch.empty(T, N_, dtype=torch.bool, device=device)
         self.log_probs, self.values, self.next_values = (torch.empty(T, N_, **f) for _ in range(3))
@@ -104,15 +134,16 @@ class RecurrentRollout:
         self.filled = 0
 
     @staticmethod
-    def from_lists(experience, device) -> "RecurrentRollout":
+    def from_lists(experience, device, continuous=False) -> "RecurrentRollout":
         cols = list(zip(*experience))
         dev_t = lambda x, dt: torch.as_tensor(np.asarray(x) if not torch.is_tensor(x) else x).to(device=device, dtype=dt)
         obs = torch.stack([dev_t(o, torch.float32) for o in cols[0]])
         T, N_, D = obs.shape
         hx0 = dev_t(cols[9][0], torch.float32).clone()                  # recurrent_ppo.py:313
-        r = RecurrentRollout(T, N_, D, hx0.shape[-1], device)
+        actions = torch.stack([dev_t(a, torch.float32 if continuous else torch.int64) for a in cols[1]])
+        r = RecurrentRollout(T, N_, D, hx0.shape[-1], device, actions.reshape(T, N_, -1).shape[-1] if continuous else None)
         r.obs.copy_(obs)
-        r.actions.copy_(torch.stack([dev_t(a, torch.int64) for a in cols[1]]))
+        r.actions.copy_(actions.reshape(r.actions.shape))
         r.rewards.copy_(dev_t(np.asarray([np.asarray(x) for x in cols[2]]), torch.float32))       # f64 -> f32 (:306)
         r.terminations.copy_(dev_t(np.asarray([np.asarray(x) for x in cols[3]]), torch.float32))
         r.truncations.copy_(dev_t(np.asarray([np.asarray(x) for x in cols[4]]), torch.float32))
@@ -137,8 +168,8 @@ class RecurrentRollout:
 class RecurrentEngine(_EngineBase):
     """learn() of the recurrent agent: sequence forward/backward under autograd, everything else on libdppo kernels."""
 
-    def __init__(self, ctx, network, cfg, device, dist: _Dist | None = None):
-        self.ctx, self.cfg, self.device = ctx, cfg, device
+    def __init__(self, ctx, network, cfg, device, dist: _Dist | None = None, continuous=False):
+        self.ctx, self.cfg, self.device, self.continuous = ctx, cfg, device, continuous
         self.dist = dist if dist is not None else _Dist(None, False)
         self.network = network
         offsets, o = {}, 0
@@ -177,8 +208,12 @@ class RecurrentEngine(_EngineBase):
         hyper = self._hyper(cfg, M * dist.world, B * dist.world)
         hyper.advantage_norm = 0                                         # already normalised above
         old_logp, adv_f, ret_f = ro.log_probs.reshape(B).contiguous(), adv.view(B), ret.view(B)
-        act_bits = ro.actions.reshape(B).to(torch.int32).view(torch.float32)
-        A = net.actor_out_layer.out_features
+        if self.continuous:
+            A = ro.actions.shape[-1]
+            act_bits = ro.actions.reshape(B, A).contiguous()
+        else:
+            act_bits = ro.actions.reshape(B).to(torch.int32).view(torch.float32)
+            A = net.actor_out_layer.out_features
         losses = torch.zeros(E * MB, 4, device=dev)
         loss_ws = torch.empty(ctx.ppo_loss_workspace_bytes(M, max(A, 32)) // 4 + 64, device=dev)
         idx = torch.empty(E, B, dtype=torch.int32, device=dev)
@@ -195,13 +230,23 @@ class RecurrentEngine(_EngineBase):
                 hyper.step = self.adam_step
                 self.G.zero_()
                 # full-sequence forward with the current parameters, then the minibatch rows (recurrent_ppo.py:337-341)
-                logits, values, _ = net.get_logits_values_and_hx(ro.obs, hx0, ro.prev_dones)
-                logits_mb = logits.reshape(B, A).index_select(0, mb64).contiguous()
-                val_mb = values.reshape(B).index_select(0, mb64).contiguous()
-                dlogits, dval = torch.empty_like(logits_mb), torch.empty_like(val_mb)
-                ctx.ppo_loss_discrete(logits_mb.detach(), val_mb.detach(), a_mb.view(torch.int32), lp_mb, adv_mb, ret_mb, hyper,
-                                      losses[e * MB + k], dlogits, dval, loss_ws)
-                torch.autograd.backward([logits_mb, val_mb], [dlogits, dval])
+                if self.continuous:
+                    means, log_stds, values, _ = net.get_means_log_stds_values_and_hx(ro.obs, hx0, ro.prev_dones)
+                    mean_mb = means.reshape(B, A).index_select(0, mb64).contiguous()
+                    ls_mb = log_stds.reshape(B, A).index_select(0, mb64).contiguous()
+                    val_mb = values.reshape(B).index_select(0, mb64).contiguous()
+                    dmean, dls, dval = torch.empty_like(mean_mb), torch.empty_like(ls_mb), torch.empty_like(val_mb)
+                    ctx.ppo_loss_gaussian(mean_mb.detach(), ls_mb.detach(), val_mb.detach(), a_mb, lp_mb, adv_mb, ret_mb, hyper,
+                                          losses[e * MB + k], dmean, dls, dval, loss_ws, log_std_row_stride=A)
+                    torch.autograd.backward([mean_mb, ls_mb, val_mb], [dmean, dls, dval])
+                else:
+                    logits, values, _ = net.get_logits_values_and_hx(ro.obs, hx0, ro.prev_dones)
+                    logits_mb = logits.reshape(B, A).index_select(0, mb64).contiguous()
+                    val_mb = values.reshape(B).index_select(0, mb64).contiguous()
+                    dlogits, dval = torch.empty_like(logits_mb), torch.empty_like(val_mb)
+                    ctx.ppo_loss_discrete(logits_mb.detach(), val_mb.detach(), a_mb.view(torch.int32), lp_mb, adv_mb, ret_mb, hyper,
+                                          losses[e * MB + k], dlogits, dval, loss_ws)
+                    torch.autograd.backward([logits_mb, val_mb], [dlogits, dval])
                 if dist.enabled:
                     dist.all_reduce_sum(self.G)
                     dist.all_reduce_sum(losses[e * MB + k])
@@ -212,17 +257,22 @@ class RecurrentEngine(_EngineBase):
 
 
 def rnn_param_slices(desc: N.RnnDesc, lay: N.RnnLayout):
-    """name (reference module naming, recurrent_ppo.py:101-125) -> (offset, shape) in the flat buffers (dppo_rnn_layout)."""
+    """name (reference module naming, recurrent_ppo.py:101-125; RecurrentContinuousActorCriticNetwork's when desc.continuous)
+    -> (offset, shape) in the flat buffers (dppo_rnn_layout)."""
     D, H, Hg, A = desc.obs_dim, desc.hidden, desc.gru_hidden, desc.act_dim
-    return {
+    actor = "actor_mean_head" if desc.continuous else "actor_head"
+    s = {
         "base.0.weight": (lay.w1, (H, D)), "base.0.bias": (lay.b1, (H,)),
         "gru.weight_ih_l0": (lay.wih, (3 * Hg, H)), "gru.weight_hh_l0": (lay.whh, (3 * Hg, Hg)),
         "gru.bias_ih_l0": (lay.bih, (3 * Hg,)), "gru.bias_hh_l0": (lay.bhh, (3 * Hg,)),
-        "actor_head.0.weight": (lay.w3, (H, Hg)), "actor_head.0.bias": (lay.b3, (H,)),
-        "actor_head.2.weight": (lay.wa, (A, H)), "actor_head.2.bias": (lay.ba, (A,)),
+        f"{actor}.0.weight": (lay.w3, (H, Hg)), f"{actor}.0.bias": (lay.b3, (H,)),
+        f"{actor}.2.weight": (lay.wa, (A, H)), f"{actor}.2.bias": (lay.ba, (A,)),
         "critic_head.0.weight": (lay.w3 + H * Hg, (H, Hg)), "critic_head.0.bias": (lay.b3 + H, (H,)),
         "critic_head.2.weight": (lay.wc, (1, H)), "critic_head.2.bias": (lay.bc, (1,)),
     }
+    if desc.continuous:
+        s["actor_log_std"] = (lay.log_std, (1, A))
+    return s
 
 
 class FusedRecurrentEngine(_EngineBase):
@@ -230,13 +280,15 @@ class FusedRecurrentEngine(_EngineBase):
 
     fused = True
 
-    def __init__(self, ctx, network, cfg, obs_dim, act_dim, device, dist: _Dist | None = None):
-        self.ctx, self.cfg, self.device = ctx, cfg, device
+    def __init__(self, ctx, network, cfg, obs_dim, act_dim, device, dist: _Dist | None = None, continuous=False):
+        self.ctx, self.cfg, self.device, self.continuous = ctx, cfg, device, continuous
         self.dist = dist if dist is not None else _Dist(None, False)
         self.network = network
-        self.desc = N.RnnDesc(int(obs_dim), int(cfg.network_hidden_dim), int(cfg.gru_hidden_dim), int(act_dim))
+        self.desc = N.RnnDesc(int(obs_dim), int(cfg.network_hidden_dim), int(cfg.gru_hidden_dim), int(act_dim), int(continuous))
         self.layout = N.rnn_layout(self.desc)
         self._adopt(network, rnn_param_slices(self.desc, self.layout), int(self.layout.total))
+        # Gaussian policy: the actor_log_std [A] the sampling kernel reads (a view of the flat parameter buffer)
+        self.log_std = self.P[self.layout.log_std:self.layout.log_std + int(act_dim)] if continuous else None
         self.last_losses = None
         self.draws = 0
         self.seed = self.dist.shared_seed(cfg.seed if cfg.seed is not None else (None if self.dist.enabled else int(np.random.randint(0, 2 ** 31 - 1))), device)
@@ -253,7 +305,8 @@ class FusedRecurrentEngine(_EngineBase):
         return self._ws[key]
 
     def forward(self, obs, hx, prev_dones, heads=3):
-        """(logits [T,N,A], values [T,N], hx [1,N,Hg]) of get_logits_values_and_hx / get_values (recurrent_ppo.py:127-149)."""
+        """(logits [T,N,A], values [T,N], hx [1,N,Hg]) of get_logits_values_and_hx / get_values (recurrent_ppo.py:127-149); with
+        a Gaussian policy the first output holds the action means."""
         T, N_ = obs.shape[:2]
         dev, A, Hg = self.device, self.desc.act_dim, self.desc.gru_hidden
         logits = torch.empty(T, N_, A, device=dev) if heads & 1 else None
@@ -273,7 +326,8 @@ class FusedRecurrentEngine(_EngineBase):
                 stats=torch.zeros(2, dtype=torch.float64, device=dev), adv=torch.empty(T, N_, device=dev), ret=torch.empty(T, N_, device=dev),
                 losses=torch.zeros(E * MB, 4, device=dev), idx=[torch.empty(B, dtype=torch.int32, device=dev) for _ in range(2)],
                 h_sets=[[torch.empty(B, dtype=torch.int32).pin_memory() for _ in range(E)] for _ in range(2)], h_set=0, h_consumed=[None, None],
-                old_logp=torch.empty(B, device=dev), actions=torch.empty(B, dtype=torch.int32, device=dev),
+                old_logp=torch.empty(B, device=dev),
+                actions=torch.empty(B, self.desc.act_dim, device=dev) if self.continuous else torch.empty(B, dtype=torch.int32, device=dev),
                 pd=torch.empty(T, N_, dtype=torch.uint8, device=dev), hx0=torch.empty(N_, self.desc.gru_hidden, device=dev),
                 values=torch.empty(T, N_, device=dev), next_values=torch.empty(T, N_, device=dev),
                 consts=[torch.zeros(MB, 4, dtype=torch.float32, device=dev) for _ in range(2)],
@@ -299,7 +353,7 @@ class FusedRecurrentEngine(_EngineBase):
         worker = _PermWorker(B, E, MB, [h.numpy() for h in h_idx])
         worker.start()
         # learn()-persistent copies in the kernels' dtypes (stable addresses: the optimiser steps are replayed as a CUDA graph)
-        b["old_logp"].copy_(ro.log_probs.reshape(B)); b["actions"].copy_(ro.actions.reshape(B))
+        b["old_logp"].copy_(ro.log_probs.reshape(B)); b["actions"].copy_(ro.actions.reshape(b["actions"].shape))
         b["pd"].copy_(ro.prev_dones); b["hx0"].copy_(ro.hx0.reshape(N_, -1))
         b["values"].copy_(ro.values); b["next_values"].copy_(ro.next_values)
         # GAE with the values stored at rollout time + returns + advantage sums (recurrent_ppo.py:315-318); the normalisation
@@ -384,6 +438,8 @@ class FusedRecurrentEngine(_EngineBase):
 
 class RecurrentPPO:
     """Recurrent (GRU) discrete-action PPO (reference: diamond/recurrent_ppo.py:164-394)."""
+    _continuous = False
+    _default_network: Any = RecurrentActorCriticNetwork
 
     def __init__(self, env_fn: Callable[[], Any], cfg: RecurrentPPOConfig = RecurrentPPOConfig(),
                  network_cls: Any = RecurrentActorCriticNetwork, *, process_group=None, dp: bool = False) -> None:
@@ -403,15 +459,18 @@ class RecurrentPPO:
             self.envs = gym.vector.SyncVectorEnv([env_fn for _ in range(cfg.num_envs)], copy=True, autoreset_mode="Disabled")
         obs_space, act_space = self.envs.single_observation_space, self.envs.single_action_space
         self.network = network_cls(obs_space, act_space, cfg=cfg).to(self.device)
-        network_parameter_init_(self.network, gain=sqrt(2.0), small_actor_out=True)     # touches nn.Linear only (:152-161)
+        # touches nn.Linear only (:152-161); no 0.01-gain output layer for the Gaussian policy (continuous_ppo.py:114-121)
+        network_parameter_init_(self.network, gain=sqrt(2.0), small_actor_out=not self._continuous)
         if self._dist.enabled:                                           # replicas start from rank 0's parameters
             for p in self.network.parameters():
                 self._dist.dist.broadcast(p.data, src=0, group=self._dist.group)
         self.obs_dim = int(np.prod(obs_space.shape))
-        if type(self.network) is RecurrentActorCriticNetwork:            # default network: libdppo kernels end to end
-            self.engine = FusedRecurrentEngine(self.ctx, self.network, cfg, self.obs_dim, int(act_space.n), self.device, self._dist)
+        self.act_dim = int(np.prod(act_space.shape)) if self._continuous else int(act_space.n)
+        if type(self.network) is self._default_network:                  # default network: libdppo kernels end to end
+            self.engine = FusedRecurrentEngine(self.ctx, self.network, cfg, self.obs_dim, self.act_dim, self.device, self._dist,
+                                               self._continuous)
         else:                                                            # custom network_cls: the module runs under autograd
-            self.engine = RecurrentEngine(self.ctx, self.network, cfg, self.device, self._dist)
+            self.engine = RecurrentEngine(self.ctx, self.network, cfg, self.device, self._dist, self._continuous)
         self.optimizer = torch.optim.Adam(self.network.parameters(), lr=cfg.lr, eps=cfg.adam_eps)
         self.engine.bind_optimizer(self.optimizer)
         self.lr_scheduler = torch.optim.lr_scheduler.LinearLR(
@@ -434,20 +493,38 @@ class RecurrentPPO:
         T, N_ = cfg.rollout_steps, cfg.num_envs
         if getattr(self.envs, "device_resident", False) and getattr(self.engine, "fused", False):
             return self._rollout_device()
-        ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev)
+        cont = self._continuous
+        ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev, self.act_dim if cont else None)
         observations, hx, prev_dones = self.current_observations, self.current_hx, self.prev_dones
         ro.hx0.copy_(hx)
         for t in range(T):
             obs_t = torch.as_tensor(np.asarray(observations, dtype=np.float32)[None, ...], device=dev)
             pd_t = torch.as_tensor(np.asarray(prev_dones)[None, ...], dtype=torch.bool, device=dev)
+            log_std = None
             if getattr(self.engine, "fused", False):
                 logits, values, new_hx = self.engine.forward(obs_t, hx, pd_t)
+                log_std = self.engine.log_std
+            elif cont:
+                with torch.inference_mode():
+                    logits, ls, values, new_hx = self.network.get_means_log_stds_values_and_hx(obs_t, hx, pd_t)
+                    ls = ls.reshape(N_, -1)
+                    log_std = ls[0].contiguous() if bool((ls == ls[:1]).all()) else ls   # shared [A] vector, else per row
             else:
                 with torch.inference_mode():
                     logits, values, new_hx = self.network.get_logits_values_and_hx(obs_t, hx, pd_t)
-            # Categorical(logits).sample() + log_prob on the device (counter-based generator, dppo_sample_categorical)
-            actions = torch.empty(N_, dtype=torch.int64, device=dev)
-            self.ctx.sample_categorical(logits.squeeze(0).contiguous(), self.engine.seed, self.engine.draws, self.engine.env_offset, actions, ro.log_probs[t])
+            if cont and log_std.dim() == 1:
+                # JointNormal(mean, exp(log_std)).sample() + log_prob on the device (counter-based generator, dppo_sample_gaussian)
+                actions = torch.empty(N_, self.act_dim, device=dev)
+                self.ctx.sample_gaussian(logits.reshape(N_, -1).contiguous(), log_std, self.engine.seed, self.engine.draws,
+                                         self.engine.env_offset, actions, ro.log_probs[t])
+            elif cont:                                                   # state-dependent std of a custom network
+                dist_t = torch.distributions.Normal(logits.reshape(N_, -1), log_std.exp())
+                actions = dist_t.sample()
+                ro.log_probs[t].copy_(dist_t.log_prob(actions).sum(-1))
+            else:
+                # Categorical(logits).sample() + log_prob on the device (counter-based generator, dppo_sample_categorical)
+                actions = torch.empty(N_, dtype=torch.int64, device=dev)
+                self.ctx.sample_categorical(logits.squeeze(0).contiguous(), self.engine.seed, self.engine.draws, self.engine.env_offset, actions, ro.log_probs[t])
             self.engine.draws += 1
             next_observations, rewards, terminations, truncations, infos = self.envs.step(actions.cpu().numpy())
             final_t = torch.as_tensor(np.asarray(next_observations, dtype=np.float32)[None, ...], device=dev)
@@ -483,11 +560,12 @@ class RecurrentPPO:
         T, N_ = cfg.rollout_steps, cfg.num_envs
         A, Hg = eng.desc.act_dim, eng.desc.gru_hidden
         ro = self._device_ro
+        cont = self._continuous
         if ro is None:
-            ro = self._device_ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev)
+            ro = self._device_ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev, A if cont else None)
             ro.next_obs = torch.empty(T, N_, self.obs_dim, device=dev)
             ro.pd_u8 = torch.zeros(N_, dtype=torch.uint8, device=dev)
-            ro.actions_dev = torch.empty(N_, dtype=torch.int64, device=dev)
+            ro.actions_dev = torch.empty(N_, A, device=dev) if cont else torch.empty(N_, dtype=torch.int64, device=dev)
             ro.pd_f32, ro.pd_bool = torch.empty(N_, device=dev), torch.zeros(N_, dtype=torch.bool, device=dev)
             ro.logits, ro.val1, ro.nv1 = torch.empty(N_, A, device=dev), torch.empty(N_, device=dev), torch.empty(N_, device=dev)
             ro.hx_buf = [torch.zeros(N_, Hg, device=dev) for _ in range(3)]      # [0], [1]: ping-pong state; [2]: discarded output
@@ -504,7 +582,10 @@ class RecurrentPPO:
                 hx, new_hx = ro.hx_buf[t & 1], ro.hx_buf[(t + 1) & 1]
                 ro.prev_dones[t].copy_(ro.pd_u8)
                 ctx.rnn_forward(eng.desc, eng.P, envs.cur_obs, ro.pd_u8, hx, 1, N_, 3, ro.logits, ro.val1, new_hx, ro.ws1)
-                ctx.sample_categorical(ro.logits, eng.seed, counter_of(t), eng.env_offset, ro.actions_dev, ro.log_probs[t])
+                if cont:                                                 # ro.logits holds the action means
+                    ctx.sample_gaussian(ro.logits, eng.log_std, eng.seed, counter_of(t), eng.env_offset, ro.actions_dev, ro.log_probs[t])
+                else:
+                    ctx.sample_categorical(ro.logits, eng.seed, counter_of(t), eng.env_offset, ro.actions_dev, ro.log_probs[t])
                 ro.actions[t].copy_(ro.actions_dev)
                 ro.values[t].copy_(ro.val1)
                 # environment kernel: writes obs[t] (the observation acted on), next_obs[t] (true final observation), rewards, masks;
@@ -556,7 +637,7 @@ class RecurrentPPO:
 
     # ---- learn (recurrent_ppo.py:301-367) ---------------------------------------------------------------
     def learn(self, experience) -> None:
-        ro = experience if isinstance(experience, RecurrentRollout) else RecurrentRollout.from_lists(experience, self.device)
+        ro = experience if isinstance(experience, RecurrentRollout) else RecurrentRollout.from_lists(experience, self.device, self._continuous)
         self.engine.learn(ro)
         self.optimizer._opt_called = True
         self.lr_scheduler.step()
@@ -592,3 +673,14 @@ class RecurrentPPO:
             self.checkpointer.save(env_steps, self.network, self.optimizer)
         self._flush_episode_stats()
         self.envs.close()
+
+
+class RecurrentContinuousPPO(RecurrentPPO):
+    """Recurrent (GRU) Gaussian-policy PPO for Box action spaces: RecurrentPPO with the actor of ContinuousPPO
+    (continuous_ppo.py:50-121: mean head, state-independent log-std, actions neither squashed nor clipped)."""
+    _continuous = True
+    _default_network = RecurrentContinuousActorCriticNetwork
+
+    def __init__(self, env_fn: Callable[[], Any], cfg: RecurrentContinuousPPOConfig = RecurrentContinuousPPOConfig(),
+                 network_cls: Any = RecurrentContinuousActorCriticNetwork, *, process_group=None, dp: bool = False) -> None:
+        super().__init__(env_fn, cfg, network_cls, process_group=process_group, dp=dp)

@@ -299,28 +299,35 @@ int64_t dppo_ppo_loss_workspace_bytes(int64_t M, int A);
 
 /* ---- recurrent actor-critic (RecurrentPPO, diamond/recurrent_ppo.py) --------------------------------- */
 /* Default RecurrentActorCriticNetwork (recurrent_ppo.py:94-125): base Linear(D,H)+Tanh -> GRU(H,Hg) -> actor head
- * Linear(Hg,H)+Tanh+Linear(H,A) and critic head Linear(Hg,H)+Tanh+Linear(H,1). */
+ * Linear(Hg,H)+Tanh+Linear(H,A) and critic head Linear(Hg,H)+Tanh+Linear(H,1).
+ * continuous = 1: RecurrentContinuousActorCriticNetwork (RecurrentContinuousPPO), the same trunk with a Gaussian policy -- the actor
+ * head (actor_mean_head) outputs the action means and a state-independent log-std vector actor_log_std [A] is a parameter. */
 typedef struct dppo_rnn_desc {
     int32_t obs_dim;      /* D */
-    int32_t hidden;       /* H  = cfg.network_hidden_dim */
+    int32_t hidden;       /* H  = cfg.network_hidden_dim (<= 512) */
     int32_t gru_hidden;   /* Hg = cfg.gru_hidden_dim (<= 512; 129-512 run on thread-block-cluster scans) */
-    int32_t act_dim;      /* A  = Discrete.n */
+    int32_t act_dim;      /* A  = Discrete.n, or the action dimensions of a Box (<= DPPO_MAX_ACT) */
+    int32_t continuous;   /* 0: categorical policy (logits), 1: Gaussian policy (means + actor_log_std) */
 } dppo_rnn_desc;
 /* Offsets (floats, multiples of 4) in the flat parameter / gradient / Adam buffers; the GRU tensors are nn.GRU's
- * weight_ih_l0 [3Hg,H], weight_hh_l0 [3Hg,Hg], bias_ih_l0, bias_hh_l0 (gate order r,z,n); w3/b3 = actor_head.0 | critic_head.0. */
+ * weight_ih_l0 [3Hg,H], weight_hh_l0 [3Hg,Hg], bias_ih_l0, bias_hh_l0 (gate order r,z,n); w3/b3 = actor_head.0 | critic_head.0
+ * (continuous: actor_mean_head.0 | critic_head.0), wa/ba = actor_head.2 (continuous: actor_mean_head.2).  log_std = actor_log_std [A],
+ * placed after bc when continuous, else -1; every other offset is the same for both kinds. */
 typedef struct dppo_rnn_layout {
     int64_t w1, b1;
     int64_t wih, whh, bih, bhh;
     int64_t w3, b3;
     int64_t wa, ba;
     int64_t wc, bc;
+    int64_t log_std;
     int64_t total;
 } dppo_rnn_layout;
 int dppo_rnn_layout_compute(const dppo_rnn_desc* desc, dppo_rnn_layout* out);
 int64_t dppo_rnn_workspace_bytes(const dppo_rnn_desc* desc, int T, int N, int64_t M, int training);
 /* get_logits_values_and_hx / get_values (recurrent_ppo.py:127-149) over a [T,N] sequence: obs [T,N,D]; prev_dones uint8 [T,N]
  * (NULL: no resets) zeroes the hidden state of an environment BEFORE step t (recurrent_ppo.py:84); hx0 [N,Hg] (NULL: zeros).
- * heads bit0: logits [T*N,A]; bit1: values [T*N]; hx_out (optional) [N,Hg] final hidden state. */
+ * heads bit0: logits [T*N,A] (continuous: the action means [T*N,A]; the log-std is params + layout.log_std); bit1: values [T*N];
+ * hx_out (optional) [N,Hg] final hidden state. */
 int dppo_rnn_forward(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* params, const float* obs,
                      const unsigned char* prev_dones, const float* hx0, int T, int N, int heads, float* logits,
                      float* values, float* hx_out, void* ws, int64_t ws_bytes, void* stream);
@@ -328,10 +335,14 @@ int dppo_rnn_forward(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* para
  * idx[0..M) of the flattened [T*N] outputs enter the PPO loss (idx NULL: all rows in order, M = T*N), back-propagation
  * through all T steps.  The entries of idx must be distinct and in [0, T*N): d(loss)/d(h_t) is scattered back to row idx[i],
  * so there are no padding rows (unlike dppo_mlp_grad_minibatch) and a repeated row would lose a contribution.
- * actions int32 [T*N]; old_log_probs / adv / returns f32 [T*N]; flat gradient -> grads, (policy, value, entropy, total) ->
- * losses[0..3]. */
+ * actions: int32 [T*N] (discrete) or f32 [T*N, A] (continuous: the Gaussian loss of continuous_ppo.py, with the gradient of
+ * actor_log_std at layout.log_std); old_log_probs / adv / returns f32 [T*N]; flat gradient -> grads, (policy, value, entropy,
+ * total) -> losses[0..3].
+ * Both calls refuse, before launching anything, hidden > 512, gru_hidden > 512, act_dim > DPPO_MAX_ACT; dppo_rnn_grad_minibatch
+ * also refuses the (hidden, act_dim) pairs whose per-warp head-gradient accumulators exceed the head kernel's 200 KB of shared
+ * memory (9 (act_dim + 1) hidden floats: e.g. act_dim <= 10 at hidden 512, <= 32 up to hidden 172). */
 int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* params, float* grads, const float* obs,
-                            const unsigned char* prev_dones, const float* hx0, int T, int N, const int32_t* actions,
+                            const unsigned char* prev_dones, const float* hx0, int T, int N, const void* actions,
                             const float* old_log_probs, const float* adv, const float* returns, const double* adv_stats,
                             const int32_t* idx, int64_t M, const dppo_hyper* hyper, float* losses, void* ws,
                             int64_t ws_bytes, void* stream);
