@@ -53,6 +53,14 @@ struct EnvArgs {
     unsigned long long seed;
     long long env_offset;
     float p_term, p_trunc;      // synthetic env
+    // per-environment normalisation (NORM instantiations only; dppo.h dppo_env_desc / dppo_env_state)
+    int norm_obs, norm_rew;
+    double gamma, eps, clip_obs, clip_rew;
+    double *obs_mean, *obs_var;  // [N, D]
+    double* obs_count;          // [N]
+    double* ret_stats;          // [N, 4]: discounted return accumulator, its running mean, variance, count
+    const int32_t* update;      // [1] nonzero: update the statistics (read at run time, so replayed graphs follow it)
+    float* raw_rew_t;           // row t of the raw reward buffer (may be null)
 };
 
 template <int KIND>
@@ -77,6 +85,8 @@ __device__ __forceinline__ void reset_state(const EnvArgs& a, int e, double* s)
     a.steps[e] = 0;
 }
 
+template <int KIND> constexpr int kObsDim = KIND == 0 ? 4 : KIND == 1 ? 3 : KIND == 4 ? 6 : 2;
+
 template <int KIND>
 __device__ __forceinline__ void write_obs(const double* s, float* o)
 {
@@ -85,6 +95,67 @@ __device__ __forceinline__ void write_obs(const double* s, float* o)
     else if constexpr (KIND == 4) {
         o[0] = (float)cos(s[0]); o[1] = (float)sin(s[0]); o[2] = (float)cos(s[1]); o[3] = (float)sin(s[1]); o[4] = (float)s[2]; o[5] = (float)s[3];
     } else { o[0] = (float)s[0]; o[1] = (float)s[1]; }
+}
+
+// Gymnasium's RunningMeanStd.update on a batch of one value x (batch mean x, batch variance 0, batch count 1), in NumPy's operation
+// order with every rounding explicit (no contraction):  delta = x - mean;  tot = count + 1;  mean += delta * 1 / tot;
+// M2 = var * count + 0 + delta^2 * count * 1 / tot;  var = M2 / tot;  count = tot.  The caller stores count = tot.
+__device__ __forceinline__ void rms_update(double& mean, double& var, double count, double x)
+{
+    const double delta = __dsub_rn(x, mean), tot = __dadd_rn(count, 1.0);
+    mean = __dadd_rn(mean, __ddiv_rn(delta, tot));
+    var = __ddiv_rn(__dadd_rn(__dmul_rn(var, count), __ddiv_rn(__dmul_rn(__dmul_rn(delta, delta), count), tot)), tot);
+}
+
+// NormalizeObservation of one feature: update (unless frozen), then float32((x - mean) / sqrt(var + eps)), clipped in float32
+__device__ __forceinline__ float norm_feature(const EnvArgs& a, int64_t i, double count, bool upd, float xf)
+{
+    double mean = a.obs_mean[i], var = a.obs_var[i];
+    if (upd) {
+        rms_update(mean, var, count, (double)xf);
+        a.obs_mean[i] = mean; a.obs_var[i] = var;
+    }
+    float y = (float)__ddiv_rn(__dsub_rn((double)xf, mean), __dsqrt_rn(__dadd_rn(var, a.eps)));
+    if (a.clip_obs > 0.0) {
+        const float c = (float)a.clip_obs;
+        y = fminf(fmaxf(y, -c), c);
+    }
+    return y;
+}
+
+// One classic environment's observation of D features through NormalizeObservation (or copied when only rewards are normalised)
+template <int D>
+__device__ __forceinline__ void norm_obs(const EnvArgs& a, int e, const float* x, float* dst)
+{
+    if (!a.norm_obs) {
+#pragma unroll
+        for (int j = 0; j < D; ++j) dst[j] = x[j];
+        return;
+    }
+    const bool upd = *a.update != 0;
+    const double count = a.obs_count[e];
+#pragma unroll
+    for (int j = 0; j < D; ++j) dst[j] = norm_feature(a, (int64_t)e * D + j, count, upd, x[j]);
+    if (upd) a.obs_count[e] = __dadd_rn(count, 1.0);
+}
+
+// NormalizeReward: acc = acc * gamma * (1 - terminated) + r; update the return statistics with acc (unless frozen);
+// emit r / sqrt(var + eps), clipped in double.  The accumulator is cut by termination only, as in Gymnasium.
+__device__ __forceinline__ float norm_reward(const EnvArgs& a, int e, double r, bool term)
+{
+    if (!a.norm_rew) return (float)r;
+    double* st = a.ret_stats + (int64_t)e * 4;
+    const double acc = __dadd_rn(__dmul_rn(__dmul_rn(st[0], a.gamma), term ? 0.0 : 1.0), r);
+    double mean = st[1], var = st[2];
+    st[0] = acc;
+    if (*a.update != 0) {
+        const double count = st[3];
+        rms_update(mean, var, count, acc);
+        st[1] = mean; st[2] = var; st[3] = __dadd_rn(count, 1.0);
+    }
+    double y = __ddiv_rn(r, __dsqrt_rn(__dadd_rn(var, a.eps)));
+    if (a.clip_rew > 0.0) y = fmin(fmax(y, -a.clip_rew), a.clip_rew);
+    return (float)y;
 }
 
 // Acrobot-v1 `_dsdt` ("book" dynamics; m1 = m2 = l1 = 1, lc1 = lc2 = 0.5, I1 = I2 = 1, g = 9.8) in Gymnasium's operation order
@@ -102,8 +173,10 @@ __device__ __forceinline__ void acrobot_dsdt(const double* y, double torque, dou
     dy[0] = dth1; dy[1] = dth2; dy[2] = -(d2 * ddth2 + phi1) / d1; dy[3] = ddth2;
 }
 
-// mode 0: step (t, actions); mode 1: reset the environments with mask[e] != 0 (mask null: all)
-template <int KIND>
+// mode 0: step (t, actions); mode 1: reset the environments with mask[e] != 0 (mask null: all).  NORM: the environment's
+// observations and rewards pass through its NormalizeObservation / NormalizeReward statistics (a.norm_obs, a.norm_rew) in this thread;
+// the NORM = false instantiations are the kernels without normalisation, unchanged.
+template <int KIND, bool NORM>
 __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __restrict__ mask)
 {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
@@ -117,11 +190,23 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
             a.ep_return[e] = 0.0;
 #pragma unroll
             for (int i = 0; i < 4; ++i) a.state[(int64_t)e * 4 + i] = s[i];
-            write_obs<KIND>(s, a.cur_obs + (int64_t)e * a.D);
+            if constexpr (NORM) {
+                float o[6];
+                write_obs<KIND>(s, o);
+                norm_obs<kObsDim<KIND>>(a, e, o, a.cur_obs + (int64_t)e * a.D);
+            } else {
+                write_obs<KIND>(s, a.cur_obs + (int64_t)e * a.D);
+            }
         }
         return;
     }
-    if (a.obs_t) write_obs<KIND>(s, a.obs_t + (int64_t)e * a.D);
+    if constexpr (NORM) {                                               // the (normalised) observation the action was sampled from
+        if (a.obs_t)
+#pragma unroll
+            for (int j = 0; j < kObsDim<KIND>; ++j) a.obs_t[(int64_t)e * a.D + j] = a.cur_obs[(int64_t)e * a.D + j];
+    } else {
+        if (a.obs_t) write_obs<KIND>(s, a.obs_t + (int64_t)e * a.D);
+    }
     double reward;
     bool term = false;
     int limit;                                                          // TimeLimit of the registered id
@@ -215,8 +300,19 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
     }
     a.steps[e] += 1;
     const bool trunc = a.steps[e] >= limit && !term;
-    write_obs<KIND>(s, a.next_obs_t + (int64_t)e * a.D);               // the true final observation (autoreset disabled)
-    a.rew_t[e] = (float)reward;
+    float fin[6];                                                       // NORM: the normalised final observation
+    if constexpr (NORM) {
+        float o[6];
+        write_obs<KIND>(s, o);
+        norm_obs<kObsDim<KIND>>(a, e, o, fin);
+#pragma unroll
+        for (int j = 0; j < kObsDim<KIND>; ++j) a.next_obs_t[(int64_t)e * a.D + j] = fin[j];
+        a.rew_t[e] = norm_reward(a, e, reward, term);
+        if (a.raw_rew_t) a.raw_rew_t[e] = (float)reward;
+    } else {
+        write_obs<KIND>(s, a.next_obs_t + (int64_t)e * a.D);           // the true final observation (autoreset disabled)
+        a.rew_t[e] = (float)reward;
+    }
     a.term_t[e] = term ? 1.0f : 0.0f;
     a.trunc_t[e] = trunc ? 1.0f : 0.0f;
     const double ret = a.ep_return[e] + reward;
@@ -230,18 +326,36 @@ __global__ void classic_env_kernel(EnvArgs a, int mode, const unsigned char* __r
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) a.state[(int64_t)e * 4 + i] = s[i];
-    write_obs<KIND>(s, a.cur_obs + (int64_t)e * a.D);
+    if constexpr (NORM) {
+        if (done && a.auto_reset) {                                     // the post-reset observation is counted too
+            float o[6];
+            write_obs<KIND>(s, o);
+            norm_obs<kObsDim<KIND>>(a, e, o, fin);
+        }                                                               // else cur_obs is next_obs[t], bit for bit
+#pragma unroll
+        for (int j = 0; j < kObsDim<KIND>; ++j) a.cur_obs[(int64_t)e * a.D + j] = fin[j];
+    } else {
+        write_obs<KIND>(s, a.cur_obs + (int64_t)e * a.D);
+    }
 }
 
 // Synthetic environment of the scale benchmark (shape-only stand-in, diamond/envs.py BatchedSyntheticVectorEnv): i.i.d.
 // standard-normal observations, reward = 0.1 * obs[0] * sign(action), Bernoulli terminations / truncations.
-// One warp per environment; lanes stride over the observation.
+// One warp per environment; lanes stride over the observation.  NORM: each lane runs its features' NormalizeObservation
+// statistics (the count is shared: every lane reads it, lane 0 advances it once the warp is done), lane 0 runs NormalizeReward, and
+// the raw observation's first feature, which the reward reads, is kept in state[e, 0] (unused by the synthetic kinds otherwise).
+template <bool NORM>
 __global__ void synthetic_env_kernel(EnvArgs a, int mode, const unsigned char* __restrict__ mask)
 {
     const int e = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5), lane = threadIdx.x & 31;
     if (e >= a.N) return;
     const unsigned long long env = (unsigned long long)(a.env_offset + e);
+    bool upd = false;
+    if constexpr (NORM) upd = a.norm_obs && *a.update != 0;
+    float raw0 = 0.f;                                                   // NORM: lane 0's raw first feature of the last draw
     auto fresh = [&](unsigned long long draw, float* dst0, float* dst1) {       // D normals into up to two destinations
+        double count = 0.0;
+        if constexpr (NORM) if (a.norm_obs) count = a.obs_count[e];
         for (int j0 = 2 * lane; j0 < a.D; j0 += 64) {
             const unsigned long long c = draw * 4096ull + (unsigned long long)(j0 / 2);
             const uint4 r = philox4x32_10(make_uint4((uint32_t)env, (uint32_t)(env >> 32), (uint32_t)c, (uint32_t)(c >> 32) ^ 0x4F425321u),
@@ -249,9 +363,21 @@ __global__ void synthetic_env_kernel(EnvArgs a, int mode, const unsigned char* _
             const float rad = sqrtf(-2.0f * logf((float)u01d(r.x)));
             float sn, cs;
             sincosf(6.28318530717958647692f * (float)u01d(r.y), &sn, &cs);
-            const float v0 = rad * cs, v1 = rad * sn;
+            float v0 = rad * cs, v1 = rad * sn;
+            if constexpr (NORM) {
+                if (j0 == 0) raw0 = v0;
+                if (a.norm_obs) {
+                    v0 = norm_feature(a, (int64_t)e * a.D + j0, count, upd, v0);
+                    if (j0 + 1 < a.D) v1 = norm_feature(a, (int64_t)e * a.D + j0 + 1, count, upd, v1);
+                }
+            }
             if (dst0) { dst0[j0] = v0; if (j0 + 1 < a.D) dst0[j0 + 1] = v1; }
             if (dst1) { dst1[j0] = v0; if (j0 + 1 < a.D) dst1[j0 + 1] = v1; }
+        }
+        if constexpr (NORM) {
+            __syncwarp();
+            if (upd && lane == 0) a.obs_count[e] = __dadd_rn(count, 1.0);
+            __syncwarp();
         }
     };
     float* cur = a.cur_obs + (int64_t)e * a.D;
@@ -261,10 +387,11 @@ __global__ void synthetic_env_kernel(EnvArgs a, int mode, const unsigned char* _
             fresh((draw << 20), cur, nullptr);
             __syncwarp();
             if (lane == 0) { a.episode[e] += 1; a.steps[e] = 0; a.ep_return[e] = 0.0; }
+            if (NORM && lane == 0) a.state[(int64_t)e * 4] = raw0;
         }
         return;
     }
-    const float o0 = cur[0];
+    const float o0 = NORM ? (float)a.state[(int64_t)e * 4] : cur[0];
     __syncwarp();
     if (a.obs_t) for (int j = lane; j < a.D; j += 32) a.obs_t[(int64_t)e * a.D + j] = cur[j];
     float asum;
@@ -293,7 +420,13 @@ __global__ void synthetic_env_kernel(EnvArgs a, int mode, const unsigned char* _
     if (done && a.auto_reset) fresh(((2ull * (unsigned long long)(a.episode[e] + 1) + 1ull) << 20) + 7ull, cur, nullptr);
     __syncwarp();
     if (lane == 0) {
-        a.rew_t[e] = reward;
+        if constexpr (NORM) {
+            a.rew_t[e] = norm_reward(a, e, (double)reward, term);
+            if (a.raw_rew_t) a.raw_rew_t[e] = reward;
+            a.state[(int64_t)e * 4] = raw0;                             // of the observation now in cur_obs
+        } else {
+            a.rew_t[e] = reward;
+        }
         a.term_t[e] = term ? 1.0f : 0.0f;
         a.trunc_t[e] = trunc ? 1.0f : 0.0f;
         const double ret = a.ep_return[e] + (double)reward;
@@ -303,22 +436,28 @@ __global__ void synthetic_env_kernel(EnvArgs a, int mode, const unsigned char* _
     }
 }
 
-int launch_env(dppo_ctx* ctx, const EnvArgs& a, int mode, const unsigned char* mask, cudaStream_t st)
+template <bool NORM>
+int launch_env_t(dppo_ctx* ctx, const EnvArgs& a, int mode, const unsigned char* mask, cudaStream_t st)
 {
     const unsigned grid = (a.N + 127) / 128;
     switch (a.kind) {
-    case 0: classic_env_kernel<0><<<grid, 128, 0, st>>>(a, mode, mask); break;
-    case 1: classic_env_kernel<1><<<grid, 128, 0, st>>>(a, mode, mask); break;
-    case 4: classic_env_kernel<4><<<grid, 128, 0, st>>>(a, mode, mask); break;
-    case 5: classic_env_kernel<5><<<grid, 128, 0, st>>>(a, mode, mask); break;
-    case 6: classic_env_kernel<6><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 0: classic_env_kernel<0, NORM><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 1: classic_env_kernel<1, NORM><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 4: classic_env_kernel<4, NORM><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 5: classic_env_kernel<5, NORM><<<grid, 128, 0, st>>>(a, mode, mask); break;
+    case 6: classic_env_kernel<6, NORM><<<grid, 128, 0, st>>>(a, mode, mask); break;
     default:
-        synthetic_env_kernel<<<(unsigned)(((int64_t)a.N * 32 + 255) / 256), 256, 0, st>>>(a, mode, mask);
+        synthetic_env_kernel<NORM><<<(unsigned)(((int64_t)a.N * 32 + 255) / 256), 256, 0, st>>>(a, mode, mask);
         DPPO_CHECK_LAUNCH(ctx, "synthetic_env_kernel");
         return 0;
     }
     DPPO_CHECK_LAUNCH(ctx, "classic_env_kernel");
     return 0;
+}
+
+int launch_env(dppo_ctx* ctx, const EnvArgs& a, int mode, const unsigned char* mask, cudaStream_t st)
+{
+    return (a.norm_obs || a.norm_rew) ? launch_env_t<true>(ctx, a, mode, mask, st) : launch_env_t<false>(ctx, a, mode, mask, st);
 }
 
 int fill_args(dppo_ctx* ctx, const dppo_env_desc* d, const dppo_env_state* s, EnvArgs& a)
@@ -335,6 +474,20 @@ int fill_args(dppo_ctx* ctx, const dppo_env_desc* d, const dppo_env_state* s, En
     a.kind = d->kind; a.N = d->num_envs; a.D = d->obs_dim; a.A = d->act_dim;
     a.state = s->state; a.steps = s->steps; a.episode = s->episode; a.ep_return = s->ep_return; a.cur_obs = s->cur_obs;
     a.seed = d->seed; a.env_offset = d->env_offset; a.p_term = d->p_term; a.p_trunc = d->p_trunc;
+    if (d->normalize & ~(DPPO_ENV_NORMALIZE_OBS | DPPO_ENV_NORMALIZE_REWARD)) DPPO_FAIL(ctx, "env: unknown normalize flags 0x%x", d->normalize);
+    a.norm_obs = (d->normalize & DPPO_ENV_NORMALIZE_OBS) != 0;
+    a.norm_rew = (d->normalize & DPPO_ENV_NORMALIZE_REWARD) != 0;
+    if (a.norm_obs || a.norm_rew) {
+        if (!s->update) DPPO_FAIL(ctx, "env: normalisation needs the device update flag");
+        if (a.norm_obs && (!s->obs_mean || !s->obs_var || !s->obs_count)) DPPO_FAIL(ctx, "env: observation normalisation needs obs_mean / obs_var / obs_count");
+        if (a.norm_rew && !s->ret_stats) DPPO_FAIL(ctx, "env: reward normalisation needs ret_stats");
+        if (a.norm_rew && !(d->gamma >= 0.0 && d->gamma <= 1.0)) DPPO_FAIL(ctx, "env: gamma %g outside [0, 1]", d->gamma);
+        if (!(d->epsilon > 0.0)) DPPO_FAIL(ctx, "env: epsilon %g must be > 0", d->epsilon);
+        if (!(d->clip_observation >= 0.0) || !(d->clip_reward >= 0.0))
+            DPPO_FAIL(ctx, "env: clips must be >= 0 (0: no clip); got %g / %g", d->clip_observation, d->clip_reward);
+        a.gamma = d->gamma; a.eps = d->epsilon; a.clip_obs = d->clip_observation; a.clip_rew = d->clip_reward;
+        a.obs_mean = s->obs_mean; a.obs_var = s->obs_var; a.obs_count = s->obs_count; a.ret_stats = s->ret_stats; a.update = s->update;
+    }
     return 0;
 }
 
@@ -351,7 +504,7 @@ extern "C" int dppo_env_reset(dppo_ctx* ctx, const dppo_env_desc* desc, const dp
 
 extern "C" int dppo_env_step(dppo_ctx* ctx, const dppo_env_desc* desc, const dppo_env_state* state, const void* actions, int t,
                              int auto_reset, float* obs, float* next_obs, void* buf_actions, float* rewards, float* terminations,
-                             float* truncations, float* done_return, void* stream)
+                             float* truncations, float* done_return, float* raw_rewards, void* stream)
 {
     if (!ctx) return 1;
     EnvArgs a = {};
@@ -365,5 +518,10 @@ extern "C" int dppo_env_step(dppo_ctx* ctx, const dppo_env_desc* desc, const dpp
     a.act_t = buf_actions ? (cont ? (void*)((float*)buf_actions + (int64_t)t * N * a.A) : (void*)((int32_t*)buf_actions + (int64_t)t * N)) : nullptr;
     a.rew_t = rewards + (int64_t)t * N; a.term_t = terminations + (int64_t)t * N; a.trunc_t = truncations + (int64_t)t * N;
     a.done_return = done_return;
-    return launch_env(ctx, a, 0, nullptr, (cudaStream_t)stream);
+    a.raw_rew_t = raw_rewards ? raw_rewards + (int64_t)t * N : nullptr;
+    if (launch_env(ctx, a, 0, nullptr, (cudaStream_t)stream)) return 1;
+    if (a.raw_rew_t && !a.norm_obs && !a.norm_rew &&                    // the kernel without normalisation writes no raw row
+        cudaMemcpyAsync(a.raw_rew_t, a.rew_t, (size_t)N * sizeof(float), cudaMemcpyDeviceToDevice, (cudaStream_t)stream) != cudaSuccess)
+        DPPO_FAIL(ctx, "env_step: raw reward copy failed");
+    return 0;
 }

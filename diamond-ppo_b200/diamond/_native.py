@@ -38,11 +38,18 @@ class RnnLayout(C.Structure):
 
 class EnvDesc(C.Structure):
     _fields_ = [("kind", C.c_int32), ("num_envs", C.c_int32), ("obs_dim", C.c_int32), ("act_dim", C.c_int32), ("seed", C.c_uint64),
-                ("env_offset", C.c_int64), ("p_term", C.c_float), ("p_trunc", C.c_float)]
+                ("env_offset", C.c_int64), ("p_term", C.c_float), ("p_trunc", C.c_float),
+                ("normalize", C.c_int32), ("pad0", C.c_int32), ("gamma", C.c_double), ("epsilon", C.c_double),
+                ("clip_observation", C.c_double), ("clip_reward", C.c_double)]
+
+
+ENV_NORMALIZE_OBS, ENV_NORMALIZE_REWARD = 1, 2     # dppo_env_desc.normalize bits
 
 
 class EnvState(C.Structure):
-    _fields_ = [("state", C.c_void_p), ("steps", C.c_void_p), ("episode", C.c_void_p), ("ep_return", C.c_void_p), ("cur_obs", C.c_void_p)]
+    _fields_ = [("state", C.c_void_p), ("steps", C.c_void_p), ("episode", C.c_void_p), ("ep_return", C.c_void_p), ("cur_obs", C.c_void_p),
+                ("obs_mean", C.c_void_p), ("obs_var", C.c_void_p), ("obs_count", C.c_void_p), ("ret_stats", C.c_void_p),
+                ("update", C.c_void_p)]
 
 
 class Hyper(C.Structure):
@@ -357,10 +364,10 @@ class Context:
         self._check(self.lib.dppo_env_reset(self.h, C.byref(desc), C.byref(state), _ptr(mask), _stream()), "dppo_env_reset")
 
     def env_step(self, desc, state, actions, t, auto_reset, obs, next_obs, buf_actions, rewards, terminations, truncations,
-                 done_return=None):
+                 done_return=None, raw_rewards=None):
         self._check(self.lib.dppo_env_step(self.h, C.byref(desc), C.byref(state), _ptr(actions), C.c_int(t), C.c_int(int(auto_reset)),
                                            _ptr(obs), _ptr(next_obs), _ptr(buf_actions), _ptr(rewards), _ptr(terminations),
-                                           _ptr(truncations), _ptr(done_return), _stream()), "dppo_env_step")
+                                           _ptr(truncations), _ptr(done_return), _ptr(raw_rewards), _stream()), "dppo_env_step")
 
     def episode_stats(self, rewards, terminations, truncations, ep_return, ep_len, window, out_returns, out_lengths, out_n, finished, ws):
         """Device-side Ticker bookkeeping of one rollout (dppo_episode_stats)."""

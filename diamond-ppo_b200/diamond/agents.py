@@ -1082,6 +1082,8 @@ class _PPOBase:
             if getattr(buf, "values", None) is None:
                 buf.values = torch.empty(buf.T, buf.N, dtype=torch.float32, device=self.device)
                 buf.logp = torch.empty(buf.T, buf.N, dtype=torch.float32, device=self.device)
+                if getattr(envs, "normalize_reward", False):            # rewards are normalised: keep the raw ones for the Ticker
+                    buf.raw_rewards = torch.empty(buf.T, buf.N, dtype=torch.float32, device=self.device)
             buf.policy_stamp = None
             stamp = self.engine.policy_stamp()
             # From the third rollout into the same buffers the T x (forward, head, sampling, environment) launches are replayed
@@ -1124,6 +1126,7 @@ class _PPOBase:
         for step_idx in range(cfg.rollout_steps):
             actions = self.network.get_actions(observations, device=self.device)
             next_observations, rewards, terminations, truncations, infos = self.envs.step(actions)
+            tick_rewards = infos.get("raw_rewards", rewards) if isinstance(infos, dict) else rewards   # raw, if the env normalises
             buf.store(step_idx, observations, next_observations, actions, rewards, terminations, truncations)
             dones = np.logical_or(terminations, truncations)
             if np.any(dones):                                          # autoreset disabled: masked reset (ppo.py:174-179)
@@ -1131,7 +1134,7 @@ class _PPOBase:
             else:
                 observations = next_observations
             if self.ticker is not None:
-                self.ticker.tick(rewards, dones)
+                self.ticker.tick(tick_rewards, dones)
         self.current_observations = observations
         return buf
 
@@ -1157,7 +1160,8 @@ class _PPOBase:
                 st["ep_return"].copy_(pend["ep_return"]); st["ep_len"].copy_(pend["ep_len"])
             self._pending_epstats = None
         self._flush_episode_stats()                                    # the previous rollout's numbers (long since copied)
-        self.ctx.episode_stats(buf.rewards, buf.terminations, buf.truncations, st["ep_return"], st["ep_len"], W, st["out"][:W],
+        rewards = getattr(buf, "raw_rewards", None)                    # a reward-normalising environment's raw rewards
+        self.ctx.episode_stats(buf.rewards if rewards is None else rewards, buf.terminations, buf.truncations, st["ep_return"], st["ep_len"], W, st["out"][:W],
                                st["out_len"], st["out_n"], st["finished"], st["ws"])
         st["out"][W:W + 1].copy_(st["finished"])
         st["out"][W + 1:W + 2].copy_(st["out_n"])
@@ -1219,7 +1223,8 @@ class _PPOBase:
             st["epstats"] = dict(ep_return=self._epstats["ep_return"].cpu(), ep_len=self._epstats["ep_len"].cpu())
         if getattr(envs, "device_resident", False):
             st["envs"] = dict(kind="device", seed=int(envs.desc.seed), env_offset=int(envs.desc.env_offset),
-                              **{k: getattr(envs, k).cpu() for k in ("state", "steps", "episode", "ep_return", "cur_obs")})
+                              update_running_mean=envs.update_running_mean,           # + normalisation statistics, if any
+                              **{k: getattr(envs, k).cpu() for k in envs.state_tensors})
         else:
             import pickle
             try:                                                       # host environments: whatever pickles (the in-repo shim does)
@@ -1251,8 +1256,10 @@ class _PPOBase:
         if es["kind"] == "device":
             envs = self.envs
             envs.desc.seed, envs.desc.env_offset = es["seed"], es["env_offset"]
-            for k in ("state", "steps", "episode", "ep_return", "cur_obs"):
+            for k in envs.state_tensors:
                 getattr(envs, k).copy_(es[k])
+            if "update_running_mean" in es:
+                envs.update_running_mean = es["update_running_mean"]
             self.current_observations = envs.cur_obs
         elif es["kind"] == "pickle":
             import pickle

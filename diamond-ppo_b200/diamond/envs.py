@@ -379,14 +379,29 @@ class DeviceVectorEnv:
     arrays; the default-network agents use `step_into`, which writes the step straight into the device rollout buffer and
     resets finished environments inside the same kernel (diamond/ppo.py:160-182 without a PCIe crossing).
 
-    Use as `env_fn = DeviceVectorEnv.factory("CartPole-v1")` (an `env_fn.vectorized` factory taking num_envs)."""
+    Use as `env_fn = DeviceVectorEnv.factory("CartPole-v1")` (an `env_fn.vectorized` factory taking num_envs).
+
+    Normalisation (`normalize_observation`, `normalize_reward`): every environment keeps its own float64 statistics, exactly as one
+    Gymnasium `NormalizeObservation(epsilon)` / `NormalizeReward(gamma, epsilon)` wrapper per sub-environment of a `SyncVectorEnv`
+    would (optionally followed by a clip to +-`clip_observation` / +-`clip_reward`), inside the environment kernel: no host round
+    trip and no extra launch per step.  Every emitted observation updates the statistics before it is normalised -- each step's
+    final observation and each post-reset observation (in-kernel reset, `reset(options={"reset_mask": m})`, `reset(seed=...)`);
+    the constructor's reset only brings the state up (it counts nothing and normalises with the initial statistics), as
+    constructing a Gymnasium wrapper does not reset its environment.  The reward accumulator is cut by termination only, never by
+    truncation or reset (Gymnasium's NormalizeReward).  `rewards` are the normalised rewards (what GAE consumes); `step()` returns
+    the raw ones as `info["raw_rewards"]`, and agents pass a raw-reward row to `step_into` so episode returns stay raw.
+    `update_running_mean = False` freezes both sets of statistics (it is read by the kernel from device memory, so replayed
+    rollout graphs follow it).  The statistics are the tensors `obs_mean` [N, D], `obs_var` [N, D], `obs_count` [N] and
+    `return_stats` [N, 4] (accumulator, mean, variance, count); include/dppo.h states the arithmetic."""
 
     device_resident = True
     _KINDS = {"CartPole-v1": (0, 4, 2, False), "Pendulum-v1": (1, 3, 1, True), "Acrobot-v1": (4, 6, 3, False),
               "MountainCar-v0": (5, 2, 3, False), "MountainCarContinuous-v0": (6, 2, 1, True)}
 
     def __init__(self, env_id: str, num_envs: int, seed: int = 0, device=None, obs_dim: int = 64, n_actions: int = 4,
-                 continuous: bool = False, p_term: float = 0.01, p_trunc: float = 0.01, env_offset: int = 0):
+                 continuous: bool = False, p_term: float = 0.01, p_trunc: float = 0.01, env_offset: int = 0,
+                 normalize_observation: bool = False, normalize_reward: bool = False, gamma: float = 0.99, epsilon: float = 1e-8,
+                 clip_observation: float | None = None, clip_reward: float | None = None):
         import torch
         from . import _native as N
         self._torch, self._N = torch, N
@@ -418,18 +433,66 @@ class DeviceVectorEnv:
         self.obs_dim, self.act_dim = D, A
         self._check_actions = kind in (4, 5)       # a host array may hold anything; the sampler's output is in range
         self.desc = N.EnvDesc(kind, self.num_envs, D, A, int(seed) & (2 ** 64 - 1), int(env_offset), float(p_term), float(p_trunc))
+        for name, clip in (("clip_observation", clip_observation), ("clip_reward", clip_reward)):
+            if clip is not None and not clip > 0:
+                raise ValueError(f"{name} must be > 0 or None (got {clip})")
+        self.normalize_observation, self.normalize_reward = bool(normalize_observation), bool(normalize_reward)
+        if self.normalize_observation or self.normalize_reward:
+            if not 0.0 <= gamma <= 1.0 or not epsilon > 0:
+                raise ValueError(f"normalisation needs 0 <= gamma <= 1 and epsilon > 0 (got {gamma}, {epsilon})")
+            self.desc.normalize = (N.ENV_NORMALIZE_OBS if self.normalize_observation else 0) | \
+                (N.ENV_NORMALIZE_REWARD if self.normalize_reward else 0)
+            self.desc.gamma, self.desc.epsilon = float(gamma), float(epsilon)
+            self.desc.clip_observation, self.desc.clip_reward = float(clip_observation or 0.0), float(clip_reward or 0.0)
+        if self.normalize_observation:                                  # as Gymnasium's NormalizeObservation
+            self.single_observation_space = Box(-np.inf, np.inf, (D,))
         n, dev = self.num_envs, self.device
         self.state = torch.zeros(n, 4, dtype=torch.float64, device=dev)
         self.steps = torch.zeros(n, dtype=torch.int32, device=dev)
         self.episode = torch.zeros(n, dtype=torch.int64, device=dev)
         self.ep_return = torch.zeros(n, dtype=torch.float64, device=dev)
         self.cur_obs = torch.zeros(n, D, dtype=torch.float32, device=dev)
+        f64 = dict(dtype=torch.float64, device=dev)
+        # normalisation statistics (Gymnasium's RunningMeanStd start: mean 0, var 1, count 1e-4) and the device freeze flag
+        self.obs_mean = torch.zeros(n, D, **f64) if self.normalize_observation else None
+        self.obs_var = torch.ones(n, D, **f64) if self.normalize_observation else None
+        self.obs_count = torch.full((n,), 1e-4, **f64) if self.normalize_observation else None
+        self.return_stats = torch.tensor([0.0, 0.0, 1.0, 1e-4], **f64).repeat(n, 1) if self.normalize_reward else None
+        self._update = torch.ones(1, dtype=torch.int32, device=dev)
+        self._update_running_mean = True
+        ptr = lambda t: None if t is None else t.data_ptr()
         self._st = N.EnvState(self.state.data_ptr(), self.steps.data_ptr(), self.episode.data_ptr(), self.ep_return.data_ptr(),
-                              self.cur_obs.data_ptr())
+                              self.cur_obs.data_ptr(), ptr(self.obs_mean), ptr(self.obs_var), ptr(self.obs_count),
+                              ptr(self.return_stats), self._update.data_ptr())
         f = dict(dtype=torch.float32, device=dev)
         self._row = dict(next_obs=torch.empty(1, n, D, **f), rew=torch.empty(1, n, **f), term=torch.empty(1, n, **f),
-                         trunc=torch.empty(1, n, **f))
+                         trunc=torch.empty(1, n, **f), raw=torch.empty(1, n, **f) if self.normalize_reward else None)
+        if self.desc.normalize:
+            self._update.zero_()               # brings the state up without counting anything
         self.ctx.env_reset(self.desc, self._st, None)
+        if self.desc.normalize:
+            self._update.fill_(1)
+
+    # the names of the tensors that hold the environments' state (checkpoints copy them)
+    @property
+    def state_tensors(self) -> tuple:
+        names = ("state", "steps", "episode", "ep_return", "cur_obs")
+        if self.normalize_observation:
+            names += ("obs_mean", "obs_var", "obs_count")
+        if self.normalize_reward:
+            names += ("return_stats",)
+        return names
+
+    @property
+    def update_running_mean(self) -> bool:
+        """Whether steps and resets update the normalisation statistics (Gymnasium's property of the same name).  Setting it is
+        stream-ordered: it takes effect for every launch (and graph replay) enqueued after it."""
+        return self._update_running_mean
+
+    @update_running_mean.setter
+    def update_running_mean(self, value: bool) -> None:
+        self._update_running_mean = bool(value)
+        self._update.fill_(int(self._update_running_mean))
 
     @classmethod
     def factory(cls, env_id: str, **kwargs):
@@ -463,15 +526,18 @@ class DeviceVectorEnv:
         a = self._actions(actions)
         if self._check_actions and bool(((a < 0) | (a >= self.act_dim)).any()):
             raise ValueError(f"{self.env_id} takes actions 0 .. {self.act_dim - 1}; got {a.min().item()} .. {a.max().item()}")
-        self.ctx.env_step(self.desc, self._st, a, 0, False, None, r["next_obs"], None, r["rew"], r["term"], r["trunc"])
+        self.ctx.env_step(self.desc, self._st, a, 0, False, None, r["next_obs"], None, r["rew"], r["term"], r["trunc"],
+                          raw_rewards=r["raw"])
+        info = {} if r["raw"] is None else {"raw_rewards": r["raw"][0].double().cpu().numpy()}
         return (r["next_obs"][0].cpu().numpy(), r["rew"][0].double().cpu().numpy(), r["term"][0].bool().cpu().numpy(),
-                r["trunc"][0].bool().cpu().numpy(), {})
+                r["trunc"][0].bool().cpu().numpy(), info)
 
     def step_into(self, buf, t: int, actions) -> None:
-        """Fused rollout step: row t of the device rollout buffer (obs, next_obs, actions, rewards, terminations, truncations)
-        is written by the kernel, finished environments are reset, `cur_obs` becomes the next step's observations."""
+        """Fused rollout step: row t of the device rollout buffer (obs, next_obs, actions, rewards, terminations, truncations,
+        and raw_rewards when the buffer has that attribute) is written by the kernel, finished environments are reset, `cur_obs`
+        becomes the next step's observations."""
         self.ctx.env_step(self.desc, self._st, self._actions(actions), t, True, buf.obs, buf.next_obs, buf.actions, buf.rewards,
-                          buf.terminations, buf.truncations)
+                          buf.terminations, buf.truncations, raw_rewards=getattr(buf, "raw_rewards", None))
         buf.filled = max(buf.filled, t + 1)
 
     def close(self):

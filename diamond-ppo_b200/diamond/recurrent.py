@@ -527,6 +527,7 @@ class RecurrentPPO:
                 self.ctx.sample_categorical(logits.squeeze(0).contiguous(), self.engine.seed, self.engine.draws, self.engine.env_offset, actions, ro.log_probs[t])
             self.engine.draws += 1
             next_observations, rewards, terminations, truncations, infos = self.envs.step(actions.cpu().numpy())
+            tick_rewards = infos.get("raw_rewards", rewards) if isinstance(infos, dict) else rewards   # raw, if the env normalises
             final_t = torch.as_tensor(np.asarray(next_observations, dtype=np.float32)[None, ...], device=dev)
             if getattr(self.engine, "fused", False):
                 _, next_values, _ = self.engine.forward(final_t, new_hx, None, heads=2)
@@ -546,7 +547,7 @@ class RecurrentPPO:
             hx = new_hx
             prev_dones = dones
             if self.ticker is not None:
-                self.ticker.tick(rewards, dones)
+                self.ticker.tick(tick_rewards, dones)
         ro.filled = T
         self.current_observations, self.current_hx, self.prev_dones = observations, hx, prev_dones
         return ro
@@ -564,6 +565,8 @@ class RecurrentPPO:
         if ro is None:
             ro = self._device_ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev, A if cont else None)
             ro.next_obs = torch.empty(T, N_, self.obs_dim, device=dev)
+            # rewards are normalised: the raw ones feed the Ticker
+            ro.raw_rewards = torch.empty(T, N_, device=dev) if getattr(envs, "normalize_reward", False) else None
             ro.pd_u8 = torch.zeros(N_, dtype=torch.uint8, device=dev)
             ro.actions_dev = torch.empty(N_, A, device=dev) if cont else torch.empty(N_, dtype=torch.int64, device=dev)
             ro.pd_f32, ro.pd_bool = torch.empty(N_, device=dev), torch.zeros(N_, dtype=torch.bool, device=dev)
@@ -591,7 +594,7 @@ class RecurrentPPO:
                 # environment kernel: writes obs[t] (the observation acted on), next_obs[t] (true final observation), rewards, masks;
                 # finished environments are reset in the same kernel
                 ctx.env_step(envs.desc, envs._st, ro.actions_dev, t, True, ro.obs, ro.next_obs, None, ro.rewards, ro.terminations,
-                             ro.truncations)
+                             ro.truncations, raw_rewards=ro.raw_rewards)
                 # V(final observation | h_{t+1}): one more GRU step from the post-step state, no reset (recurrent_ppo.py:226-232)
                 ctx.rnn_forward(eng.desc, eng.P, ro.next_obs[t], None, new_hx, 1, N_, 2, None, ro.nv1, ro.hx_buf[2], ro.ws1)
                 ro.next_values[t].copy_(ro.nv1)

@@ -354,7 +354,26 @@ int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* desc, const floa
  * classic-control dynamics, float64 state; MountainCarContinuous keeps Gymnasium's float32 state), 2 / 3: synthetic discrete /
  * continuous (i.i.d. normal observations; the scale benchmark's shape stand-in).  Autoreset-DISABLED contract: next_obs[t]
  * is the true final observation; with auto_reset != 0 finished environments are then reset inside the same kernel and
- * cur_obs holds the post-reset observation (ppo.py:174-179), else the caller resets them with dppo_env_reset(mask). */
+ * cur_obs holds the post-reset observation (ppo.py:174-179), else the caller resets them with dppo_env_reset(mask).
+ *
+ * Normalisation (normalize != 0): every environment e keeps its own float64 statistics, as one Gymnasium NormalizeObservation /
+ * NormalizeReward(gamma) wrapper per sub-environment would; the kernel that steps e updates them in the same thread (warp).
+ *   Observations: mean[e, D] (start 0), var[e, D] (start 1), count[e] (start 1e-4).  Every observation the environment emits
+ *   updates them before it is normalised: each step's true final observation (next_obs[t]) and each post-reset observation (the
+ *   in-kernel reset and dppo_env_reset).  The update is RunningMeanStd.update on a batch of one float32 observation x widened to
+ *   double: delta = x - mean; tot = count + 1; mean += delta * 1 / tot; var = (var * count + 0 + delta^2 * count * 1 / tot) / tot;
+ *   count = tot.  The environment emits float32((x - mean) / sqrt(var + epsilon)), then clipped to [-clip_observation,
+ *   clip_observation] in float32.  Every operation is an explicitly rounded double intrinsic, so the statistics are bit-identical
+ *   to a float64 NumPy restatement.  next_obs[t] and cur_obs of an environment that did not finish are the same float32 values.
+ *   Rewards: per step acc = acc * gamma * (1 - terminated) + r (r: the float64 reward of the dynamics); a scalar RunningMeanStd
+ *   (mean 0, var 1, count 1e-4) is updated with acc; rewards[t] receives r / sqrt(var + epsilon), clipped to [-clip_reward,
+ *   clip_reward] in double, then cast to float32.  As in Gymnasium's NormalizeReward the accumulator is cut by termination
+ *   only: not by truncation, and not by a reset.  Episode returns (ep_return, done_return) stay raw.
+ *   *update == 0 (read by the kernel at run time, so replayed CUDA graphs follow it) freezes both sets of statistics
+ *   (Gymnasium's update_running_mean); the reward accumulator keeps running.
+ * Zero-initialised fields (normalize = 0) leave the environments exactly as without them. */
+#define DPPO_ENV_NORMALIZE_OBS 1
+#define DPPO_ENV_NORMALIZE_REWARD 2
 typedef struct dppo_env_desc {
     int32_t kind;
     int32_t num_envs;
@@ -363,6 +382,12 @@ typedef struct dppo_env_desc {
     uint64_t seed;          /* reset / synthetic draws: Philox4x32-10 keyed by (seed, env_offset + env, episode or step) */
     int64_t env_offset;     /* global id of env 0 (env-sharded data parallelism) */
     float p_term, p_trunc;  /* synthetic kinds only */
+    int32_t normalize;      /* DPPO_ENV_NORMALIZE_OBS | DPPO_ENV_NORMALIZE_REWARD; 0: off */
+    int32_t pad0;
+    double gamma;           /* reward discount of the return accumulator, in [0, 1] */
+    double epsilon;         /* > 0 when normalising */
+    double clip_observation;/* >= 0; 0: no clip */
+    double clip_reward;     /* >= 0; 0: no clip */
 } dppo_env_desc;
 typedef struct dppo_env_state {  /* caller-allocated device buffers */
     double* state;          /* [N, 4] */
@@ -370,15 +395,24 @@ typedef struct dppo_env_state {  /* caller-allocated device buffers */
     int64_t* episode;       /* [N] episodes started */
     double* ep_return;      /* [N] running return of the current episode */
     float* cur_obs;         /* [N, D] observation the next sampling step reads */
+    double* obs_mean;       /* [N, D] observation normalisation (may be NULL without DPPO_ENV_NORMALIZE_OBS) */
+    double* obs_var;        /* [N, D] */
+    double* obs_count;      /* [N] */
+    double* ret_stats;      /* [N, 4] accumulated discounted return, its running mean, variance, count (DPPO_ENV_NORMALIZE_REWARD) */
+    const int32_t* update;  /* device int32 [1]: nonzero updates the statistics (required when normalising) */
 } dppo_env_state;
-/* mask: uint8 [N] (NULL: reset every environment). */
+/* mask: uint8 [N] (NULL: reset every environment).  Refused before any launch: normalisation with a NULL statistics buffer or
+ * update flag, gamma outside [0, 1], epsilon <= 0, a negative clip, unknown normalize bits.  With normalisation on, the synthetic
+ * kinds keep the raw first observation feature (which their reward reads) in state[e, 0]. */
 int dppo_env_reset(dppo_ctx* ctx, const dppo_env_desc* desc, const dppo_env_state* state, const unsigned char* mask, void* stream);
 /* actions: int64 [N] (what dppo_sample_categorical writes) or f32 [N, A].  obs / next_obs / buf_actions / rewards /
  * terminations / truncations are the BASES of the [T, N, ...] buffers (obs and buf_actions may be NULL); row t is written with
- * the casts of ppo.py:229-232.  done_return (optional, f32 [N]) receives the return of every episode that ended at this step. */
+ * the casts of ppo.py:229-232.  done_return (optional, f32 [N]) receives the return of every episode that ended at this step.
+ * raw_rewards (optional) is the base of a [T, N] f32 buffer whose row t receives the rewards before normalisation (the same
+ * values as rewards[t] when the descriptor does not normalise rewards). */
 int dppo_env_step(dppo_ctx* ctx, const dppo_env_desc* desc, const dppo_env_state* state, const void* actions, int t, int auto_reset,
                   float* obs, float* next_obs, void* buf_actions, float* rewards, float* terminations, float* truncations,
-                  float* done_return, void* stream);
+                  float* done_return, float* raw_rewards, void* stream);
 
 /* ---- device-side episode statistics (SURVEY.md 8 f4) ------------------------------------------- */
 /* Replaces the per-step host Ticker.tick(rewards, dones) (diamond/utils.py:99-123, call site ppo.py:181-182) for rollouts that
