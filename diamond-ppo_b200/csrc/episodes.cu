@@ -44,6 +44,41 @@ episode_scan_kernel(const float* __restrict__ rewards, const float* __restrict__
     if (threadIdx.x == 0) atomicAdd(finished, s[0] + s[1] + s[2] + s[3]);
 }
 
+// Evaluation bookkeeping: the arithmetic of episode_scan_kernel (f32 rewards summed in fp64, length + 1 per step, done = termination
+// | truncation, running values carried across chunks), but environment e keeps only its first quota[e] finished episodes, in
+// out[slot_offset[e] + k], and counts itself off `remaining` when it reaches its quota.
+__global__ void __launch_bounds__(128)
+eval_episodes_kernel(const float* __restrict__ rewards, const float* __restrict__ terms, const float* __restrict__ truncs, int T, int N,
+                     const int* __restrict__ quota, const int64_t* __restrict__ slot_offset, double* __restrict__ ep_return,
+                     int* __restrict__ ep_len, int* __restrict__ recorded, double* __restrict__ out_ret, int* __restrict__ out_len,
+                     int* __restrict__ remaining)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= N) return;
+    const int q = quota[e];
+    const int64_t base = slot_offset[e];
+    double ret = ep_return[e];
+    int len = ep_len[e];
+    int k = recorded[e];
+    for (int t = 0; t < T; ++t) {
+        const int64_t i = (int64_t)t * N + e;
+        ret += (double)rewards[i];
+        len += 1;
+        if (terms[i] != 0.0f || truncs[i] != 0.0f) {
+            if (k < q) {
+                out_ret[base + k] = ret;
+                out_len[base + k] = len;
+                if (++k == q) atomicSub(remaining, 1);
+            }
+            ret = 0.0;
+            len = 0;
+        }
+    }
+    ep_return[e] = ret;
+    ep_len[e] = len;
+    recorded[e] = k;
+}
+
 constexpr int WIN_THREADS = 1024;
 
 __global__ void __launch_bounds__(WIN_THREADS)
@@ -107,5 +142,20 @@ extern "C" int dppo_episode_stats(dppo_ctx* ctx, const float* rewards, const flo
     DPPO_CHECK_LAUNCH(ctx, "episode_scan_kernel");
     episode_window_kernel<<<1, WIN_THREADS, 0, st>>>(ev_ret, ev_len, T, N, window, finished, out_returns, out_lengths, out_n);
     DPPO_CHECK_LAUNCH(ctx, "episode_window_kernel");
+    return 0;
+}
+
+extern "C" int dppo_eval_episodes(dppo_ctx* ctx, const float* rewards, const float* terminations, const float* truncations, int T, int N,
+                                  const int32_t* quota, const int64_t* slot_offset, double* ep_return, int32_t* ep_len, int32_t* recorded,
+                                  double* out_returns, int32_t* out_lengths, int32_t* remaining, void* stream)
+{
+    if (!ctx) return 1;
+    if (!rewards || !terminations || !truncations || !quota || !slot_offset || !ep_return || !ep_len || !recorded || !out_returns ||
+        !out_lengths || !remaining)
+        DPPO_FAIL(ctx, "eval_episodes: null argument");
+    if (T < 1 || N < 1) DPPO_FAIL(ctx, "eval_episodes: bad shape T=%d N=%d", T, N);
+    eval_episodes_kernel<<<(N + 127) / 128, 128, 0, (cudaStream_t)stream>>>(rewards, terminations, truncations, T, N, quota, slot_offset,
+                                                                              ep_return, ep_len, recorded, out_returns, out_lengths, remaining);
+    DPPO_CHECK_LAUNCH(ctx, "eval_episodes_kernel");
     return 0;
 }

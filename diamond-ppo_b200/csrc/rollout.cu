@@ -48,6 +48,30 @@ __global__ void sample_categorical_kernel(const float* __restrict__ logits, int 
     if (logp) logp[e] = z[a] - (mx + logf(s));
 }
 
+// Greedy action of a categorical policy: torch.argmax(logits, -1) -- the first index of the maximum, where a NaN counts as the
+// maximum (so the first NaN of a row wins).  The log-prob is sample_categorical_kernel's formula.
+__global__ void select_greedy_categorical_kernel(const float* __restrict__ logits, int N, int A, int64_t* __restrict__ actions,
+                                                 float* __restrict__ logp)
+{
+    const int e = blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= N) return;
+    const float* z = logits + (int64_t)e * A;
+    float best = z[0];
+    int a = 0;
+    for (int j = 1; j < A && !isnan(best); ++j) {
+        const float v = z[j];
+        if (isnan(v) || v > best) { best = v; a = j; }
+    }
+    actions[e] = a;
+    if (logp) {
+        float mx = -CUDART_INF_F;
+        for (int j = 0; j < A; ++j) mx = fmaxf(mx, z[j]);
+        float s = 0.f;
+        for (int j = 0; j < A; ++j) s += expf(z[j] - mx);
+        logp[e] = z[a] - (mx + logf(s));
+    }
+}
+
 __global__ void sample_gaussian_kernel(const float* __restrict__ mean, const float* __restrict__ log_std, int N, int A,
                                        uint64_t seed, uint64_t counter, const unsigned long long* __restrict__ counter_base,
                                        int64_t env_offset, float* __restrict__ actions, float* __restrict__ logp)
@@ -148,6 +172,17 @@ extern "C" int dppo_sample_categorical(dppo_ctx* ctx, const float* logits, int N
     if (N <= 0 || A <= 0) DPPO_FAIL(ctx, "sample_categorical: bad shape N=%d A=%d", N, A);
     sample_categorical_kernel<<<(N + 127) / 128, 128, 0, (cudaStream_t)stream>>>(logits, N, A, seed, counter, ctx->draw_base, env_offset, actions, log_probs);
     DPPO_CHECK_LAUNCH(ctx, "sample_categorical_kernel");
+    return 0;
+}
+
+extern "C" int dppo_select_greedy_categorical(dppo_ctx* ctx, const float* logits, int N, int A, int64_t* actions, float* log_probs,
+                                              void* stream)
+{
+    if (!ctx) return 1;
+    if (N <= 0 || A <= 0) DPPO_FAIL(ctx, "select_greedy_categorical: bad shape N=%d A=%d", N, A);
+    if (!logits || !actions) DPPO_FAIL(ctx, "select_greedy_categorical: null argument");
+    select_greedy_categorical_kernel<<<(N + 127) / 128, 128, 0, (cudaStream_t)stream>>>(logits, N, A, actions, log_probs);
+    DPPO_CHECK_LAUNCH(ctx, "select_greedy_categorical_kernel");
     return 0;
 }
 

@@ -73,6 +73,7 @@ EXPORTS = [
     "dppo_tc_colsum_parts", "dppo_tc_wgrad_f32", "dppo_tc_wgrad_workspace_bytes", "dppo_tc_mma_probe", "dppo_dp_create", "dppo_dp_handle_bytes", "dppo_dp_handle", "dppo_dp_connect", "dppo_dp_destroy", "dppo_dp_status",
     "dppo_permutation_device", "dppo_perm_shard_filter", "dppo_dp_slot", "dppo_dp_zero_slot", "dppo_dp_workspace_bytes", "dppo_dp_allreduce_clip_adam",
     "dppo_env_reset", "dppo_env_step", "dppo_set_draw_counter_base", "dppo_episode_stats", "dppo_episode_stats_workspace_bytes",
+    "dppo_select_greedy_categorical", "dppo_eval_episodes",
     "dppo_rnn_layout_compute", "dppo_rnn_workspace_bytes", "dppo_rnn_forward", "dppo_rnn_grad_minibatch",
 ]
 
@@ -281,6 +282,14 @@ class Context:
         self.launches += 1
         return actions
 
+    def select_greedy_categorical(self, logits, actions=None, log_probs=None):
+        """torch.argmax(logits, -1) (first maximum, NaN counts as the maximum) -> int64 [N] (dppo_select_greedy_categorical)."""
+        N, A = logits.shape
+        actions = torch.empty(N, dtype=torch.int64, device=logits.device) if actions is None else actions
+        self._check(self.lib.dppo_select_greedy_categorical(self.h, _ptr(logits), C.c_int(N), C.c_int(A), _ptr(actions), _ptr(log_probs),
+                                                            _stream()), "dppo_select_greedy_categorical")
+        return actions
+
     def set_draw_counter_base(self, counter_base):
         """counter_base: device int64/uint64 tensor [1] (None clears); added to every sampling draw counter at run time."""
         self._check(self.lib.dppo_set_draw_counter_base(self.h, _ptr(counter_base)), "dppo_set_draw_counter_base")
@@ -377,6 +386,14 @@ class Context:
                                                 _ptr(out_n), _ptr(finished), _ptr(ws), C.c_int64(ws.numel() * ws.element_size()),
                                                 _stream()), "dppo_episode_stats")
         self.launches += 2
+
+    def eval_episodes(self, rewards, terminations, truncations, quota, slot_offset, ep_return, ep_len, recorded, out_returns, out_lengths,
+                      remaining):
+        """Evaluation bookkeeping of one [T, N] chunk (dppo_eval_episodes)."""
+        T, N = rewards.shape
+        self._check(self.lib.dppo_eval_episodes(self.h, _ptr(rewards), _ptr(terminations), _ptr(truncations), C.c_int(T), C.c_int(N),
+                                                _ptr(quota), _ptr(slot_offset), _ptr(ep_return), _ptr(ep_len), _ptr(recorded),
+                                                _ptr(out_returns), _ptr(out_lengths), _ptr(remaining), _stream()), "dppo_eval_episodes")
 
     def episode_stats_workspace_bytes(self, T, N):
         return int(self.lib.dppo_episode_stats_workspace_bytes(C.c_int(T), C.c_int(N)))

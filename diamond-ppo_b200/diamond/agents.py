@@ -25,6 +25,7 @@ import torch.nn as nn
 
 from . import _native as N
 from .config import PPOConfig, ContinuousPPOConfig
+from .evaluation import PolicyEvaluation, as_device_obs, select_actions, shared_log_std
 from .flat import FlatMlp
 from .networks import ActorCriticNetwork, ContinuousActorCriticNetwork, network_parameter_init_
 from .utils import Ticker, Logger, Timer, Checkpointer
@@ -468,6 +469,8 @@ class _EngineBase:
 
 class FusedMlpEngine(_EngineBase):
     """learn() for the default MLP networks: libdppo kernels only."""
+
+    fused = True
 
     def __init__(self, ctx, network, cfg, obs_dim, act_dim, continuous, device, dist: _Dist):
         self.ctx, self.cfg, self.device, self.dist, self.continuous = ctx, cfg, device, dist, continuous
@@ -1014,7 +1017,7 @@ class AutogradEngine(_EngineBase):
 # ------------------------------------------------------------------------------------------------
 # Agents
 # ------------------------------------------------------------------------------------------------
-class _PPOBase:
+class _PPOBase(PolicyEvaluation):
     _continuous = False
     _default_network: Any = None
 
@@ -1029,6 +1032,7 @@ class _PPOBase:
         if self._dist.perm_mode == "numpy":
             self._dist.sync_numpy_stream(self.device)
 
+        self._env_fn = env_fn                                          # evaluate() builds new environments from it
         if getattr(env_fn, "vectorized", False):                       # additive: env_fn(num_envs) -> batched vector env
             self.envs = env_fn(cfg.num_envs)
             # env-sharded data parallelism: this rank simulates global envs [rank*N, (rank+1)*N) -- distinct reset / dynamics
@@ -1137,6 +1141,33 @@ class _PPOBase:
                 self.ticker.tick(tick_rewards, dones)
         self.current_observations = observations
         return buf
+
+    # ---- evaluation (diamond/evaluation.py) --------------------------------------------------------------------------
+    def predict(self, observations, deterministic: bool = True):
+        """Actions of the current policy for observations [n, obs_dim]: a host array in, a NumPy array out; a device tensor in, a
+        device tensor out.  deterministic=True: the greedy action (the first argmax of the logits, or the Gaussian means, not
+        clipped); False: a draw of the evaluation generator (its own key and counter: the training sampling counter and the numpy /
+        torch streams do not move).  Default networks run the fused forward and the greedy / sampling kernels; a custom
+        network_cls runs its get_logits_and_values / get_means_log_stds_and_values under inference_mode."""
+        obs = as_device_obs(observations, self.obs_dim, self.device)
+        n = obs.shape[0]
+        eng, log_std = self.engine, None
+        if getattr(eng, "fused", False):
+            head = torch.empty(n, eng.A, dtype=torch.float32, device=self.device)
+            self.ctx.mlp_forward(eng.fm.desc, eng.P, obs, n, 1, head, None, eng.fwd_ws)
+            if self._continuous:
+                log_std = eng.P[eng.fm.layout.log_std:eng.fm.layout.log_std + eng.A]
+        else:
+            with torch.inference_mode():
+                if self._continuous:
+                    head, log_stds, _ = self.network.get_means_log_stds_and_values(obs)
+                    log_std = shared_log_std(log_stds)
+                else:
+                    head, _ = self.network.get_logits_and_values(obs)
+                head = head.reshape(n, -1).contiguous()
+        key, counter = self._eval_draw() if not deterministic else (0, 0)
+        actions = select_actions(self.ctx, head, log_std, deterministic, key, counter, greedy_kernel=getattr(eng, "fused", False))
+        return actions if torch.is_tensor(observations) else actions.cpu().numpy()
 
     # ---- episode statistics of device-resident rollouts (utils.py:99-123 without the per-step host loop) ------------
     def _device_episode_stats(self, buf):

@@ -494,6 +494,20 @@ class DeviceVectorEnv:
         self._update_running_mean = bool(value)
         self._update.fill_(int(self._update_running_mean))
 
+    def load_frozen_statistics(self, source: "DeviceVectorEnv") -> None:
+        """Freezes this environment's normalisation statistics (update_running_mean = False) and gives environment i the
+        statistics of `source`'s environment i mod source.num_envs: obs_mean / obs_var / obs_count and return_stats.  Evaluation
+        environments take them from the training environments this way, which are only read."""
+        torch = self._torch
+        if (self.normalize_observation and not source.normalize_observation) or (self.normalize_reward and not source.normalize_reward):
+            raise ValueError("load_frozen_statistics: the source environments do not keep every statistic this one normalises with")
+        self.update_running_mean = False
+        idx = torch.arange(self.num_envs, device=source.device) % source.num_envs
+        names = (("obs_mean", "obs_var", "obs_count") if self.normalize_observation else ()) + \
+            (("return_stats",) if self.normalize_reward else ())
+        for name in names:
+            getattr(self, name).copy_(getattr(source, name)[idx])
+
     @classmethod
     def factory(cls, env_id: str, **kwargs):
         def env_fn(num_envs):

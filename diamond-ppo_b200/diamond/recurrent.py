@@ -36,6 +36,7 @@ except ImportError:                     # pragma: no cover - the GPU image has n
     from . import envs as gym
 from .agents import _Dist, _EngineBase, _PermWorker, _PPOBase, _require_cuda
 from .config import RecurrentContinuousPPOConfig, RecurrentPPOConfig
+from .evaluation import PolicyEvaluation, as_device_obs, select_actions, shared_log_std
 from .networks import _obs_dim, network_parameter_init_
 from .utils import Checkpointer, Logger, Ticker, Timer
 
@@ -436,9 +437,10 @@ class FusedRecurrentEngine(_EngineBase):
         self.last_losses = losses
 
 
-class RecurrentPPO:
+class RecurrentPPO(PolicyEvaluation):
     """Recurrent (GRU) discrete-action PPO (reference: diamond/recurrent_ppo.py:164-394)."""
     _continuous = False
+    _recurrent = True
     _default_network: Any = RecurrentActorCriticNetwork
 
     def __init__(self, env_fn: Callable[[], Any], cfg: RecurrentPPOConfig = RecurrentPPOConfig(),
@@ -451,6 +453,7 @@ class RecurrentPPO:
             np.random.seed(cfg.seed)                                    # recurrent_ppo.py:173-175
             torch.manual_seed(cfg.seed)
         self._dist = _Dist(process_group, dp, "local", "nccl", "numpy")
+        self._env_fn = env_fn                                            # evaluate() builds new environments from it
         if getattr(env_fn, "vectorized", False):
             self.envs = env_fn(cfg.num_envs)
             if self._dist.enabled and getattr(self.envs, "device_resident", False) and self.envs.desc.env_offset == 0:
@@ -631,6 +634,38 @@ class RecurrentPPO:
             self._device_episode_stats(ro)
         self.current_observations, self.current_hx, self.prev_dones = envs.cur_obs, ro.hx_buf[0].reshape(1, N_, Hg), ro.pd_u8
         return ro
+
+    # ---- evaluation (diamond/evaluation.py) --------------------------------------------------------------------------------
+    def predict(self, observations, hx=None, dones=None, deterministic: bool = True):
+        """One step of the current policy: observations [n, obs_dim], hidden state hx [1, n, Hg] (None: zeros) and dones [n] (None:
+        no resets; True zeroes the hidden state of that environment before the step, as prev_dones in a rollout).  Returns
+        (actions, new_hx): NumPy arrays for host observations, device tensors for device tensors.  deterministic=True: the first
+        argmax of the logits or the Gaussian means (not clipped); False: a draw of the evaluation generator, which leaves the
+        training sampling counter and the numpy / torch streams alone.  The default network runs dppo_rnn_forward and the greedy /
+        sampling kernels; a custom network_cls its get_logits_values_and_hx / get_means_log_stds_values_and_hx under inference_mode."""
+        dev, Hg = self.device, self.cfg.gru_hidden_dim
+        obs = as_device_obs(observations, self.obs_dim, dev)
+        n = obs.shape[0]
+        h = torch.zeros(1, n, Hg, device=dev) if hx is None else as_device_obs(hx, Hg, dev).reshape(1, n, Hg)
+        pd = None if dones is None else torch.as_tensor(np.asarray(dones) if not torch.is_tensor(dones) else dones).to(dev, torch.bool).reshape(1, n)
+        eng, log_std = self.engine, None
+        if getattr(eng, "fused", False):
+            head, _, new_hx = eng.forward(obs.reshape(1, n, -1), h, pd, heads=1)
+            log_std = eng.log_std
+        else:
+            with torch.inference_mode():
+                if self._continuous:
+                    head, log_stds, _, new_hx = self.network.get_means_log_stds_values_and_hx(obs.reshape(1, n, -1), h, pd)
+                    log_std = shared_log_std(log_stds.reshape(n, -1))
+                else:
+                    head, _, new_hx = self.network.get_logits_values_and_hx(obs.reshape(1, n, -1), h, pd)
+        head = head.reshape(n, -1).contiguous()
+        key, counter = self._eval_draw() if not deterministic else (0, 0)
+        actions = select_actions(self.ctx, head, log_std, deterministic, key, counter, greedy_kernel=getattr(eng, "fused", False))
+        new_hx = new_hx.reshape(1, n, Hg).clone()
+        if torch.is_tensor(observations):
+            return actions, new_hx
+        return actions.cpu().numpy(), new_hx.cpu().numpy()
 
     # ---- GAE (recurrent_ppo.py:265-299) ----------------------------------------------------------------
     def calculate_advantage(self, rewards, terminations, truncations, values, next_values) -> torch.Tensor:

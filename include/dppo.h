@@ -128,6 +128,11 @@ int64_t dppo_step_record_bytes(int N, int D, int act_dim, int continuous);
  * Also emits log_prob(action) (recurrent_ppo.py:219-221).  actions: int64 [N]. */
 int dppo_sample_categorical(dppo_ctx* ctx, const float* logits, int N, int A, uint64_t seed, uint64_t counter,
                             int64_t env_offset, int64_t* actions, float* log_probs, void* stream);
+/* Greedy action of a categorical policy (evaluation): actions[e] = torch.argmax(logits[e], -1), the FIRST index of the row's
+ * maximum; a NaN counts as the maximum, so a row holding a NaN selects its first NaN.  log_probs (optional) receives
+ * log_softmax(logits[e])[actions[e]] with the arithmetic of dppo_sample_categorical.  No generator is involved.  The greedy action of
+ * a Gaussian policy is its mean (heads bit 0 of dppo_mlp_forward / dppo_rnn_forward), which needs no kernel of its own. */
+int dppo_select_greedy_categorical(dppo_ctx* ctx, const float* logits, int N, int A, int64_t* actions, float* log_probs, void* stream);
 /* JointNormal(mean, exp(log_std)).sample() (continuous_ppo.py:92). actions: f32 [N, A]. */
 int dppo_sample_gaussian(dppo_ctx* ctx, const float* mean, const float* log_std, int N, int A, uint64_t seed,
                          uint64_t counter, int64_t env_offset, float* actions, float* log_probs, void* stream);
@@ -424,6 +429,16 @@ int64_t dppo_episode_stats_workspace_bytes(int T, int N);
 int dppo_episode_stats(dppo_ctx* ctx, const float* rewards, const float* terminations, const float* truncations, int T, int N,
                        double* ep_return, int32_t* ep_len, int window, double* out_returns, int32_t* out_lengths, int32_t* out_n,
                        unsigned long long* finished, void* ws, int64_t ws_bytes, void* stream);
+/* Episode bookkeeping of an evaluation, one launch per chunk of T steps of N environments ([T, N] rewards / terminations /
+ * truncations).  The arithmetic of dppo_episode_stats: f32 rewards summed in fp64, length + 1 per step, done = termination |
+ * truncation; the running return and length in ep_return / ep_len carry across chunks (caller zeroes them with the reset).
+ * Environment e records only its first quota[e] finished episodes: the k-th (k counted by recorded[e], caller zeroes it) goes to
+ * out_returns / out_lengths[slot_offset[e] + k].  When recorded[e] reaches quota[e], *remaining is decremented once (the caller
+ * sets it to the number of environments with quota > 0, so it reads 0 when every quota is met).  Later episodes of e are ignored,
+ * so an environment past its quota may keep stepping and every launch keeps its shape. */
+int dppo_eval_episodes(dppo_ctx* ctx, const float* rewards, const float* terminations, const float* truncations, int T, int N,
+                       const int32_t* quota, const int64_t* slot_offset, double* ep_return, int32_t* ep_len, int32_t* recorded,
+                       double* out_returns, int32_t* out_lengths, int32_t* remaining, void* stream);
 
 /* ---- tensor-core building blocks of the fused update (unit tests, A/B measurements) ---------- */
 /* C[M,N] = epi(A[M,K] * op(W)) as an error-compensated 3xTF32 tcgen05 GEMM (fp32-accurate, SURVEY.md 0.6) on CTA pairs
