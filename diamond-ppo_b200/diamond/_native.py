@@ -29,7 +29,8 @@ class MlpLayout(C.Structure):
 
 
 class RnnDesc(C.Structure):
-    _fields_ = [("obs_dim", C.c_int32), ("hidden", C.c_int32), ("gru_hidden", C.c_int32), ("act_dim", C.c_int32), ("continuous", C.c_int32)]
+    _fields_ = [("obs_dim", C.c_int32), ("hidden", C.c_int32), ("gru_hidden", C.c_int32), ("act_dim", C.c_int32), ("continuous", C.c_int32),
+                ("cell", C.c_int32)]                                 # cell 0: GRU, 1: LSTM (hx packed h | c, [N, 2 gru_hidden])
 
 
 class RnnLayout(C.Structure):

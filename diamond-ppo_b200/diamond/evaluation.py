@@ -86,16 +86,17 @@ class _MlpDevicePolicy:
 
 
 class _RnnDevicePolicy:
-    """One step of the default GRU network, carrying the hidden state and the prev_dones resets as RecurrentPPO's device rollout."""
+    """One step of the default GRU or LSTM network, carrying the recurrent state and the prev_dones resets as RecurrentPPO's device
+    rollout."""
 
     def __init__(self, agent, n):
         eng, dev = agent.engine, agent.device
         self.ctx, self.eng, self.n = agent.ctx, eng, n
-        A, Hg = eng.desc.act_dim, eng.desc.gru_hidden
+        A, S = eng.desc.act_dim, agent.state_dim
         self.head = torch.empty(n, A, dtype=torch.float32, device=dev)
         self.log_std = eng.log_std
         self.out = torch.empty(n, A, dtype=torch.float32, device=dev) if eng.continuous else torch.empty(n, dtype=torch.int64, device=dev)
-        self.hx = [torch.zeros(n, Hg, dtype=torch.float32, device=dev) for _ in range(2)]
+        self.hx = [torch.zeros(n, S, dtype=torch.float32, device=dev) for _ in range(2)]
         self.pd_u8 = torch.zeros(n, dtype=torch.uint8, device=dev)
         self.pd_f32, self.pd_bool = torch.empty(n, device=dev), torch.zeros(n, dtype=torch.bool, device=dev)
         self.ws = eng._workspace(1, n, n, False)

@@ -18,6 +18,12 @@ every call; the intended `is None` semantics are implemented (SURVEY.md §0.4).
 Beyond the reference: `RecurrentContinuousPPO` / `RecurrentContinuousActorCriticNetwork`, the same agent with a Gaussian policy for
 Box action spaces (the heads of continuous_ppo.py on the GRU trunk).  It runs the same code, selected by the class attribute
 `_continuous` as in agents.py, and the same kernels (the Gaussian instantiation of the head kernel in dppo_rnn_grad_minibatch).
+
+LSTM networks: `RecurrentLSTMActorCriticNetwork` / `RecurrentContinuousLSTMActorCriticNetwork` (pass one as network_cls) replace
+the GRU core with `LSTMCore` (nn.LSTM's parameters, width cfg.gru_hidden_dim) and run on the fused kernels too (dppo_rnn_desc.cell
+= 1).  Their recurrent state is one tensor [1, N, 2 Hg], h | c.  The agent sizes every recurrent buffer by the network's
+`recurrent_state_dim` (cfg.gru_hidden_dim when a network has none), so a custom LSTM network_cls with that attribute runs on the
+autograd engine.
 """
 from __future__ import annotations
 
@@ -71,6 +77,46 @@ class GRUCore(nn.GRU):
         return torch.stack(outs, dim=0), h.unsqueeze(0)
 
 
+class LSTMCore(nn.LSTM):
+    """LSTM with per-timestep state resets, the counterpart of GRUCore.  Parameters are nn.LSTM's (`weight_ih_l0 [4Hg, H]`,
+    `weight_hh_l0 [4Hg, Hg]`, `bias_ih_l0`, `bias_hh_l0`; gate order i, f, g, o), so state dicts load into torch.nn.LSTM.  The
+    state is packed into one tensor hx [1, B, 2Hg]: h in [..., :Hg], c in [..., Hg:]; where dones[t] is set both are zeroed before
+    step t (the GRU's recurrent_ppo.py:84 rule)."""
+
+    def __init__(self, input_dim: int, hidden_dim: int) -> None:
+        super().__init__(input_dim, hidden_dim)
+
+    def forward(self, x: torch.Tensor, hx: torch.Tensor | None, dones: torch.Tensor | None):
+        T, B = x.shape[:2]
+        Hg = self.hidden_size
+        if hx is None:
+            h = torch.zeros(B, Hg, dtype=x.dtype, device=x.device)
+            c = torch.zeros(B, Hg, dtype=x.dtype, device=x.device)
+        else:
+            hc = hx.reshape(B, 2 * Hg)
+            h, c = hc[:, :Hg], hc[:, Hg:]
+        # all T input projections in one GEMM; only the hidden-to-hidden product is sequential
+        gi = torch.addmm(self.bias_ih_l0, x.reshape(T * B, -1), self.weight_ih_l0.t()).view(T, B, 4 * Hg)
+        keep = None if dones is None else (~dones.to(torch.bool)).to(x.dtype).unsqueeze(-1)      # [T, B, 1]
+        outs = []
+        for t in range(T):
+            if keep is not None:
+                h, c = h * keep[t], c * keep[t]
+            gates = gi[t] + torch.addmm(self.bias_hh_l0, h, self.weight_hh_l0.t())
+            i, f, g, o = gates.chunk(4, dim=-1)
+            c = torch.sigmoid(f) * c + torch.sigmoid(i) * torch.tanh(g)
+            h = torch.sigmoid(o) * torch.tanh(c)
+            outs.append(h)
+        return torch.stack(outs, dim=0), torch.cat([h, c], dim=-1).unsqueeze(0)
+
+
+def _lstm_width(cfg) -> int:
+    hg = int(cfg.gru_hidden_dim)
+    if hg % 4 != 0 or not 8 <= hg <= 256:
+        raise ValueError(f"LSTM networks need gru_hidden_dim a multiple of 4 from 8 to 256 (the fused LSTM scans' widths), got {hg}")
+    return hg
+
+
 class RecurrentActorCriticNetwork(nn.Module):
     """Linear-Tanh -> GRU -> actor / critic heads (recurrent_ppo.py:94-149)."""
 
@@ -119,11 +165,64 @@ class RecurrentContinuousActorCriticNetwork(nn.Module):
         return mean, torch.broadcast_to(self.actor_log_std, mean.shape), self.critic_head(x).squeeze(-1), hx
 
 
+class RecurrentLSTMActorCriticNetwork(nn.Module):
+    """Linear-Tanh -> LSTM (width cfg.gru_hidden_dim) -> RecurrentActorCriticNetwork's actor / critic heads.  The recurrent state is
+    hx [1, B, 2Hg], h | c (recurrent_state_dim)."""
+
+    def __init__(self, observation_space, action_space, cfg: RecurrentPPOConfig) -> None:
+        super().__init__()
+        assert hasattr(action_space, "n"), "Only Discrete action spaces are supported."
+        hg = _lstm_width(cfg)
+        d, h = _obs_dim(observation_space), int(cfg.network_hidden_dim)
+        self.recurrent_state_dim = 2 * hg
+        self.base = nn.Sequential(nn.Linear(d, h), nn.Tanh())
+        self.lstm = LSTMCore(h, hg)
+        self.actor_head = nn.Sequential(nn.Linear(hg, h), nn.Tanh(), nn.Linear(h, int(action_space.n)))
+        self.actor_out_layer = self.actor_head[-1]
+        self.critic_head = nn.Sequential(nn.Linear(hg, h), nn.Tanh(), nn.Linear(h, 1))
+
+    def get_values(self, observations, hx, dones) -> torch.Tensor:
+        x, _ = self.lstm.forward(self.base(observations), hx, dones)
+        return self.critic_head(x).squeeze(-1)
+
+    def get_logits_values_and_hx(self, observations, hx, dones):
+        x, hx = self.lstm.forward(self.base(observations), hx, dones)
+        return self.actor_head(x), self.critic_head(x).squeeze(-1), hx
+
+
+class RecurrentContinuousLSTMActorCriticNetwork(nn.Module):
+    """Linear-Tanh -> LSTM -> RecurrentContinuousActorCriticNetwork's Gaussian actor / critic heads; hx [1, B, 2Hg], h | c."""
+
+    def __init__(self, observation_space, action_space, cfg: RecurrentContinuousPPOConfig) -> None:
+        super().__init__()
+        assert hasattr(action_space, "shape") and not hasattr(action_space, "n"), "Only Box action spaces are supported."
+        hg = _lstm_width(cfg)
+        d, h = _obs_dim(observation_space), int(cfg.network_hidden_dim)
+        a = int(np.prod(action_space.shape))
+        self.recurrent_state_dim = 2 * hg
+        self.base = nn.Sequential(nn.Linear(d, h), nn.Tanh())
+        self.lstm = LSTMCore(h, hg)
+        self.actor_mean_head = nn.Sequential(nn.Linear(hg, h), nn.Tanh(), nn.Linear(h, a))
+        self.actor_log_std = nn.Parameter(torch.zeros(1, a))
+        self.critic_head = nn.Sequential(nn.Linear(hg, h), nn.Tanh(), nn.Linear(h, 1))
+
+    def get_values(self, observations, hx, dones) -> torch.Tensor:
+        x, _ = self.lstm.forward(self.base(observations), hx, dones)
+        return self.critic_head(x).squeeze(-1)
+
+    def get_means_log_stds_values_and_hx(self, observations, hx, dones):
+        """(mean [T,B,A], log_std broadcast to [T,B,A], values [T,B], hx [1,B,2Hg])."""
+        x, hx = self.lstm.forward(self.base(observations), hx, dones)
+        mean = self.actor_mean_head(x)
+        return mean, torch.broadcast_to(self.actor_log_std, mean.shape), self.critic_head(x).squeeze(-1), hx
+
+
 class RecurrentRollout:
     """Device-resident rollout of the recurrent agent; iterating yields the reference's 10-item step records
-    (recurrent_ppo.py:234-245).  Actions: int64 [T, N], or f32 [T, N, act_dim] when act_dim is given (Gaussian policy)."""
+    (recurrent_ppo.py:234-245).  Actions: int64 [T, N], or f32 [T, N, act_dim] when act_dim is given (Gaussian policy).  S is the
+    width of the recurrent state (the network's recurrent_state_dim: Hg for a GRU, 2 Hg for an LSTM)."""
 
-    def __init__(self, T, N_, D, Hg, device, act_dim=None):
+    def __init__(self, T, N_, D, S, device, act_dim=None):
         f = dict(dtype=torch.float32, device=device)
         self.T, self.N = T, N_
         self.obs = torch.empty(T, N_, D, **f)
@@ -131,7 +230,7 @@ class RecurrentRollout:
         self.rewards, self.terminations, self.truncations = (torch.empty(T, N_, **f) for _ in range(3))
         self.prev_dones = torch.empty(T, N_, dtype=torch.bool, device=device)
         self.log_probs, self.values, self.next_values = (torch.empty(T, N_, **f) for _ in range(3))
-        self.hx0 = torch.zeros(1, N_, Hg, **f)
+        self.hx0 = torch.zeros(1, N_, S, **f)
         self.filled = 0
 
     @staticmethod
@@ -258,14 +357,15 @@ class RecurrentEngine(_EngineBase):
 
 
 def rnn_param_slices(desc: N.RnnDesc, lay: N.RnnLayout):
-    """name (reference module naming, recurrent_ppo.py:101-125; RecurrentContinuousActorCriticNetwork's when desc.continuous)
-    -> (offset, shape) in the flat buffers (dppo_rnn_layout)."""
+    """name (reference module naming, recurrent_ppo.py:101-125; RecurrentContinuousActorCriticNetwork's when desc.continuous;
+    the LSTM networks' lstm.* tensors of 4 Hg rows when desc.cell == 1) -> (offset, shape) in the flat buffers (dppo_rnn_layout)."""
     D, H, Hg, A = desc.obs_dim, desc.hidden, desc.gru_hidden, desc.act_dim
     actor = "actor_mean_head" if desc.continuous else "actor_head"
+    core, G = ("lstm", 4 * Hg) if desc.cell else ("gru", 3 * Hg)
     s = {
         "base.0.weight": (lay.w1, (H, D)), "base.0.bias": (lay.b1, (H,)),
-        "gru.weight_ih_l0": (lay.wih, (3 * Hg, H)), "gru.weight_hh_l0": (lay.whh, (3 * Hg, Hg)),
-        "gru.bias_ih_l0": (lay.bih, (3 * Hg,)), "gru.bias_hh_l0": (lay.bhh, (3 * Hg,)),
+        f"{core}.weight_ih_l0": (lay.wih, (G, H)), f"{core}.weight_hh_l0": (lay.whh, (G, Hg)),
+        f"{core}.bias_ih_l0": (lay.bih, (G,)), f"{core}.bias_hh_l0": (lay.bhh, (G,)),
         f"{actor}.0.weight": (lay.w3, (H, Hg)), f"{actor}.0.bias": (lay.b3, (H,)),
         f"{actor}.2.weight": (lay.wa, (A, H)), f"{actor}.2.bias": (lay.ba, (A,)),
         "critic_head.0.weight": (lay.w3 + H * Hg, (H, Hg)), "critic_head.0.bias": (lay.b3 + H, (H,)),
@@ -277,15 +377,16 @@ def rnn_param_slices(desc: N.RnnDesc, lay: N.RnnLayout):
 
 
 class FusedRecurrentEngine(_EngineBase):
-    """learn() / forward of the default recurrent network on the libdppo kernels only (csrc/rnn.cu)."""
+    """learn() / forward of the default GRU or LSTM recurrent network on the libdppo kernels only (csrc/rnn.cu)."""
 
     fused = True
 
-    def __init__(self, ctx, network, cfg, obs_dim, act_dim, device, dist: _Dist | None = None, continuous=False):
+    def __init__(self, ctx, network, cfg, obs_dim, act_dim, device, dist: _Dist | None = None, continuous=False, lstm=False):
         self.ctx, self.cfg, self.device, self.continuous = ctx, cfg, device, continuous
         self.dist = dist if dist is not None else _Dist(None, False)
         self.network = network
-        self.desc = N.RnnDesc(int(obs_dim), int(cfg.network_hidden_dim), int(cfg.gru_hidden_dim), int(act_dim), int(continuous))
+        self.desc = N.RnnDesc(int(obs_dim), int(cfg.network_hidden_dim), int(cfg.gru_hidden_dim), int(act_dim), int(continuous), int(lstm))
+        self.state_dim = (2 if lstm else 1) * int(cfg.gru_hidden_dim)
         self.layout = N.rnn_layout(self.desc)
         self._adopt(network, rnn_param_slices(self.desc, self.layout), int(self.layout.total))
         # Gaussian policy: the actor_log_std [A] the sampling kernel reads (a view of the flat parameter buffer)
@@ -306,13 +407,13 @@ class FusedRecurrentEngine(_EngineBase):
         return self._ws[key]
 
     def forward(self, obs, hx, prev_dones, heads=3):
-        """(logits [T,N,A], values [T,N], hx [1,N,Hg]) of get_logits_values_and_hx / get_values (recurrent_ppo.py:127-149); with
-        a Gaussian policy the first output holds the action means."""
+        """(logits [T,N,A], values [T,N], hx [1,N,S]) of get_logits_values_and_hx / get_values (recurrent_ppo.py:127-149); with
+        a Gaussian policy the first output holds the action means.  S = state_dim (LSTM: h | c)."""
         T, N_ = obs.shape[:2]
-        dev, A, Hg = self.device, self.desc.act_dim, self.desc.gru_hidden
+        dev, A = self.device, self.desc.act_dim
         logits = torch.empty(T, N_, A, device=dev) if heads & 1 else None
         values = torch.empty(T, N_, device=dev) if heads & 2 else None
-        hx_out = torch.empty(1, N_, Hg, device=dev)
+        hx_out = torch.empty(1, N_, self.state_dim, device=dev)
         pd = None if prev_dones is None else prev_dones.to(torch.uint8).contiguous()
         self.ctx.rnn_forward(self.desc, self.P, obs.contiguous(), pd, None if hx is None else hx.contiguous(), T, N_, heads,
                              logits, values, hx_out, self._workspace(T, N_, T * N_, False))
@@ -329,7 +430,7 @@ class FusedRecurrentEngine(_EngineBase):
                 h_sets=[[torch.empty(B, dtype=torch.int32).pin_memory() for _ in range(E)] for _ in range(2)], h_set=0, h_consumed=[None, None],
                 old_logp=torch.empty(B, device=dev),
                 actions=torch.empty(B, self.desc.act_dim, device=dev) if self.continuous else torch.empty(B, dtype=torch.int32, device=dev),
-                pd=torch.empty(T, N_, dtype=torch.uint8, device=dev), hx0=torch.empty(N_, self.desc.gru_hidden, device=dev),
+                pd=torch.empty(T, N_, dtype=torch.uint8, device=dev), hx0=torch.empty(N_, self.state_dim, device=dev),
                 values=torch.empty(T, N_, device=dev), next_values=torch.empty(T, N_, device=dev),
                 consts=[torch.zeros(MB, 4, dtype=torch.float32, device=dev) for _ in range(2)],
                 h_consts=[torch.zeros(MB, 4, dtype=torch.float32).pin_memory() for _ in range(2)],
@@ -438,10 +539,12 @@ class FusedRecurrentEngine(_EngineBase):
 
 
 class RecurrentPPO(PolicyEvaluation):
-    """Recurrent (GRU) discrete-action PPO (reference: diamond/recurrent_ppo.py:164-394)."""
+    """Recurrent (GRU) discrete-action PPO (reference: diamond/recurrent_ppo.py:164-394).  network_cls=RecurrentLSTMActorCriticNetwork
+    selects an LSTM core on the same fused kernels."""
     _continuous = False
     _recurrent = True
     _default_network: Any = RecurrentActorCriticNetwork
+    _lstm_network: Any = RecurrentLSTMActorCriticNetwork
 
     def __init__(self, env_fn: Callable[[], Any], cfg: RecurrentPPOConfig = RecurrentPPOConfig(),
                  network_cls: Any = RecurrentActorCriticNetwork, *, process_group=None, dp: bool = False) -> None:
@@ -469,9 +572,11 @@ class RecurrentPPO(PolicyEvaluation):
                 self._dist.dist.broadcast(p.data, src=0, group=self._dist.group)
         self.obs_dim = int(np.prod(obs_space.shape))
         self.act_dim = int(np.prod(act_space.shape)) if self._continuous else int(act_space.n)
-        if type(self.network) is self._default_network:                  # default network: libdppo kernels end to end
+        # width of every recurrent buffer: the network's recurrent_state_dim (LSTM: h | c), else the GRU's gru_hidden_dim
+        self.state_dim = int(getattr(self.network, "recurrent_state_dim", cfg.gru_hidden_dim))
+        if type(self.network) in (self._default_network, self._lstm_network):   # default networks: libdppo kernels end to end
             self.engine = FusedRecurrentEngine(self.ctx, self.network, cfg, self.obs_dim, self.act_dim, self.device, self._dist,
-                                               self._continuous)
+                                               self._continuous, lstm=type(self.network) is self._lstm_network)
         else:                                                            # custom network_cls: the module runs under autograd
             self.engine = RecurrentEngine(self.ctx, self.network, cfg, self.device, self._dist, self._continuous)
         self.optimizer = torch.optim.Adam(self.network.parameters(), lr=cfg.lr, eps=cfg.adam_eps)
@@ -497,7 +602,7 @@ class RecurrentPPO(PolicyEvaluation):
         if getattr(self.envs, "device_resident", False) and getattr(self.engine, "fused", False):
             return self._rollout_device()
         cont = self._continuous
-        ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev, self.act_dim if cont else None)
+        ro = RecurrentRollout(T, N_, self.obs_dim, self.state_dim, dev, self.act_dim if cont else None)
         observations, hx, prev_dones = self.current_observations, self.current_hx, self.prev_dones
         ro.hx0.copy_(hx)
         for t in range(T):
@@ -562,11 +667,11 @@ class RecurrentPPO(PolicyEvaluation):
         persistent, so learn() replays its optimiser steps as CUDA graphs.  Episode statistics: dppo_episode_stats, read lazily."""
         cfg, dev, envs, eng, ctx = self.cfg, self.device, self.envs, self.engine, self.ctx
         T, N_ = cfg.rollout_steps, cfg.num_envs
-        A, Hg = eng.desc.act_dim, eng.desc.gru_hidden
+        A, S = eng.desc.act_dim, self.state_dim
         ro = self._device_ro
         cont = self._continuous
         if ro is None:
-            ro = self._device_ro = RecurrentRollout(T, N_, self.obs_dim, cfg.gru_hidden_dim, dev, A if cont else None)
+            ro = self._device_ro = RecurrentRollout(T, N_, self.obs_dim, S, dev, A if cont else None)
             ro.next_obs = torch.empty(T, N_, self.obs_dim, device=dev)
             # rewards are normalised: the raw ones feed the Ticker
             ro.raw_rewards = torch.empty(T, N_, device=dev) if getattr(envs, "normalize_reward", False) else None
@@ -574,13 +679,13 @@ class RecurrentPPO(PolicyEvaluation):
             ro.actions_dev = torch.empty(N_, A, device=dev) if cont else torch.empty(N_, dtype=torch.int64, device=dev)
             ro.pd_f32, ro.pd_bool = torch.empty(N_, device=dev), torch.zeros(N_, dtype=torch.bool, device=dev)
             ro.logits, ro.val1, ro.nv1 = torch.empty(N_, A, device=dev), torch.empty(N_, device=dev), torch.empty(N_, device=dev)
-            ro.hx_buf = [torch.zeros(N_, Hg, device=dev) for _ in range(3)]      # [0], [1]: ping-pong state; [2]: discarded output
+            ro.hx_buf = [torch.zeros(N_, S, device=dev) for _ in range(3)]      # [0], [1]: ping-pong state; [2]: discarded output
             ro.ws1 = eng._workspace(1, N_, N_, False)
             self._ro_graph, self._ro_seen = None, 0
         if not torch.is_tensor(self.prev_dones):
             ro.pd_u8.copy_(torch.as_tensor(np.asarray(self.prev_dones, dtype=np.uint8)))
         if self.current_hx.data_ptr() != ro.hx_buf[0].data_ptr():
-            ro.hx_buf[0].copy_(self.current_hx.reshape(N_, Hg))
+            ro.hx_buf[0].copy_(self.current_hx.reshape(N_, S))
         ro.hx0.copy_(ro.hx_buf[0].reshape(ro.hx0.shape))
 
         def steps(counter_of):
@@ -632,21 +737,22 @@ class RecurrentPPO(PolicyEvaluation):
         ro.filled = T
         if self.ticker is not None:
             self._device_episode_stats(ro)
-        self.current_observations, self.current_hx, self.prev_dones = envs.cur_obs, ro.hx_buf[0].reshape(1, N_, Hg), ro.pd_u8
+        self.current_observations, self.current_hx, self.prev_dones = envs.cur_obs, ro.hx_buf[0].reshape(1, N_, S), ro.pd_u8
         return ro
 
     # ---- evaluation (diamond/evaluation.py) --------------------------------------------------------------------------------
     def predict(self, observations, hx=None, dones=None, deterministic: bool = True):
-        """One step of the current policy: observations [n, obs_dim], hidden state hx [1, n, Hg] (None: zeros) and dones [n] (None:
+        """One step of the current policy: observations [n, obs_dim], recurrent state hx [1, n, S] (None: zeros; S = state_dim: Hg
+        for a GRU, 2 Hg for an LSTM, h | c) and dones [n] (None:
         no resets; True zeroes the hidden state of that environment before the step, as prev_dones in a rollout).  Returns
         (actions, new_hx): NumPy arrays for host observations, device tensors for device tensors.  deterministic=True: the first
         argmax of the logits or the Gaussian means (not clipped); False: a draw of the evaluation generator, which leaves the
         training sampling counter and the numpy / torch streams alone.  The default network runs dppo_rnn_forward and the greedy /
         sampling kernels; a custom network_cls its get_logits_values_and_hx / get_means_log_stds_values_and_hx under inference_mode."""
-        dev, Hg = self.device, self.cfg.gru_hidden_dim
+        dev, S = self.device, self.state_dim
         obs = as_device_obs(observations, self.obs_dim, dev)
         n = obs.shape[0]
-        h = torch.zeros(1, n, Hg, device=dev) if hx is None else as_device_obs(hx, Hg, dev).reshape(1, n, Hg)
+        h = torch.zeros(1, n, S, device=dev) if hx is None else as_device_obs(hx, S, dev).reshape(1, n, S)
         pd = None if dones is None else torch.as_tensor(np.asarray(dones) if not torch.is_tensor(dones) else dones).to(dev, torch.bool).reshape(1, n)
         eng, log_std = self.engine, None
         if getattr(eng, "fused", False):
@@ -662,7 +768,7 @@ class RecurrentPPO(PolicyEvaluation):
         head = head.reshape(n, -1).contiguous()
         key, counter = self._eval_draw() if not deterministic else (0, 0)
         actions = select_actions(self.ctx, head, log_std, deterministic, key, counter, greedy_kernel=getattr(eng, "fused", False))
-        new_hx = new_hx.reshape(1, n, Hg).clone()
+        new_hx = new_hx.reshape(1, n, S).clone()
         if torch.is_tensor(observations):
             return actions, new_hx
         return actions.cpu().numpy(), new_hx.cpu().numpy()
@@ -692,7 +798,7 @@ class RecurrentPPO(PolicyEvaluation):
             seed = cfg.seed + self._dist.rank * cfg.num_envs
         self.current_observations, _ = self.envs.reset(seed=seed)
         self.prev_dones = np.zeros(cfg.num_envs, dtype=bool)
-        self.current_hx = torch.zeros(1, cfg.num_envs, cfg.gru_hidden_dim, device=self.device)
+        self.current_hx = torch.zeros(1, cfg.num_envs, self.state_dim, device=self.device)
         if self._epstats is not None:                                  # fresh environments: running returns / lengths restart
             self._flush_episode_stats()
             self._epstats["ep_return"].zero_()
@@ -718,6 +824,7 @@ class RecurrentContinuousPPO(RecurrentPPO):
     (continuous_ppo.py:50-121: mean head, state-independent log-std, actions neither squashed nor clipped)."""
     _continuous = True
     _default_network = RecurrentContinuousActorCriticNetwork
+    _lstm_network = RecurrentContinuousLSTMActorCriticNetwork
 
     def __init__(self, env_fn: Callable[[], Any], cfg: RecurrentContinuousPPOConfig = RecurrentContinuousPPOConfig(),
                  network_cls: Any = RecurrentContinuousActorCriticNetwork, *, process_group=None, dp: bool = False) -> None:

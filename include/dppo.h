@@ -306,15 +306,22 @@ int64_t dppo_ppo_loss_workspace_bytes(int64_t M, int A);
 /* Default RecurrentActorCriticNetwork (recurrent_ppo.py:94-125): base Linear(D,H)+Tanh -> GRU(H,Hg) -> actor head
  * Linear(Hg,H)+Tanh+Linear(H,A) and critic head Linear(Hg,H)+Tanh+Linear(H,1).
  * continuous = 1: RecurrentContinuousActorCriticNetwork (RecurrentContinuousPPO), the same trunk with a Gaussian policy -- the actor
- * head (actor_mean_head) outputs the action means and a state-independent log-std vector actor_log_std [A] is a parameter. */
+ * head (actor_mean_head) outputs the action means and a state-independent log-std vector actor_log_std [A] is a parameter.
+ * cell = 1: the same networks with an LSTM(H,Hg) core (RecurrentLSTMActorCriticNetwork / RecurrentContinuousLSTMActorCriticNetwork):
+ * nn.LSTM's weight_ih_l0 [4Hg,H], weight_hh_l0 [4Hg,Hg], bias_ih_l0, bias_hh_l0 (gate order i,f,g,o), c' = f c + i g, h' = o tanh(c'),
+ * h and c both zeroed where prev_dones is set.  The recurrent state is packed: hx0 / hx_out are [N,2Hg], h in [:, :Hg] and c in
+ * [:, Hg:].  Widths: Hg a multiple of 4 with 8 <= Hg <= 256 (8 / 16 / 32 on warp scans, other multiples of 4 up to 96 on tiled
+ * scans, 100-256 on thread-block-cluster scans); both calls below refuse any other width before launching. */
 typedef struct dppo_rnn_desc {
     int32_t obs_dim;      /* D */
     int32_t hidden;       /* H  = cfg.network_hidden_dim (<= 512) */
     int32_t gru_hidden;   /* Hg = cfg.gru_hidden_dim (<= 512; 129-512 run on thread-block-cluster scans) */
     int32_t act_dim;      /* A  = Discrete.n, or the action dimensions of a Box (<= DPPO_MAX_ACT) */
     int32_t continuous;   /* 0: categorical policy (logits), 1: Gaussian policy (means + actor_log_std) */
+    int32_t cell;         /* 0: GRU (default), 1: LSTM */
 } dppo_rnn_desc;
-/* Offsets (floats, multiples of 4) in the flat parameter / gradient / Adam buffers; the GRU tensors are nn.GRU's
+/* Offsets (floats, multiples of 4) in the flat parameter / gradient / Adam buffers (cell = 1: wih, whh, bih, bhh sized 4Hg, the
+ * lstm.* tensors of nn.LSTM; the same offsets structure otherwise); the GRU tensors are nn.GRU's
  * weight_ih_l0 [3Hg,H], weight_hh_l0 [3Hg,Hg], bias_ih_l0, bias_hh_l0 (gate order r,z,n); w3/b3 = actor_head.0 | critic_head.0
  * (continuous: actor_mean_head.0 | critic_head.0), wa/ba = actor_head.2 (continuous: actor_mean_head.2).  log_std = actor_log_std [A],
  * placed after bc when continuous, else -1; every other offset is the same for both kinds. */
@@ -330,9 +337,10 @@ typedef struct dppo_rnn_layout {
 int dppo_rnn_layout_compute(const dppo_rnn_desc* desc, dppo_rnn_layout* out);
 int64_t dppo_rnn_workspace_bytes(const dppo_rnn_desc* desc, int T, int N, int64_t M, int training);
 /* get_logits_values_and_hx / get_values (recurrent_ppo.py:127-149) over a [T,N] sequence: obs [T,N,D]; prev_dones uint8 [T,N]
- * (NULL: no resets) zeroes the hidden state of an environment BEFORE step t (recurrent_ppo.py:84); hx0 [N,Hg] (NULL: zeros).
+ * (NULL: no resets) zeroes the hidden state of an environment BEFORE step t (recurrent_ppo.py:84); hx0 [N,Hg] (NULL: zeros;
+ * cell = 1: [N,2Hg], h | c).
  * heads bit0: logits [T*N,A] (continuous: the action means [T*N,A]; the log-std is params + layout.log_std); bit1: values [T*N];
- * hx_out (optional) [N,Hg] final hidden state. */
+ * hx_out (optional) [N,Hg] final hidden state (cell = 1: [N,2Hg], h | c). */
 int dppo_rnn_forward(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* params, const float* obs,
                      const unsigned char* prev_dones, const float* hx0, int T, int N, int heads, float* logits,
                      float* values, float* hx_out, void* ws, int64_t ws_bytes, void* stream);
@@ -343,7 +351,8 @@ int dppo_rnn_forward(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* para
  * actions: int32 [T*N] (discrete) or f32 [T*N, A] (continuous: the Gaussian loss of continuous_ppo.py, with the gradient of
  * actor_log_std at layout.log_std); old_log_probs / adv / returns f32 [T*N]; flat gradient -> grads, (policy, value, entropy,
  * total) -> losses[0..3].
- * Both calls refuse, before launching anything, hidden > 512, gru_hidden > 512, act_dim > DPPO_MAX_ACT; dppo_rnn_grad_minibatch
+ * Both calls refuse, before launching anything, hidden > 512, gru_hidden > 512, act_dim > DPPO_MAX_ACT, an LSTM width outside the
+ * rule above (cell = 1: a multiple of 4 from 8 to 256); dppo_rnn_grad_minibatch
  * also refuses the (hidden, act_dim) pairs whose per-warp head-gradient accumulators exceed the head kernel's 200 KB of shared
  * memory (9 (act_dim + 1) hidden floats: e.g. act_dim <= 10 at hidden 512, <= 32 up to hidden 172). */
 int dppo_rnn_grad_minibatch(dppo_ctx* ctx, const dppo_rnn_desc* desc, const float* params, float* grads, const float* obs,
