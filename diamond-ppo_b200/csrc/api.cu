@@ -210,6 +210,15 @@ TrainWs carve_train(const dppo_mlp_desc* d, int64_t M, int sm_count, char* base,
     return w;
 }
 
+// Operand format of the forward launches whose A operand is the output of a tanh epilogue (layers 2 and 3): |A| <= 1 + 3e-7 < 4,
+// so A * 2^14 cannot leave fp16's range and the fp16-pair GEMM keeps the 3xTF32 accuracy at twice the tensor rate (gemm_tc.cuh).
+// Layer 1 (raw observations), the dgrad launches (unbounded loss gradients) and the weight gradients stay on 3xTF32.
+// tc_debug bit 2048 forces TF32 here (timing builds only: A/B runs on one box).
+int tanh_input_fmt(const dppo_ctx* ctx)
+{
+    return DPPO_DBG(ctx->tc_debug, 2048) ? DPPO_TC_FMT_TF32 : DPPO_TC_FMT_F16;
+}
+
 int current_sm_count()
 {
     int dev = 0, sms = 148;
@@ -291,17 +300,19 @@ extern "C" int dppo_mlp_forward(dppo_ctx* ctx, const dppo_mlp_desc* d, const flo
     const int64_t first = rows < chunk ? rows : chunk;
     const bool tc1 = tc_on && dppo_tc3_gemm_supported(first, H, D), tc2 = tc_on && dppo_tc3_gemm_supported(first, H, H),
                tc3 = tc_on && dppo_tc3_gemm_supported(first, n3, H);
+    const int hfmt = tanh_input_fmt(ctx);              // layers 2 and 3: A = h1, h2 are tanh outputs
     {
         PrepJobs jobs;
         jobs.n = 0;
         jobs.gather = GatherJob{nullptr, nullptr, nullptr, 0, 0};
-        auto job = [&](bool on, const float* W, int rows_w, int cols_w, unsigned char* im) {
+        auto job = [&](bool on, const float* W, int rows_w, int cols_w, int fmt, unsigned char* im) {
             if (on) { jobs.job[jobs.n].W = W; jobs.job[jobs.n].rows_w = rows_w; jobs.job[jobs.n].cols_w = cols_w;
-                      jobs.job[jobs.n].transpose = 0; jobs.job[jobs.n].n_tile = 0; jobs.job[jobs.n].img = im; ++jobs.n; }
+                      jobs.job[jobs.n].transpose = 0; jobs.job[jobs.n].n_tile = 0; jobs.job[jobs.n].f16 = fmt == DPPO_TC_FMT_F16;
+                      jobs.job[jobs.n].img = im; ++jobs.n; }
         };
-        job(tc1, params + L.w1, H, D, img.w1f);
-        job(tc2, params + L.w2, H, H, img.w2f);
-        job(tc3, params + L.w3 + w3off, n3, H, img.w3f);
+        job(tc1, params + L.w1, H, D, DPPO_TC_FMT_TF32, img.w1f);
+        job(tc2, params + L.w2, H, H, hfmt, img.w2f);
+        job(tc3, params + L.w3 + w3off, n3, H, hfmt, img.w3f);
         if (dppo_tc_prep_weights_multi(ctx, jobs, st)) return 1;
     }
     for (int64_t r0 = 0; r0 < rows; r0 += chunk) {
@@ -316,11 +327,11 @@ extern "C" int dppo_mlp_forward(dppo_ctx* ctx, const dppo_mlp_desc* d, const flo
             if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, x, D, img.w1f, params + L.b1, nullptr, 0, h1, H, nullptr, n, H, D, hint, st)) return 1;
         } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, x, D, rowsel, params + L.w1, D, params + L.b1, h1, H, n, H, D, st)) return 1;
         if (tc2 && dppo_tc3_gemm_supported(n, H, H)) {
-            if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, h1, H, img.w2f, params + L.b2, nullptr, 0, h2, H, nullptr, n, H, H, (sweep & 1) | hint, st)) return 1;
+            if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, h1, H, img.w2f, params + L.b2, nullptr, 0, h2, H, nullptr, n, H, H, (sweep & 1) | hint, st, hfmt)) return 1;
         } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, h1, H, nullptr, params + L.w2, H, params + L.b2, h2, H, n, H, H, st)) return 1;
         // first head layers: both (one [2H,H] product) or only the requested half
         if (tc3 && dppo_tc3_gemm_supported(n, n3, H)) {
-            if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, h2, H, img.w3f, params + L.b3 + b3off, nullptr, 0, h3, n3, nullptr, n, n3, H, hint, st)) return 1;
+            if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, h2, H, img.w3f, params + L.b3 + b3off, nullptr, 0, h3, n3, nullptr, n, n3, H, hint, st, hfmt)) return 1;
         } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, h2, H, nullptr, params + L.w3 + w3off, H, params + L.b3 + b3off, h3, n3, n, n3, H, st)) return 1;
         const float* ha = actor ? h3 : nullptr;
         const float* hc = critic ? (actor ? h3 + H : h3) : nullptr;
@@ -362,6 +373,7 @@ static int mlp_grad_minibatch_impl(dppo_ctx* ctx, const char* what, bool gemm_he
     const bool g1 = tc_on && dppo_tc3_gemm_supported(M, H, D), g2 = tc_on && dppo_tc3_gemm_supported(M, H, H),
                g3 = tc_on && dppo_tc3_gemm_supported(M, 2 * H, H), gb3 = tc_on && dppo_tc3_gemm_supported(M, H, 2 * H), gb2 = g2;
     const bool wg3 = tc_on && w.t3 > 0, wg2 = tc_on && w.t2 > 0, wg1 = tc_on && w.t1 > 0;
+    const int hfmt = tanh_input_fmt(ctx);              // forward layers 2 and 3: A = h1, h2 are tanh outputs
     // Row sweeps along the chain (dppo_tc3_gemm): L1 up, L2 down, L3 up, head kernel down, dgrad3 up, dgrad2 down -- every launch
     // starts with the rows its predecessor wrote last (still in the L2).
     const int sweep = ctx->row_sweep;
@@ -377,15 +389,16 @@ static int mlp_grad_minibatch_impl(dppo_ctx* ctx, const char* what, bool gemm_he
         PrepJobs jobs;
         jobs.n = 0;
         jobs.gather = GatherJob{nullptr, nullptr, nullptr, 0, 0};
-        auto job = [&](bool on, const float* W, int rows_w, int cols_w, int transpose, unsigned char* im) {
+        auto job = [&](bool on, const float* W, int rows_w, int cols_w, int transpose, int fmt, unsigned char* im) {
             if (on) { jobs.job[jobs.n].W = W; jobs.job[jobs.n].rows_w = rows_w; jobs.job[jobs.n].cols_w = cols_w;
-                      jobs.job[jobs.n].transpose = transpose; jobs.job[jobs.n].n_tile = 0; jobs.job[jobs.n].img = im; ++jobs.n; }
+                      jobs.job[jobs.n].transpose = transpose; jobs.job[jobs.n].n_tile = 0; jobs.job[jobs.n].f16 = fmt == DPPO_TC_FMT_F16;
+                      jobs.job[jobs.n].img = im; ++jobs.n; }
         };
-        job(g1, params + L.w1, H, D, 0, img.w1f);
-        job(g2, params + L.w2, H, H, 0, img.w2f);
-        job(g3, params + L.w3, 2 * H, H, 0, img.w3f);
-        job(gb3, params + L.w3, 2 * H, H, 1, img.w3b);
-        job(gb2, params + L.w2, H, H, 1, img.w2b);
+        job(g1, params + L.w1, H, D, 0, DPPO_TC_FMT_TF32, img.w1f);
+        job(g2, params + L.w2, H, H, 0, hfmt, img.w2f);
+        job(g3, params + L.w3, 2 * H, H, 0, hfmt, img.w3f);
+        job(gb3, params + L.w3, 2 * H, H, 1, DPPO_TC_FMT_TF32, img.w3b);
+        job(gb2, params + L.w2, H, H, 1, DPPO_TC_FMT_TF32, img.w2b);
         if (gather_pending && D % 4 == 0 && (reinterpret_cast<uintptr_t>(obs) & 15u) == 0 && (reinterpret_cast<uintptr_t>(w.xg) & 15u) == 0) {
             jobs.gather = GatherJob{reinterpret_cast<const float4*>(obs), idx, reinterpret_cast<float4*>(w.xg), M, D / 4};
             gather_pending = false;
@@ -399,10 +412,10 @@ static int mlp_grad_minibatch_impl(dppo_ctx* ctx, const char* what, bool gemm_he
         if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, x1, D, img.w1f, params + L.b1, nullptr, 0, w.h1, H, nullptr, M, H, D, hint, st)) return 1;
     } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, x1, D, x1_idx, params + L.w1, D, params + L.b1, w.h1, H, M, H, D, st)) return 1;
     if (g2) {
-        if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, img.w2f, params + L.b2, nullptr, 0, w.h2, H, nullptr, M, H, H, (sweep & 1) | hint, st)) return 1;
+        if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, img.w2f, params + L.b2, nullptr, 0, w.h2, H, nullptr, M, H, H, (sweep & 1) | hint, st, hfmt)) return 1;
     } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, nullptr, params + L.w2, H, params + L.b2, w.h2, H, M, H, H, st)) return 1;
     if (g3) {
-        if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, img.w3f, params + L.b3, nullptr, 0, w.h3, 2 * H, nullptr, M, 2 * H, H, hint, st)) return 1;
+        if (dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, img.w3f, params + L.b3, nullptr, 0, w.h3, 2 * H, nullptr, M, 2 * H, H, hint, st, hfmt)) return 1;
     } else if (dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, nullptr, params + L.w3, H, params + L.b3, w.h3, 2 * H, M, 2 * H, H, st)) return 1;
 
     // heads + loss (ppo.py:264-280) + backward into the first head layers
@@ -614,26 +627,28 @@ extern "C" int dppo_mlp_next_values(dppo_ctx* ctx, const dppo_mlp_desc* d, const
     WImages img = carve_images(d, img_base);
     const bool tc_on = ctx->use_tensor_cores != 0;
     const bool tc1 = tc_on && dppo_tc3_gemm_supported(B, H, D), tc2 = tc_on && dppo_tc3_gemm_supported(B, H, H);
+    const int hfmt = tanh_input_fmt(ctx);              // layer 2 and the critic layer 3: A = h1, h2 are tanh outputs
     {
         PrepJobs jobs;
         jobs.n = 0;
         jobs.gather = GatherJob{nullptr, nullptr, nullptr, 0, 0};
-        auto job = [&](bool on, const float* W, int rows_w, int cols_w, unsigned char* im) {
+        auto job = [&](bool on, const float* W, int rows_w, int cols_w, int fmt, unsigned char* im) {
             if (on) { jobs.job[jobs.n].W = W; jobs.job[jobs.n].rows_w = rows_w; jobs.job[jobs.n].cols_w = cols_w;
-                      jobs.job[jobs.n].transpose = 0; jobs.job[jobs.n].n_tile = 0; jobs.job[jobs.n].img = im; ++jobs.n; }
+                      jobs.job[jobs.n].transpose = 0; jobs.job[jobs.n].n_tile = 0; jobs.job[jobs.n].f16 = fmt == DPPO_TC_FMT_F16;
+                      jobs.job[jobs.n].img = im; ++jobs.n; }
         };
-        job(tc1, params + L.w1, H, D, img.w1f);
-        job(tc2, params + L.w2, H, H, img.w2f);
-        job(tc2, params + L.w3 + (int64_t)H * H, H, H, img.w3f);          // critic_head.0
+        job(tc1, params + L.w1, H, D, DPPO_TC_FMT_TF32, img.w1f);
+        job(tc2, params + L.w2, H, H, hfmt, img.w2f);
+        job(tc2, params + L.w3 + (int64_t)H * H, H, H, hfmt, img.w3f);          // critic_head.0
         if (dppo_tc_prep_weights_multi(ctx, jobs, st)) return 1;
     }
     ctx->rows_dev = w.count;
     int rc = dppo_gather_rows_f32(ctx, next_obs, w.idx, w.xg, B, D, stream);
     if (!rc) rc = tc1 ? dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.xg, D, img.w1f, params + L.b1, nullptr, 0, w.h1, H, nullptr, B, H, D, 0, st)
                       : dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.xg, D, nullptr, params + L.w1, D, params + L.b1, w.h1, H, B, H, D, st);
-    if (!rc) rc = tc2 ? dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, img.w2f, params + L.b2, nullptr, 0, w.h2, H, nullptr, B, H, H, 0, st)
+    if (!rc) rc = tc2 ? dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, img.w2f, params + L.b2, nullptr, 0, w.h2, H, nullptr, B, H, H, 0, st, hfmt)
                       : dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h1, H, nullptr, params + L.w2, H, params + L.b2, w.h2, H, B, H, H, st);
-    if (!rc) rc = tc2 ? dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, img.w3f, params + L.b3 + H, nullptr, 0, w.h3, H, nullptr, B, H, H, 0, st)
+    if (!rc) rc = tc2 ? dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, img.w3f, params + L.b3 + H, nullptr, 0, w.h3, H, nullptr, B, H, H, 0, st, hfmt)
                       : dppo_gemm_nt(ctx, DPPO_EPI_BIAS_TANH, w.h2, H, nullptr, params + L.w3 + (int64_t)H * H, H, params + L.b3 + H, w.h3, H, B, H, H, st);
     if (!rc) rc = launch_heads_forward(ctx, nullptr, w.h3, H, params + L.wa, params + L.ba, params + L.wc, params + L.bc, nullptr, w.tmp, B, H,
                                        d->act_dim, 0, st);
@@ -668,6 +683,29 @@ extern "C" int dppo_tc_linear_f32(dppo_ctx* ctx, int epi, const float* A, int64_
     // prepared != 0: the images an earlier call with the same weights left in ws are re-used (kernel-only timing)
     if (!prepared && dppo_tc_prep_weights(ctx, W, rows_w, cols_w, transpose, img, st)) return 1;
     return dppo_tc3_gemm(ctx, epi, A, K, img, bias, Hact, N, C, N, colsum, M, N, K, 0, st);
+}
+
+extern "C" int dppo_tc_linear_forward(dppo_ctx* ctx, int fmt, const float* A, int64_t M, int K, const float* W, int N, const float* bias,
+                                      float* C, const int* rows_dev, void* ws, int64_t ws_bytes, int prepared, void* stream)
+{
+    if (!ctx) return 1;
+    if (!A || !W || !bias || !C || !ws) DPPO_FAIL(ctx, "tc_linear_forward: null argument");
+    if (fmt != DPPO_TC_FMT_TF32 && fmt != DPPO_TC_FMT_F16) DPPO_FAIL(ctx, "tc_linear_forward: unknown operand format %d", fmt);
+    if (!dppo_tc3_gemm_supported(M, N, K)) DPPO_FAIL(ctx, "tc_linear_forward: unsupported shape M=%lld N=%d K=%d", (long long)M, N, K);
+    unsigned char* img = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(ws) + 1023) & ~(uintptr_t)1023);
+    if ((img - (unsigned char*)ws) + dppo_tc_image_bytes(N, K) > ws_bytes) DPPO_FAIL(ctx, "tc_linear_forward: workspace too small");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!prepared) {
+        PrepJobs jobs;
+        jobs.n = 1;
+        jobs.job[0] = PrepJob{W, N, K, 0, 0, fmt == DPPO_TC_FMT_F16, img};
+        jobs.gather = GatherJob{nullptr, nullptr, nullptr, 0, 0};
+        if (dppo_tc_prep_weights_multi(ctx, jobs, st)) return 1;
+    }
+    ctx->rows_dev = rows_dev;
+    const int rc = dppo_tc3_gemm(ctx, DPPO_EPI_BIAS_TANH, A, K, img, bias, nullptr, 0, C, N, nullptr, M, N, K, 0, st, fmt);
+    ctx->rows_dev = nullptr;
+    return rc;
 }
 
 extern "C" int64_t dppo_tc_wgrad_workspace_bytes(dppo_ctx* ctx, int64_t M, int N1, int N2)

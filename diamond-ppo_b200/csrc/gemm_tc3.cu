@@ -14,6 +14,12 @@
 //   warps 2-5   split    : hi/lo split of this CTA's activation chunk, then one arrival per warp on the LEADER's barrier
 //   warps 6-13  epilogue : tcgen05.ld of this CTA's 128 x 256 accumulator half, layer epilogue, staged TMA store
 // Accumulators are double-buffered in TMEM (2 x 256 columns), so the epilogue of tile i overlaps the MMAs of tile i+1.
+//
+// FMT = DPPO_TC_FMT_F16 (forward launches whose A is a tanh output, gemm_tc.cuh): the split warps write fp16 hi/lo images of
+// A * 2^14 beside the raw fp32 chunk, the weight images are fp16 pairs of W * s_n, and the MMA warp issues three kind::f16
+// MMAs (K = 16) per chunk -- the tensor pipe's 16-bit rate, twice the FLOPs per clock of kind::tf32.  The epilogue scales the
+// accumulator back by 2^-14 / s_n before the bias.  A stage is 24 KB ([A raw 8 | A hi 4 | A lo 4 | B hi 4 | B lo 4]) and holds
+// half the MMA time of a TF32 stage, so the ring is eight stages deep.
 #include <cuda.h>
 
 #include "tc_common.cuh"
@@ -29,14 +35,20 @@ constexpr int SPLIT_THREADS = N_SPLIT * 32;
 constexpr int KC = 16;                     // k per chunk (one SWIZZLE_64B atom width)
 constexpr int BM = 128;                    // rows per CTA (the pair computes 256)
 constexpr int A_IMG = BM * KC * 4;         // 8 KB: one image (hi or lo) of this CTA's activation chunk
-constexpr int MAX_STAGES = 6;
+constexpr int MAX_STAGES = 8;
 // Ring depth: six 32 KB stages for the forward GEMM; the dgrad variant gives one stage to the epilogue warps, which receive their
 // 32 x 32 tiles of the layer's activations (tanh' factors) by TMA instead of thread-per-row global loads (32 different 128-byte
 // lines per load instruction: 1.27x the algorithmic DRAM traffic and 12 us per launch, profiles/r1f_kernels.csv).
-template <int EPI> struct RingDepth { static constexpr int v = EPI == DPPO_EPI_TANH_BWD ? 5 : 6; };
+template <int EPI, int FMT> struct RingDepth { static constexpr int v = FMT == DPPO_TC_FMT_F16 ? 8 : EPI == DPPO_EPI_TANH_BWD ? 5 : 6; };
+template <int FMT> struct Fmt {
+    static constexpr bool f16 = FMT == DPPO_TC_FMT_F16;
+    static constexpr int b_row = f16 ? KC * 2 : KC * 4;                // bytes of one weight row of a chunk image
+    static constexpr int a_hi = f16 ? A_IMG : 0;                       // stage offsets of the A images (TF32: the raw chunk is hi)
+    static constexpr int a_lo = f16 ? A_IMG + A_IMG / 2 : A_IMG;
+};
 constexpr int STG_BLK = 32 * 128;          // one 32-row x 32-column fp32 staging block (SWIZZLE_128B layout)
 
-template <int EPI>
+template <int EPI, int FMT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmH,
                 const unsigned char* __restrict__ Wimg, const float* __restrict__ bias, float* __restrict__ colsum, int64_t M,
@@ -49,7 +61,8 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         if (tail_halves == 1) tail_halves = 0;           // the tail split was planned for the host's row count
     }
     extern __shared__ unsigned char dyn_raw[];
-    constexpr int STAGES = RingDepth<EPI>::v;
+    constexpr int STAGES = RingDepth<EPI, FMT>::v;
+    using F = Fmt<FMT>;
     __shared__ __align__(8) uint64_t full[MAX_STAGES], ready[MAX_STAGES], empty[MAX_STAGES], tfull[2], tempty[2], hbar[N_EPI];
     __shared__ uint32_t s_tmem;
 
@@ -61,9 +74,9 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     const bool no_pf = (rev & 4) != 0;                   // no L2 prefetch of the next tile's activations (the default, see dppo_tc3_gemm)
     rev &= 1;
     const int half_n = n_tile / 2;                       // weight rows held by each CTA
-    const int b_half = half_n * KC * 4;                  // bytes of one image (hi or lo) of this CTA's weight rows
-    const int b_img = n_tile * KC * 4;                   // bytes of one full image in the weight-image buffer
-    const int stage_bytes = 2 * A_IMG + 2 * b_half;      // [A_hi | A_lo | B_hi(half) | B_lo(half)]
+    const int b_half = half_n * F::b_row;                // bytes of one image (hi or lo) of this CTA's weight rows
+    const int b_img = n_tile * F::b_row;                 // bytes of one full image in the weight-image buffer
+    const int stage_bytes = 2 * A_IMG + 2 * b_half;      // [A_hi | A_lo | B_hi(half) | B_lo(half)], f16: [A | A_hi | A_lo | ...]
     const int n_tiles = N / n_tile;
     const int total = pair_tiles * n_tiles;
     const int chunks = K / KC;
@@ -113,9 +126,9 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 const int m_pair = tile / n_tiles, n_blk = tile - m_pair * n_tiles;
                 const int m0 = m_pair * 2 * BM + (int)rank * BM;
                 const int n_eff = half < 0 ? n_tile : n_tile / 2;                  // columns of this tile
-                const int hb = (n_eff / 2) * KC * 4;                               // bytes of this CTA's rows of one image
+                const int hb = (n_eff / 2) * F::b_row;                             // bytes of this CTA's rows of one image
                 const int row_off = (half < 0 ? 0 : half * (n_tile / 2)) + (int)rank * (n_eff / 2);
-                const unsigned char* wsrc = Wimg + (int64_t)n_blk * chunks * 2 * b_img + (int64_t)row_off * KC * 4;
+                const unsigned char* wsrc = Wimg + (int64_t)n_blk * chunks * 2 * b_img + (int64_t)row_off * F::b_row;
                 int next_m = -1;
                 if (i + 1 < n_my) { int nt, nh; tile_of(i + 1, nt, nh); next_m = nt / n_tiles; }
                 for (int c = 0; c < chunks; ++c) {
@@ -142,7 +155,8 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         __syncwarp();
     } else if (warp == W_MMA) {
         if (rank == 0 && lane == 0) {
-            const uint32_t idesc_full = idesc_tf32(2 * BM, n_tile, 0, 0), idesc_half = idesc_tf32(2 * BM, n_tile / 2, 0, 0);
+            const uint32_t idesc_full = F::f16 ? idesc_f16(2 * BM, n_tile) : idesc_tf32(2 * BM, n_tile, 0, 0);
+            const uint32_t idesc_half = F::f16 ? idesc_f16(2 * BM, n_tile / 2) : idesc_tf32(2 * BM, n_tile / 2, 0, 0);
             int s = 0;
             uint32_t ph = 0;
             for (uint32_t it = 0; it < (uint32_t)n_my; ++it) {
@@ -156,8 +170,17 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 for (int c = 0; c < chunks; ++c) {
                     mbar_wait(&ready[s], ph);                           // both CTAs: chunk landed and split
                     fence_after();
-                    const uint32_t a_hi = smem_u32(dyn + s * stage_bytes), a_lo = a_hi + A_IMG;
-                    const uint32_t b_hi = a_hi + 2 * A_IMG, b_lo = b_hi + (uint32_t)b_half;
+                    const uint32_t st0 = smem_u32(dyn + s * stage_bytes), a_hi = st0 + F::a_hi, a_lo = st0 + F::a_lo;
+                    const uint32_t b_hi = st0 + 2 * A_IMG, b_lo = b_hi + (uint32_t)b_half;
+                    if (F::f16) {                                       // one 16-wide k-step: the whole SWIZZLE_32B row
+                        if (!DPPO_DBG(dbg, 4)) {
+                            umma_f16_2cta(d, desc_k_sw32(a_hi), desc_k_sw32(b_lo), idesc, c != 0);
+                            umma_f16_2cta(d, desc_k_sw32(a_lo), desc_k_sw32(b_hi), idesc, 1u);
+                            umma_f16_2cta(d, desc_k_sw32(a_hi), desc_k_sw32(b_hi), idesc, 1u);
+                        } else {
+                            umma_f16_2cta(d, desc_k_sw32(a_hi), desc_k_sw32(b_hi), idesc, c != 0);
+                        }
+                    } else {
 #pragma unroll
                     for (int ks = 0; ks < KC / 8; ++ks) {
                         const uint32_t ko = ks * 32;                    // 8 tf32 = 32 bytes along K inside the swizzle atom
@@ -168,6 +191,7 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                         } else {
                             umma_tf32_2cta(d, desc_k_sw64(a_hi + ko), desc_k_sw64(b_hi + ko), idesc, (c | ks) != 0);
                         }
+                    }
                     }
                     umma_commit_2cta(&empty[s], 3);                     // frees the stage in both CTAs
                     if (++s == STAGES) { s = 0; ph ^= 1; }
@@ -185,6 +209,32 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         for (int i = 0; i < n_my; ++i) {
             for (int c = 0; c < chunks; ++c) {
                 mbar_wait(&full[s], ph);
+                if (F::f16) {
+                    // thread -> (row, 8-wide k half) pairs: two 16-byte segments of the raw SWIZZLE_64B row in, one 16-byte segment
+                    // of each SWIZZLE_32B fp16 image out (both conflict-free per quarter warp)
+                    const uint32_t raw = smem_u32(dyn + s * stage_bytes);
+                    float4 x[4];
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        const int p = ct + j * SPLIT_THREADS, row = p >> 1, c2 = (p & 1) * 2, sw = (row >> 1) & 3;
+                        x[2 * j] = lds128(raw + row * 64 + ((c2 ^ sw) << 4));
+                        x[2 * j + 1] = lds128(raw + row * 64 + (((c2 + 1) ^ sw) << 4));
+                    }
+#pragma unroll
+                    for (int j = 0; j < 2; ++j) {
+                        const int p = ct + j * SPLIT_THREADS, row = p >> 1;
+                        const uint32_t o = (uint32_t)(row * 32 + ((((p & 1) ^ (row >> 2)) & 1) << 4));
+                        uint4 h, l;
+                        split_f16x8(x[2 * j], x[2 * j + 1], (float)(1 << DPPO_F16_A_EXP), h, l);
+                        sts128u(raw + F::a_hi + o, h);
+                        sts128u(raw + F::a_lo + o, l);
+                    }
+                    fence_proxy_async();
+                    __syncwarp();
+                    if (lane == 0) mbar_arrive_cluster(mapa(smem_u32(&ready[s]), 0));
+                    if (++s == STAGES) { s = 0; ph ^= 1; }
+                    continue;
+                }
                 const uint32_t hi = smem_u32(dyn + s * stage_bytes) + ct * 16;
                 float4 x[PER];
 #pragma unroll
@@ -241,9 +291,15 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 uint32_t r[32];
                 tmem_ld32_issue(tmem + set * 256 + ((uint32_t)(q * 32) << 16) + (uint32_t)(col0 + k * 32), r);
                 float4 aux[8];                                          // bias (forward) or the layer's activations (dgrad)
+                float4 fac[8];                                          // f16: column factors 2^-14 / s_n
                 if (EPI == DPPO_EPI_BIAS_TANH) {
 #pragma unroll
                     for (int j = 0; j < 8; ++j) aux[j] = __ldg(reinterpret_cast<const float4*>(bias + n) + j);
+                    if (F::f16) {
+                        const float* f = reinterpret_cast<const float*>(Wimg + dppo_tc_f16_factor_offset(N, K));
+#pragma unroll
+                        for (int j = 0; j < 8; ++j) fac[j] = __ldg(reinterpret_cast<const float4*>(f + n) + j);
+                    }
                 } else {
                     mbar_wait(&hbar[ew], hph);
                     hph ^= 1u;
@@ -260,6 +316,12 @@ tc3_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                 float v[32];
 #pragma unroll
                 for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
+                if (EPI == DPPO_EPI_BIAS_TANH && F::f16) {
+#pragma unroll
+                    for (int j = 0; j < 8; ++j) {                               // exact: powers of two, no over- or underflow
+                        v[4 * j] *= fac[j].x; v[4 * j + 1] *= fac[j].y; v[4 * j + 2] *= fac[j].z; v[4 * j + 3] *= fac[j].w;
+                    }
+                }
                 if (EPI == DPPO_EPI_BIAS_TANH) {
 #pragma unroll
                     for (int j = 0; j < 8; ++j) {
@@ -389,9 +451,11 @@ bool dppo_tc3_gemm_supported(int64_t M, int N, int K)
 // without it (profiles/r4e_prefetch_ab.md) -- and the optimiser step is 1.4 % faster without (2.7 % with the weight-gradient
 // kernel's chunk prefetch off as well).
 int dppo_tc3_gemm(dppo_ctx* ctx, int epi, const float* A, int lda, const unsigned char* Wimg, const float* bias, const float* Hact,
-                  int ldh, float* C, int ldc, float* colsum, int64_t M, int N, int K, int rev, cudaStream_t st)
+                  int ldh, float* C, int ldc, float* colsum, int64_t M, int N, int K, int rev, cudaStream_t st, int fmt)
 {
     if (!dppo_tc3_gemm_supported(M, N, K)) DPPO_FAIL(ctx, "tc3_gemm: unsupported shape M=%lld N=%d K=%d", (long long)M, N, K);
+    const bool f16 = fmt == DPPO_TC_FMT_F16;
+    if (fmt != DPPO_TC_FMT_TF32 && !(f16 && epi == DPPO_EPI_BIAS_TANH)) DPPO_FAIL(ctx, "tc3_gemm: operand format %d with epilogue %d", fmt, epi);
     if (lda % 4 != 0 || ldc % 4 != 0 || !al16(A) || !al16(C) || !al16(Wimg) || (Hact && (!al16(Hact) || ldh % 4 != 0)) || (bias && !al16(bias)))
         DPPO_FAIL(ctx, "tc3_gemm: operands must be 16-byte aligned with row pitches multiple of 4 floats");
     CUtensorMap tmA, tmC, tmH;
@@ -402,8 +466,10 @@ int dppo_tc3_gemm(dppo_ctx* ctx, int epi, const float* A, int lda, const unsigne
         DPPO_FAIL(ctx, "tc3_gemm: cuTensorMapEncodeTiled(Hact) failed");
     const int n_tile = dppo_tc_n_tile(N);
     const int pair_tiles = (int)((M + 2 * BM - 1) / (2 * BM));
-    const int stages = epi == DPPO_EPI_TANH_BWD ? RingDepth<DPPO_EPI_TANH_BWD>::v : RingDepth<DPPO_EPI_BIAS_TANH>::v;
-    const size_t smem = (size_t)stages * (2 * A_IMG + n_tile * KC * 4) + (size_t)N_EPI * STG_BLK * (epi == DPPO_EPI_TANH_BWD ? 2 : 1) + 1024;
+    const int stages = epi == DPPO_EPI_TANH_BWD ? RingDepth<DPPO_EPI_TANH_BWD, DPPO_TC_FMT_TF32>::v
+                       : f16 ? RingDepth<DPPO_EPI_BIAS_TANH, DPPO_TC_FMT_F16>::v : RingDepth<DPPO_EPI_BIAS_TANH, DPPO_TC_FMT_TF32>::v;
+    const int b_row = f16 ? Fmt<DPPO_TC_FMT_F16>::b_row : Fmt<DPPO_TC_FMT_TF32>::b_row;
+    const size_t smem = (size_t)stages * (2 * A_IMG + n_tile * b_row) + (size_t)N_EPI * STG_BLK * (epi == DPPO_EPI_TANH_BWD ? 2 : 1) + 1024;
     int grid, tail_halves;
     tc3_plan(ctx, M, N, &grid, &tail_halves);
     if (!(ctx->tc_prefetch & (epi == DPPO_EPI_TANH_BWD ? 2 : 1))) rev |= 4;
@@ -411,16 +477,17 @@ int dppo_tc3_gemm(dppo_ctx* ctx, int epi, const float* A, int lda, const unsigne
         cudaMemsetAsync(colsum + (size_t)grid * N, 0, (size_t)4 * grid * N * sizeof(float), st) != cudaSuccess)
         DPPO_FAIL(ctx, "tc3_gemm: cudaMemsetAsync(colsum) failed");
     if (epi == DPPO_EPI_BIAS_TANH) {
-        cudaFuncSetAttribute(tc3_gemm_kernel<DPPO_EPI_BIAS_TANH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        const auto kern = f16 ? tc3_gemm_kernel<DPPO_EPI_BIAS_TANH, DPPO_TC_FMT_F16> : tc3_gemm_kernel<DPPO_EPI_BIAS_TANH, DPPO_TC_FMT_TF32>;
+        cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         // forward launches follow each other (and the weight-image kernel) directly: with programmatic stream serialisation the
         // launch latency and the per-CTA set-up (barriers, TMEM allocation, tensor-map fetch) of layer i + 1 hide under the tail of
         // layer i (pre-update pass 3.07 -> 2.93 ms at config S; neutral inside the training step).  The kernel touches global
         // memory only after griddepcontrol.wait.
-        dppo_launch_pdl_if(true, tc3_gemm_kernel<DPPO_EPI_BIAS_TANH>, dim3(grid), dim3(THREADS), smem, st, tmA, tmC, tmH, Wimg, bias, colsum, M,
+        dppo_launch_pdl_if(true, kern, dim3(grid), dim3(THREADS), smem, st, tmA, tmC, tmH, Wimg, bias, colsum, M,
                            N, K, n_tile, pair_tiles, tail_halves, rev, ctx->tc_debug, ctx->rows_dev);
     } else if (epi == DPPO_EPI_TANH_BWD) {
-        cudaFuncSetAttribute(tc3_gemm_kernel<DPPO_EPI_TANH_BWD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        dppo_launch_pdl(ctx, tc3_gemm_kernel<DPPO_EPI_TANH_BWD>, dim3(grid), dim3(THREADS), smem, st, tmA, tmC, tmH, Wimg, bias, colsum, M,
+        cudaFuncSetAttribute(tc3_gemm_kernel<DPPO_EPI_TANH_BWD, DPPO_TC_FMT_TF32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        dppo_launch_pdl(ctx, tc3_gemm_kernel<DPPO_EPI_TANH_BWD, DPPO_TC_FMT_TF32>, dim3(grid), dim3(THREADS), smem, st, tmA, tmC, tmH, Wimg, bias, colsum, M,
                         N, K, n_tile, pair_tiles, tail_halves, rev, ctx->tc_debug, ctx->rows_dev);
     } else {
         DPPO_FAIL(ctx, "tc3_gemm: unknown epilogue %d", epi);

@@ -2,6 +2,7 @@
 // mbarrier / TMA / bulk-copy / tcgen05 PTX wrappers and the shared-memory + instruction descriptors.
 #pragma once
 #include <cuda.h>
+#include <cuda_fp16.h>
 
 #include "common.cuh"
 
@@ -162,6 +163,16 @@ __device__ __forceinline__ void umma_tf32_2cta(uint32_t d_tmem, uint64_t a_desc,
         "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t"
         "}" ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
+// the same with 16-bit operands (kind::f16, K = 16, fp32 accumulator)
+__device__ __forceinline__ void umma_f16_2cta(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
+{
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
+        "}" ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+}
 // arrives on the mbarrier at this shared-memory offset in every CTA of `mask` once all MMAs issued so far are complete
 __device__ __forceinline__ void umma_commit_2cta(uint64_t* bar, uint16_t mask)
 {
@@ -175,6 +186,11 @@ __device__ __forceinline__ void umma_commit_2cta(uint64_t* bar, uint16_t mask)
 __device__ __forceinline__ uint64_t desc_k_sw64(uint32_t saddr)
 {
     return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)(512 >> 4) << 32) | (1ull << 46) | (4ull << 61);
+}
+// K-major SWIZZLE_32B (layout type 6): rows of 16 fp16 (32 B), 8-row atoms of 256 B; SBO = 256 B.
+__device__ __forceinline__ uint64_t desc_k_sw32(uint32_t saddr)
+{
+    return (uint64_t)((saddr & 0x3FFFFu) >> 4) | (1ull << 16) | ((uint64_t)(256 >> 4) << 32) | (1ull << 46) | (6ull << 61);
 }
 // MN-major fp32/tf32 operands have exactly one legal swizzled layout, SWIZZLE_128B_BASE32B (layout type 1; what a
 // CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B box delivers): groups of 32 fp32 along M/N (128 B rows), one row per k, 32-byte
@@ -191,6 +207,11 @@ __device__ __forceinline__ uint32_t idesc_tf32(int m, int n, int a_mn, int b_mn)
 {
     return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)b_mn << 16) | ((uint32_t)(n >> 3) << 17) |
            ((uint32_t)(m >> 4) << 24);
+}
+// kind::f16 instruction descriptor: D = f32, A = B = fp16 (format 0), both K-major
+__device__ __forceinline__ uint32_t idesc_f16(int m, int n)
+{
+    return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 __device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate)
 {
@@ -276,6 +297,30 @@ __device__ __forceinline__ float lo_of_trunc(float x)
 __device__ __forceinline__ float4 lo_of_trunc_x4(const float4& x)
 {
     return make_float4(lo_of_trunc(x.x), lo_of_trunc(x.y), lo_of_trunc(x.z), lo_of_trunc(x.w));
+}
+
+// fp16 hi/lo pair of 8 scaled values x' = x * scale (a power of two): hi = fp16_rn(x'), lo = fp16_rn(x' - hi), x' - hi exact in
+// fp32.  Each is one 16-byte row segment of a K-major fp16 image (element order = k order).
+__device__ __forceinline__ void split_f16x8(const float4& a, const float4& b, float scale, uint4& hi, uint4& lo)
+{
+    const float x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+    uint32_t h[4], l[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const float x0 = x[2 * i] * scale, x1 = x[2 * i + 1] * scale;
+        uint32_t p;
+        asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(p) : "f"(x1), "f"(x0));           // upper half <- x1, lower half <- x0
+        h[i] = p;
+        const float r0 = x0 - __half2float(__ushort_as_half((unsigned short)(p & 0xFFFFu)));
+        const float r1 = x1 - __half2float(__ushort_as_half((unsigned short)(p >> 16)));
+        asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(l[i]) : "f"(r1), "f"(r0));
+    }
+    hi = make_uint4(h[0], h[1], h[2], h[3]);
+    lo = make_uint4(l[0], l[1], l[2], l[3]);
+}
+__device__ __forceinline__ void sts128u(uint32_t saddr, const uint4& v)
+{
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(saddr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
 }
 
 }  // namespace tc

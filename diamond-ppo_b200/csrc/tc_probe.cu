@@ -18,10 +18,10 @@ __device__ __forceinline__ void umma_f16(uint32_t d_tmem, uint64_t a_desc, uint6
                      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
 }
 
-// mode bit0: CTA pairs (cta_group::2, M = 256), bit1: bf16 (K = 16) instead of tf32 (K = 8); n = MMA N
+// fmt: 0 tf32 (K = 8), 1 bf16, 2 fp16 (K = 16; kind::f16 with A/B format 1 or 0); n = MMA N
 template <int PAIR>
 __global__ void __launch_bounds__(128, 1)
-mma_probe_kernel(int bf16, int n, int iters, long long* __restrict__ out)
+mma_probe_kernel(int fmt, int n, int iters, long long* __restrict__ out)
 {
     extern __shared__ unsigned char dyn_raw[];
     __shared__ __align__(8) uint64_t done;
@@ -40,11 +40,11 @@ mma_probe_kernel(int bf16, int n, int iters, long long* __restrict__ out)
     if (tid == 0 && rank == 0) {
         const uint32_t a = smem_u32(dyn), b = a + 16 * 1024;
         uint32_t idesc = idesc_tf32(PAIR ? 256 : 128, n, 0, 0);
-        if (bf16) idesc = (idesc & ~((7u << 7) | (7u << 10))) | (1u << 7) | (1u << 10);
+        if (fmt) idesc = (idesc & ~((7u << 7) | (7u << 10))) | (fmt == 1 ? (1u << 7) | (1u << 10) : 0u);
         const uint64_t da = desc_k_sw64(a), db = desc_k_sw64(b);
         const long long t0 = clock64();
         for (int i = 0; i < iters; ++i) {
-            if (bf16) umma_f16(tmem, da, db, idesc, 1u, PAIR);
+            if (fmt) umma_f16(tmem, da, db, idesc, 1u, PAIR);
             else if (PAIR) umma_tf32_2cta(tmem, da, db, idesc, 1u);
             else umma_tf32(tmem, da, db, idesc, 1u);
         }
@@ -58,7 +58,7 @@ mma_probe_kernel(int bf16, int n, int iters, long long* __restrict__ out)
 }
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1)
-mma_probe_pair(int bf16, int n, int iters, long long* __restrict__ out)
+mma_probe_pair(int fmt, int n, int iters, long long* __restrict__ out)
 {
     extern __shared__ unsigned char dyn_raw[];
     __shared__ __align__(8) uint64_t done;
@@ -76,11 +76,11 @@ mma_probe_pair(int bf16, int n, int iters, long long* __restrict__ out)
     if (tid == 0 && cluster_ctarank() == 0) {
         const uint32_t a = smem_u32(dyn), b = a + 16 * 1024;
         uint32_t idesc = idesc_tf32(256, n, 0, 0);
-        if (bf16) idesc = (idesc & ~((7u << 7) | (7u << 10))) | (1u << 7) | (1u << 10);
+        if (fmt) idesc = (idesc & ~((7u << 7) | (7u << 10))) | (fmt == 1 ? (1u << 7) | (1u << 10) : 0u);
         const uint64_t da = desc_k_sw64(a), db = desc_k_sw64(b);
         const long long t0 = clock64();
         for (int i = 0; i < iters; ++i) {
-            if (bf16) umma_f16(tmem, da, db, idesc, 1u, 1);
+            if (fmt) umma_f16(tmem, da, db, idesc, 1u, 1);
             else umma_tf32_2cta(tmem, da, db, idesc, 1u);
         }
         umma_commit_2cta(&done, 1);
@@ -94,19 +94,19 @@ mma_probe_pair(int bf16, int n, int iters, long long* __restrict__ out)
 }  // namespace
 
 // out: int64 [grid] SM cycles for `iters` MMAs (entries of non-leader CTAs of a pair stay untouched)
-extern "C" int dppo_tc_mma_probe(dppo_ctx* ctx, int pair, int bf16, int n, int iters, long long* out, int* grid_out, void* stream)
+extern "C" int dppo_tc_mma_probe(dppo_ctx* ctx, int pair, int fmt, int n, int iters, long long* out, int* grid_out, void* stream)
 {
     if (!ctx) return 1;
-    if (n % 16 != 0 || n < 16 || n > 256 || iters < 1) DPPO_FAIL(ctx, "tc_mma_probe: bad arguments");
+    if (n % 16 != 0 || n < 16 || n > 256 || iters < 1 || fmt < 0 || fmt > 2) DPPO_FAIL(ctx, "tc_mma_probe: bad arguments");
     const int grid = ctx->sm_count / 2 * 2;
     const size_t smem = 49 * 1024 + 1024;
     cudaStream_t st = (cudaStream_t)stream;
     if (pair) {
         cudaFuncSetAttribute(mma_probe_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        mma_probe_pair<<<grid, 128, smem, st>>>(bf16, n, iters, out);
+        mma_probe_pair<<<grid, 128, smem, st>>>(fmt, n, iters, out);
     } else {
         cudaFuncSetAttribute(mma_probe_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        mma_probe_kernel<0><<<grid, 128, smem, st>>>(bf16, n, iters, out);
+        mma_probe_kernel<0><<<grid, 128, smem, st>>>(fmt, n, iters, out);
     }
     DPPO_CHECK_LAUNCH(ctx, "mma_probe_kernel");
     if (grid_out) *grid_out = grid;

@@ -7,7 +7,14 @@
 // The images are laid out in the canonical K-major SWIZZLE_64B shared-memory layout (16 fp32 of K per 64-byte row,
 // 8-row atoms of 512 B) so that a GEMM CTA fetches a k-chunk of its weight rows with one bulk async copy.
 // One launch per optimiser step rebuilds every image (and gathers the minibatch observations, ppo.py:261).
+//
+// fp16 images (PrepJob::f16, forward images of the layers whose input is a tanh output): the same three-MMA scheme on fp16
+// pairs of W' = W * s_n, hi = fp16_rn(W'), lo = fp16_rn(W' - hi) (22 significant bits).  s_n = 2^e is one power of two per
+// output row n with max |W'| in [2^14, 2^15), so that neither half leaves fp16's normal range; the image ends with the column
+// factors 2^-14 / s_n the GEMM epilogue applies (dppo_tc_f16_factor_offset).  Layout: K-major SWIZZLE_32B (16 fp16 of K per
+// 32-byte row, 8-row atoms of 256 B), [hi | lo] per N tile and 16-wide k chunk as for TF32.
 #include <cuda.h>
+#include <cuda_fp16.h>
 
 #include "common.cuh"
 #include "gemm_tc.cuh"
@@ -20,6 +27,12 @@ constexpr int KC = 16;                     // k elements per chunk (one SWIZZLE_
 __host__ __device__ __forceinline__ int sw64_offset(int row, int kk)
 {
     return (row >> 3) * 512 + (row & 7) * 64 + ((((kk >> 2) ^ ((row & 7) >> 1)) & 3) << 4) + ((kk & 3) << 2);
+}
+
+// byte offset of fp16 element (row, kk) inside a K-major SWIZZLE_32B image (rows x 16 fp16)
+__device__ __forceinline__ int sw32_offset(int row, int kk)
+{
+    return row * 32 + ((((kk >> 3) ^ (row >> 2)) & 1) << 4) + ((kk & 7) << 1);
 }
 
 __device__ __forceinline__ void split_tf32(float x, float& hi, float& lo)
@@ -89,6 +102,36 @@ __global__ void prep_weights_multi_kernel(PrepJobs jobs)
     const int K = j.transpose ? j.rows_w : j.cols_w;
     const int64_t total = (int64_t)N * K;
     const int chunks = K / KC;
+    if (j.f16) {
+        // one warp per weight row n.  The row's largest magnitude is an integer max over the magnitude bits, so Inf and NaN rank
+        // above every finite value: such a row keeps s_n = 1 and its Inf / NaN reach the products (lo = Inf - Inf is NaN).  e is
+        // clamped so that s_n and the column factor stay normal fp32 numbers (rows whose largest |w| is below 2^-98 keep
+        // 2^112 and lose relative, not absolute, accuracy).
+        const int lane = threadIdx.x & 31, warps = blockDim.x >> 5;
+        const int img_bytes = j.n_tile * KC * 2;
+        float* factor = reinterpret_cast<float*>(j.img + dppo_tc_f16_factor_offset(N, K));
+        for (int n = blockIdx.x * warps + (threadIdx.x >> 5); n < N; n += gridDim.x * warps) {
+            const float* w = j.W + (int64_t)n * K;
+            unsigned mx = 0;
+            for (int k = lane; k < K; k += 32) mx = max(mx, __float_as_uint(w[k]) & 0x7FFFFFFFu);
+            mx = __reduce_max_sync(0xffffffffu, mx);
+            int e = 0;
+            if (mx != 0 && mx < 0x7F800000u) e = min(112, 14 - ((int)(mx >> 23) - 127));
+            const float sc = __int_as_float((127 + e) << 23);
+            if (lane == 0) factor[n] = __int_as_float((127 - DPPO_F16_A_EXP - e) << 23);
+            const int tile = n / j.n_tile, row = n % j.n_tile;
+            for (int k = lane; k < K; k += 32) {
+                const float x = w[k] * sc;
+                const __half hi = __float2half_rn(x);
+                const __half lo = __float2half_rn(x - __half2float(hi));
+                unsigned char* base = j.img + ((int64_t)(tile * chunks + k / KC) * 2) * img_bytes;
+                const int off = sw32_offset(row, k % KC);
+                *reinterpret_cast<__half*>(base + off) = hi;
+                *reinterpret_cast<__half*>(base + img_bytes + off) = lo;
+            }
+        }
+        return;
+    }
     const int img_bytes = j.n_tile * KC * 4;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
         int n, k;
@@ -109,6 +152,7 @@ __global__ void prep_weights_multi_kernel(PrepJobs jobs)
 
 int dppo_tc_n_tile(int N) { return N % 256 == 0 ? 256 : 128; }
 
+// the TF32 images; the fp16 ones (N K 4 bytes + N column factors) fit the same space
 int64_t dppo_tc_image_bytes(int N, int K) { return (int64_t)N * K * 4 * 2; }
 
 int dppo_tc_prep_weights(dppo_ctx* ctx, const float* W, int rows_w, int cols_w, int transpose, unsigned char* img, cudaStream_t st)
@@ -128,6 +172,7 @@ int dppo_tc_prep_weights_multi(dppo_ctx* ctx, PrepJobs jobs, cudaStream_t st)
     if (jobs.n < 1 && !with_gather) return 0;
     int64_t most = with_gather ? jobs.gather.rows * jobs.gather.row_vec / 8 : 0;
     for (int i = 0; i < jobs.n; ++i) {
+        if (jobs.job[i].f16 && jobs.job[i].transpose) DPPO_FAIL(ctx, "prep_weights_multi: fp16 images are built for forward (untransposed) weights only");
         const int64_t t = (int64_t)jobs.job[i].rows_w * jobs.job[i].cols_w;
         jobs.job[i].n_tile = dppo_tc_n_tile(jobs.job[i].transpose ? jobs.job[i].cols_w : jobs.job[i].rows_w);
         if (t > most) most = t;

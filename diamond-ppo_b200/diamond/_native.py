@@ -70,7 +70,7 @@ EXPORTS = [
     "dppo_logprob_categorical", "dppo_logprob_gaussian", "dppo_mlp_grad_minibatch", "dppo_mlp_fused_heads_supported",
     "dppo_mlp_gemm_heads_workspace_bytes", "dppo_mlp_grad_minibatch_gemm_heads", "dppo_small_update", "dppo_small_update_supported", "dppo_clip_adam_step",
     "dppo_clip_adam_workspace_bytes", "dppo_grad_sumsq_bytes", "dppo_ppo_loss_discrete", "dppo_ppo_loss_gaussian",
-    "dppo_ppo_loss_workspace_bytes", "dppo_fma_peak_kernel", "dppo_tc_linear_f32", "dppo_tc_linear_workspace_bytes",
+    "dppo_ppo_loss_workspace_bytes", "dppo_fma_peak_kernel", "dppo_tc_linear_f32", "dppo_tc_linear_workspace_bytes", "dppo_tc_linear_forward",
     "dppo_tc_colsum_parts", "dppo_tc_wgrad_f32", "dppo_tc_wgrad_workspace_bytes", "dppo_tc_mma_probe", "dppo_dp_create", "dppo_dp_handle_bytes", "dppo_dp_handle", "dppo_dp_connect", "dppo_dp_destroy", "dppo_dp_status",
     "dppo_permutation_device", "dppo_perm_shard_filter", "dppo_dp_slot", "dppo_dp_zero_slot", "dppo_dp_workspace_bytes", "dppo_dp_allreduce_clip_adam",
     "dppo_env_reset", "dppo_env_step", "dppo_set_draw_counter_base", "dppo_episode_stats", "dppo_episode_stats_workspace_bytes",
@@ -491,6 +491,20 @@ class Context:
         self.launches += 2
         return Cm, cs
 
+    def tc_linear_forward(self, fmt, A, W, bias, rows_dev=None, out=None, ws=None, prepared=False):
+        """C = tanh(A W^T + bias) on the tensor cores in operand format fmt (0: 3xTF32, 1: fp16 pairs, needs |A| < 4;
+        dppo_tc_linear_forward).  rows_dev: optional int32 device tensor holding the row count the GEMM reads on the device."""
+        M, K = A.shape
+        N = W.shape[0]
+        Cm = torch.empty(M, N, device=A.device, dtype=torch.float32) if out is None else out
+        if ws is None:
+            ws = torch.empty(self.lib.dppo_tc_linear_workspace_bytes(C.c_int(N), C.c_int(K)), device=A.device, dtype=torch.uint8)
+        self._check(self.lib.dppo_tc_linear_forward(self.h, C.c_int(fmt), _ptr(A), C.c_int64(M), C.c_int(K), _ptr(W), C.c_int(N),
+                                                    _ptr(bias), _ptr(Cm), _ptr(rows_dev), _ptr(ws), C.c_int64(ws.numel()),
+                                                    C.c_int(int(prepared)), _stream()), "dppo_tc_linear_forward")
+        self.launches += 1 if prepared else 2
+        return Cm
+
     def tc_wgrad(self, Dm, Hm):
         """dW = Dm^T Hm on the tensor cores (dppo_tc_wgrad_f32)."""
         M, N1 = Dm.shape
@@ -503,11 +517,12 @@ class Context:
         self.launches += 2
         return dW
 
-    def mma_probe(self, pair, bf16, n, iters):
-        """SM cycles per tcgen05.mma (shared-memory operands) measured on every SM; returns (cycles tensor, iters)."""
+    def mma_probe(self, pair, fmt, n, iters):
+        """SM cycles per tcgen05.mma (shared-memory operands; fmt 0 tf32, 1 bf16, 2 fp16) measured on every SM; returns the
+        cycles per MMA of every reporting CTA."""
         out = torch.zeros(self.sm_count, dtype=torch.int64, device="cuda")
         g = C.c_int()
-        self._check(self.lib.dppo_tc_mma_probe(self.h, C.c_int(pair), C.c_int(bf16), C.c_int(n), C.c_int(iters), _ptr(out), C.byref(g),
+        self._check(self.lib.dppo_tc_mma_probe(self.h, C.c_int(pair), C.c_int(fmt), C.c_int(n), C.c_int(iters), _ptr(out), C.byref(g),
                                                _stream()), "dppo_tc_mma_probe")
         self.launches += 1
         torch.cuda.synchronize()

@@ -462,6 +462,13 @@ int dppo_tc_linear_f32(dppo_ctx* ctx, int epi, const float* A, int64_t M, int K,
                        const float* bias, const float* Hact, float* C, float* colsum, void* ws, int64_t ws_bytes,
                        int prepared, void* stream);
 int64_t dppo_tc_linear_workspace_bytes(int N, int K);
+/* C[M,N] = tanh(A[M,K] W^T + bias) (W [N,K] row-major) on the forward GEMM in operand format fmt: 0 is 3xTF32 (as
+ * dppo_tc_linear_f32 with epi 1), 1 is three fp16 MMAs per k-step on hi/lo pairs of A * 2^14 and of W * s_n, with one power of
+ * two s_n per weight row (twice the tensor rate of TF32 at the same accuracy).  Format 1 requires |A| < 4; the MLP entry points
+ * use it for the layers whose input is a tanh output.  rows_dev != NULL: the GEMM reads its row count from that device int
+ * (clipped to [0, M]; 256-row tiles past it are not written).  ws and prepared as for dppo_tc_linear_f32 (ws holds either format). */
+int dppo_tc_linear_forward(dppo_ctx* ctx, int fmt, const float* A, int64_t M, int K, const float* W, int N, const float* bias,
+                           float* C, const int* rows_dev, void* ws, int64_t ws_bytes, int prepared, void* stream);
 int dppo_tc_colsum_parts(dppo_ctx* ctx, int64_t M, int N);
 /* dW[N1,N2] = sum_m D[m,N1] * H[m,N2]  (weight gradient of a Linear layer, ppo.py:283): split over row
  * ranges on tcgen05, partials summed in a fixed order (bit-reproducible). */
@@ -476,10 +483,10 @@ int64_t dppo_tc_wgrad_workspace_bytes(dppo_ctx* ctx, int64_t M, int N1, int N2);
 int dppo_fma_peak_kernel(dppo_ctx* ctx, float* sink, int64_t iters, int* blocks_out, int* threads_out, void* stream);
 
 /* Issue rate of tcgen05.mma with shared-memory operands: every CTA (pair != 0: every CTA pair, cta_group::2, M = 256;
- * else M = 128) issues iters back-to-back MMAs of N = n, K = 32 bytes (tf32, or bf16 if bf16 != 0) and writes the SM
+ * else M = 128) issues iters back-to-back MMAs of N = n, K = 32 bytes (fmt 0: tf32, 1: bf16, 2: fp16) and writes the SM
  * cycles they took to out[blockIdx] (int64 [*grid_out]; only the leader of a pair writes).  bench.py derives the
  * tensor-pipe peak the 3xTF32 GEMMs are measured against from it. */
-int dppo_tc_mma_probe(dppo_ctx* ctx, int pair, int bf16, int n, int iters, long long* out, int* grid_out, void* stream);
+int dppo_tc_mma_probe(dppo_ctx* ctx, int pair, int fmt, int n, int iters, long long* out, int* grid_out, void* stream);
 
 #ifdef __cplusplus
 }
