@@ -20,7 +20,22 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key)
     }
     return ctr;
 }
-__device__ __forceinline__ float u01(uint32_t x) { return ((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f); }   // (0,1)
+// The top 24 bits of a word -> a uniform in the open interval (0, 1).  For x >> 8 == 0xFFFFFF the sum 16777215.5f rounds (to
+// even) up to 2^24, so the top word is clamped to the largest float below 1: a categorical draw's target u*s then stays below
+// s (s >= 1) and the walk stops at an action whose probability is not zero.
+__device__ __forceinline__ float u01(uint32_t x)
+{
+    return fminf(((float)(x >> 8) + 0.5f) * (1.0f / 16777216.0f), 0x1.fffffep-1f);
+}
+
+// Draw-counter tag of Gaussian dimension pair p (dimensions 2p, 2p + 1): t = p + 1, low byte in counter bits 56-63 and the next
+// byte in bits 48-55.  Non-zero (0 is the categorical stream) and distinct for every pair up to p = 65534 while the draw counter
+// stays below 2^48.  Pairs 0-254 get (p + 1) << 56, so their streams are those of the one-byte tag.
+__device__ __forceinline__ uint64_t gaussian_pair_tag(int p)
+{
+    const uint64_t t = (uint64_t)p + 1;
+    return ((t & 0xFF) << 56) | ((t >> 8) << 48);
+}
 
 __global__ void sample_categorical_kernel(const float* __restrict__ logits, int N, int A, uint64_t seed, uint64_t counter,
                                           const unsigned long long* __restrict__ counter_base, int64_t env_offset,
@@ -82,8 +97,7 @@ __global__ void sample_gaussian_kernel(const float* __restrict__ mean, const flo
     const uint64_t env = (uint64_t)(env_offset + e);
     float lp = 0.f;
     for (int j0 = 0; j0 < A; j0 += 2) {
-        // the draw counter's top byte carries the dimension-pair index
-        const uint64_t c = counter ^ ((uint64_t)(j0 / 2 + 1) << 56);
+        const uint64_t c = counter ^ gaussian_pair_tag(j0 / 2);
         const uint4 r = philox4x32_10(make_uint4((uint32_t)env, (uint32_t)(env >> 32), (uint32_t)c, (uint32_t)(c >> 32)),
                                       make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
         const float rad = sqrtf(-2.0f * logf(u01(r.x)));

@@ -123,9 +123,15 @@ int dppo_buffer_store_step(dppo_ctx* ctx, const void* record, int t, int N, int 
                            float* terminations, float* truncations, void* stream);
 int64_t dppo_step_record_bytes(int N, int D, int act_dim, int continuous);
 
-/* Categorical(logits).sample() (ppo.py:81) with a counter-based generator keyed by
+/* Stream layout of both samplers: Philox4x32-10 with key (seed lo, seed hi) and counter (env lo, env hi, c lo, c hi), where
+ * env = env_offset + row and c = counter (+ the device counter base, mod 2^64).  A word x maps to the fp32 uniform
+ * ((x >> 8) + 0.5) * 2^-24, clamped to 1 - 2^-24: it lies in the open interval (0, 1).
+ *
+ * Categorical(logits).sample() (ppo.py:81) with a counter-based generator keyed by
  * (seed, global env id, draw counter): results do not depend on the launch shape or GPU count.
- * Also emits log_prob(action) (recurrent_ppo.py:219-221).  actions: int64 [N]. */
+ * Also emits log_prob(action) (recurrent_ppo.py:219-221).  actions: int64 [N].  Word x of counter c is the inverse-CDF uniform;
+ * the walk stops at the first action whose running fp32 sum of exp(logit - max) exceeds u * sum, so an action of probability
+ * zero (logit -inf) is never drawn.  Rows must hold at least one finite logit and no NaN or +inf. */
 int dppo_sample_categorical(dppo_ctx* ctx, const float* logits, int N, int A, uint64_t seed, uint64_t counter,
                             int64_t env_offset, int64_t* actions, float* log_probs, void* stream);
 /* Greedy action of a categorical policy (evaluation): actions[e] = torch.argmax(logits[e], -1), the FIRST index of the row's
@@ -133,7 +139,10 @@ int dppo_sample_categorical(dppo_ctx* ctx, const float* logits, int N, int A, ui
  * log_softmax(logits[e])[actions[e]] with the arithmetic of dppo_sample_categorical.  No generator is involved.  The greedy action of
  * a Gaussian policy is its mean (heads bit 0 of dppo_mlp_forward / dppo_rnn_forward), which needs no kernel of its own. */
 int dppo_select_greedy_categorical(dppo_ctx* ctx, const float* logits, int N, int A, int64_t* actions, float* log_probs, void* stream);
-/* JointNormal(mean, exp(log_std)).sample() (continuous_ppo.py:92). actions: f32 [N, A]. */
+/* JointNormal(mean, exp(log_std)).sample() (continuous_ppo.py:92). actions: f32 [N, A].  Dimensions 2p and 2p + 1 share one
+ * Box-Muller draw (words x: radius, y: angle) at counter c ^ tag(p), tag(p) = ((t & 0xFF) << 56) | ((t >> 8) << 48) with
+ * t = p + 1: distinct and non-zero for every pair up to A = 131070 (so no pair shares the categorical stream or another pair's
+ * noise) while c stays below 2^48. */
 int dppo_sample_gaussian(dppo_ctx* ctx, const float* mean, const float* log_std, int N, int A, uint64_t seed,
                          uint64_t counter, int64_t env_offset, float* actions, float* log_probs, void* stream);
 
